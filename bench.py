@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- leapfrog gradient-evals/sec (and ESS/sec) of the fused HMC trajectory kernel (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload = "case3c_65536"): Case 3c of the reference (case3-script.py:136-181, README:40-45): MVN D=100,
 rho=0.95, random trajectory length L in {5..19}, dt=0.1, 1000 iterations of which 200 are warm-up, scaled to 65,536
@@ -54,6 +54,7 @@ CHAINS_PER_GPU = 65536
 NITER, WARM = 1000, 200            # README:40-45 (Case 3c as listed; case3-script.py runs 2000 / 1000)
 METRIC = "leapfrog grad-evals/sec, D=100 rho=0.95 MVN (Case 3c), 65536 chains per B200"
 UNIT = "grad-evals/s"
+DUMP_CHAINS = 128                  # --dump-outputs: 128 chains x 801 samples x 100 dims of float32 is 41 MB
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -397,6 +398,22 @@ def secondary_measurements(torch, dist, S, U, L, lib, rank, world, dev, log):
     return out
 
 
+def dump_last_step(out_dir, torch, H, step_counters, log):
+    """What a caller of the timed path receives from its last step, for comparing two builds output for output: stored
+    samples and energies of a fixed seeded sample of chains, and that step's counters (warm-up accepts, accepts, sum L,
+    sum L^2)."""
+    Nc, Lc, D = H._q_dev.shape
+    n = min(Nc, DUMP_CHAINS, max(1, (48 << 20) // (Lc * (D * 4 + 16))))
+    idx = np.sort(np.random.RandomState(0).choice(Nc, n, replace=False))
+    idx_d = torch.from_numpy(idx).to(H._q_dev.device)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"q_chain": H._q_dev.index_select(0, idx_d), "E_chain": H._E_dev.index_select(0, idx_d),
+              "dE_chain": H._dE_dev.index_select(0, idx_d), "counters": step_counters[:4].to(torch.float64)}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+    log("outputs of the last step (%d of %d chains) written to %s" % (n, Nc, out_dir))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -407,13 +424,20 @@ def main():
     ap.add_argument("--niter", type=int, default=NITER)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0: a fixed sample of %d chains) as DIR/<name>.npy"
+                         % DUMP_CHAINS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none")
     T0 = time.time()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
-    W = max(args.warmup, 0)
-    K = max(args.steps, 1)
+    W = args.warmup
+    K = args.steps
     Niter = args.niter
     warm = min(WARM, Niter // 5)
     Lc = 1 + (Niter - warm)
@@ -498,6 +522,10 @@ def main():
     ev0.record()
     for i in range(W, W + K):
         a.seed = 2026 + i
+        if args.dump_outputs and i == W + K - 1:
+            # the counters accumulate over launches: snapshot them before the last step to get its own.  With --steps
+            # above 1 this one 64-byte device copy falls inside the timed window (microseconds against a ~120 ms step)
+            c_last = counters.clone() if i > W else c0
         L.check(lib.hmc_random_run(a, stream))
     ev1.record()
     barrier()
@@ -505,6 +533,8 @@ def main():
         sampler_thread.stop()
     ms = ev0.elapsed_time(ev1)
     log("timed region done: %.1f ms for %d steps" % (ms, K))
+    if args.dump_outputs and rank == 0:
+        dump_last_step(args.dump_outputs, torch, H, counters - c_last, log)
     dc = (counters - c0).cpu().numpy().astype(np.int64)
     acc_post, sumL = int(dc[1]), int(dc[2])
     n_traj = Nc * K * Niter

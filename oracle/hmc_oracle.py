@@ -4,12 +4,11 @@ Nothing under ``oracle/`` is part of the product path.  Only ``tests/``, ``tests
 ``__graft_entry__.smoke()`` and ``bench.py``'s CPU-baseline / ``--impl reference`` legs may import it, and
 there only as the checker (or as the timed CPU baseline), never as something the product calls.
 
-Parity status: PINNED.  ``tests/test_oracle_vs_reference.py`` runs the real reference (through
-``oracle/ref_shim.py``, build container only) against this restatement on the same ``np.random`` stream and
-requires agreement to 1e-12; the committed fixtures under ``tests/golden/`` were produced by the reference
-itself (``tests/golden/make_golden.py``) and are what the restatement is checked against on the GPU box,
-where ``/root/reference`` does not exist.  The README known-answer tables (README:332-358) pin the NUTS
-index helpers.
+Parity status: PINNED.  The committed fixtures under ``tests/golden/`` were produced by the reference itself
+(``tests/golden/make_golden.py``, through ``oracle/ref_shim.py``).  ``tests/test_oracle_golden.py`` replays their
+recorded draws through this restatement, and ``tests/test_oracle_vs_reference.py`` reruns each case from its seed on
+the same ``np.random`` stream; both require agreement to 1e-12.  The README known-answer tables (README:332-358) pin
+the NUTS index helpers.
 
 Every function cites the reference ``file:line`` it follows (paths relative to /root/reference).
 """

@@ -10,6 +10,34 @@ RANDOM_FIXTURES = ["random_case1a", "random_d10_thin3", "random_case3c_small", "
                    "random_case2c_small", "random_vecdt_covp", "random_constL"]
 NUTS_FIXTURES = ["nuts_d2", "nuts_d10", "nuts_case3c_small", "nuts_covp"]
 
+# The cases the fixtures were generated from (tests/golden/make_golden.py runs the reference on each).
+CASES = [
+    # name, sampler, D, rho, Nchain, Niter, warm, thin, dt, extra kwargs, start scale, seed, N_save_chain0
+    ("random_case1a", "Random", 2, 0.0, 10, 1000, 200, 1, 0.1, dict(L_low=5, L_high=20), 2.0, 0, 20),
+    ("random_d10_thin3", "Random", 10, 0.95, 6, 90, 30, 3, 0.1, dict(L_low=5, L_high=20), 2.0, 1, 0),
+    ("random_case3c_small", "Random", 100, 0.95, 4, 60, 20, 1, 0.1, dict(L_low=5, L_high=20), 2.0, 2, 10),
+    ("random_case3d_small", "Random", 100, 0.95, 2, 12, 4, 1, 0.1, dict(L_low=50, L_high=200), 2.0, 3, 0),
+    ("random_case2c_small", "Random", 100, 0.0, 4, 40, 10, 1, 0.1, dict(L_low=5, L_high=20), 100.0, 4, 0),
+    ("random_vecdt_covp", "Random", 6, 0.5, 4, 50, 10, 2, "vec", dict(L_low=3, L_high=9, cov_p="diag"), 2.0, 5, 0),
+    # the reference's live sampler with L_low = L, L_high = L + 1: randint(7, 8) is always 7 -- a FIXED trajectory length with
+    # the live bookkeeping; pins sampler_type="Fixed" of the B200 build (a silent no-op upstream, SURVEY H8)
+    ("random_constL", "Random", 10, 0.9, 5, 40, 10, 1, 0.15, dict(L_low=7, L_high=8), 2.0, 9, 6),
+    ("nuts_d2", "NUTS", 2, 0.0, 4, 40, 10, 1, 0.3, dict(d_max=10), 2.0, 6, 0),
+    ("nuts_d10", "NUTS", 10, 0.95, 3, 30, 10, 2, 0.1, dict(d_max=12), 2.0, 7, 0),
+    ("nuts_case3c_small", "NUTS", 100, 0.95, 2, 8, 2, 1, 0.2, dict(d_max=10), 1.0, 8, 0),
+    # NUTS with a non-identity momentum metric (samplers.py:352-356, 811-817, 835-837: force times M^-1, q moved by p, Q9)
+    ("nuts_covp", "NUTS", 6, 0.5, 3, 25, 5, 1, 0.15, dict(d_max=10, cov_p="diag"), 2.0, 10, 0),
+]
+
+
+def pin_start(name, q_start):
+    """The case's own edits of the drawn start points: case 2c puts chain 0 far out (case2-script.py:58-61)."""
+    if name == "random_case2c_small":
+        q_start[0, :] = 0
+        q_start[0, 0] = 1000
+        q_start[0, 1] = -750
+    return q_start
+
 
 def load(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)

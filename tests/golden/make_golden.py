@@ -14,26 +14,10 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))
 
 from oracle import ref_shim  # noqa: E402
-
-CASES = [
-    # name, sampler, D, rho, Nchain, Niter, warm, thin, dt, extra kwargs, start scale, seed, N_save_chain0
-    ("random_case1a", "Random", 2, 0.0, 10, 1000, 200, 1, 0.1, dict(L_low=5, L_high=20), 2.0, 0, 20),
-    ("random_d10_thin3", "Random", 10, 0.95, 6, 90, 30, 3, 0.1, dict(L_low=5, L_high=20), 2.0, 1, 0),
-    ("random_case3c_small", "Random", 100, 0.95, 4, 60, 20, 1, 0.1, dict(L_low=5, L_high=20), 2.0, 2, 10),
-    ("random_case3d_small", "Random", 100, 0.95, 2, 12, 4, 1, 0.1, dict(L_low=50, L_high=200), 2.0, 3, 0),
-    ("random_case2c_small", "Random", 100, 0.0, 4, 40, 10, 1, 0.1, dict(L_low=5, L_high=20), 100.0, 4, 0),
-    ("random_vecdt_covp", "Random", 6, 0.5, 4, 50, 10, 2, "vec", dict(L_low=3, L_high=9, cov_p="diag"), 2.0, 5, 0),
-    # the reference's live sampler with L_low = L, L_high = L + 1: randint(7, 8) is always 7 -- a FIXED trajectory length with
-    # the live bookkeeping; pins sampler_type="Fixed" of the B200 build (a silent no-op upstream, SURVEY H8)
-    ("random_constL", "Random", 10, 0.9, 5, 40, 10, 1, 0.15, dict(L_low=7, L_high=8), 2.0, 9, 6),
-    ("nuts_d2", "NUTS", 2, 0.0, 4, 40, 10, 1, 0.3, dict(d_max=10), 2.0, 6, 0),
-    ("nuts_d10", "NUTS", 10, 0.95, 3, 30, 10, 2, 0.1, dict(d_max=12), 2.0, 7, 0),
-    ("nuts_case3c_small", "NUTS", 100, 0.95, 2, 8, 2, 1, 0.2, dict(d_max=10), 1.0, 8, 0),
-    # NUTS with a non-identity momentum metric (samplers.py:352-356, 811-817, 835-837: force times M^-1, q moved by p, Q9)
-    ("nuts_covp", "NUTS", 6, 0.5, 3, 25, 5, 1, 0.15, dict(d_max=10, cov_p="diag"), 2.0, 10, 0),
-]
+from _util import CASES, pin_start  # noqa: E402
 
 
 def split_tape(tape, sampler, Nchain, Niter, D):
@@ -94,11 +78,7 @@ def main():
             return np.dot(inv_cov0, (q - q0))
 
         np.random.seed(seed)
-        q_start = ru.start_pts(q0, np.diag(np.ones(D)) * sscale, Nchain)
-        if name == "random_case2c_small":          # case2-script.py:58-61
-            q_start[0, :] = 0
-            q_start[0, 0] = 1000
-            q_start[0, 1] = -750
+        q_start = pin_start(name, ru.start_pts(q0, np.diag(np.ones(D)) * sscale, Nchain))
         dt_val = dt
         if isinstance(dt, str):
             dt_val = 0.05 + 0.1 * np.arange(D) / D

@@ -1,50 +1,36 @@
-"""Live pin of the oracle against the real reference (build container only; skipped where /root/reference is absent)."""
+"""The oracle against the reference on the same ``np.random`` stream.
+
+The reference's outputs are the committed fixtures (tests/golden/make_golden.py ran the reference from the seed of each
+case).  Here the oracle starts from the same seed, draws the start points with the reference's call, then consumes the
+global stream through ``NumpyDraws`` exactly as the reference did, and must land on the reference's numbers."""
 import numpy as np
 import pytest
 
 from oracle import hmc_oracle as O
-from oracle import ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference source tree not present")
+from _util import CASES, load, pin_start
 
 
-def _run_both(D, rho, Nchain, Niter, warm, thin, stype, seed, dt=0.1, **kw):
-    ru, rs = ref_shim.load_reference()
-    tgt = O.MVNTarget(np.zeros(D), O.equicorrelated_cov(D, rho))
-    q0, cov0, inv_cov0 = tgt.q0, tgt.cov0, np.linalg.inv(tgt.cov0)
-    V = lambda q: -ru.normal_lnL(q, q0, cov0)            # case1-script.py:39-43
-    dVdq = lambda q: np.dot(inv_cov0, (q - q0))          # case1-script.py:45-49
+@pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
+def test_same_stream_same_numbers(case):
+    name, stype, D, rho, Nchain, Niter, warm, thin, dt, kw, sscale, seed, nsave = case
+    fx = load(name)
+    tgt = O.MVNTarget(fx["q0"], fx["cov0"])
     np.random.seed(seed)
-    q_start = ru.start_pts(q0, np.diag(np.ones(D)) * 2, Nchain)
-    state = np.random.get_state()
-    H = rs.HMC_sampler(D, V, dVdq, Niter=Niter, Nchain=Nchain, sampler_type=stype, dt=dt, thin_rate=thin,
-                       warm_up_num=warm, **kw)
-    H.gen_sample(q_start, N_save_chain0=0, verbose=False)
-    H.compute_convergence_stats()
-    np.random.set_state(state)
-    draws = O.NumpyDraws(D)
+    q_start = np.random.multivariate_normal(tgt.q0, np.diag(np.ones(D)) * sscale, size=Nchain)     # utils.py:204-209
+    np.testing.assert_array_equal(pin_start(name, q_start), fx["q_start"])
+    dt = fx["dt"] if fx["dt"].ndim else float(fx["dt"])
+    draws = O.NumpyDraws(D, fx["cov_p"])
     if stype == "Random":
         R = O.gen_sample_random(D, tgt.V, tgt.dVdq, q_start, draws, Nchain, Niter, thin, warm, dt,
-                                kw["L_low"], kw["L_high"])
+                                kw["L_low"], kw["L_high"], cov_p=fx["cov_p"], N_save_chain0=nsave)
     else:
-        R = O.gen_sample_NUTS(D, tgt.V, tgt.dVdq, q_start, draws, Nchain, Niter, thin, warm, dt, kw["d_max"])
-    return H, R
-
-
-@pytest.mark.parametrize("args,kw", [
-    ((2, 0.0, 4, 60, 20, 1, "Random", 10), dict(L_low=5, L_high=20)),
-    ((10, 0.95, 3, 40, 10, 3, "Random", 11), dict(L_low=5, L_high=20)),
-    ((100, 0.95, 2, 12, 4, 1, "Random", 12), dict(L_low=5, L_high=20)),
-    ((2, 0.0, 3, 30, 10, 1, "NUTS", 13), dict(dt=0.3, d_max=10)),
-    ((10, 0.95, 2, 12, 4, 2, "NUTS", 14), dict(dt=0.1, d_max=12)),
-])
-def test_same_stream_same_numbers(args, kw):
-    H, R = _run_both(*args, **kw)
-    np.testing.assert_allclose(R.q_chain, H.q_chain, rtol=0, atol=1e-12)
-    np.testing.assert_allclose(R.E_chain, H.E_chain, rtol=0, atol=1e-10)
-    np.testing.assert_allclose(R.dE_chain, H.dE_chain, rtol=0, atol=1e-10)
-    assert R.N_total_steps == H.N_total_steps
-    assert R.accept_R == H.accept_R
+        R = O.gen_sample_NUTS(D, tgt.V, tgt.dVdq, q_start, draws, Nchain, Niter, thin, warm, dt, kw["d_max"],
+                              cov_p=fx["cov_p"])
+    np.testing.assert_allclose(R.q_chain, fx["q_chain"], rtol=0, atol=1e-12)
+    np.testing.assert_allclose(R.E_chain, fx["E_chain"], rtol=0, atol=1e-10)
+    np.testing.assert_allclose(R.dE_chain, fx["dE_chain"], rtol=0, atol=1e-10)
+    assert R.N_total_steps == int(fx["N_total_steps"])
+    assert R.accept_R == float(fx["accept_R"])
     Rq, neff = O.convergence_stats(R.q_chain[:, 1:, :], 1, 0)
-    np.testing.assert_allclose(Rq, H.R_q, rtol=1e-12)
-    np.testing.assert_allclose(neff, H.n_eff_q, rtol=1e-12)
+    np.testing.assert_allclose(Rq, fx["R_q"], rtol=1e-12)
+    np.testing.assert_allclose(neff, fx["n_eff_q"], rtol=1e-12)
