@@ -41,14 +41,15 @@ enum { HMC_F32 = 0, HMC_F64 = 1 };
 
 /* which kernel implements the run */
 enum {
-    HMC_KERNEL_AUTO = 0,    /* tensor-core kernel if it covers the run, else the large-D GEMM path (when a workspace is given), else
-                               the FFMA2 kernel, else the generic one */
+    HMC_KERNEL_AUTO = 0,    /* tensor-core kernel if it covers the run, else the large-D GEMM path (when a workspace is given and
+                               D % 256 == 0 or D > 1024), else the FFMA2 kernel, else the generic one */
     HMC_KERNEL_GENERIC = 1, /* one warp per chain, any D <= 1024, float or double (parity workhorse) */
     HMC_KERNEL_FAST = 2,    /* FP32 FFMA2 register-tile kernel, 20 < D <= 128, identity momentum metric */
     HMC_KERNEL_TC = 3,      /* tcgen05 tensor-core kernel (bf16x3 / fp16x2 split, fp32 accumulate in TMEM), D <= 100 and a multiple of 4
                                (smaller targets run zero padded in the 100-wide tile; AUTO picks it from D = 52), identity metric */
-    HMC_KERNEL_BIGD = 4     /* large D (multiple of 256): one tcgen05 GEMM over all chains per leapfrog step, operands by TMA, the
-                               leapfrog update fused into the epilogue; needs hmc_random_args.workspace */
+    HMC_KERNEL_BIGD = 4     /* large D, any 128 <= D <= 8192, float32, identity metric: one tcgen05 GEMM over all chains per leapfrog
+                               step, operands by TMA, the leapfrog update fused into the epilogue; works on D rounded up to 32 (the
+                               padded dimensions stay zero); needs hmc_random_args.workspace */
 };
 
 /* hmc_random_args.flags */
@@ -147,7 +148,8 @@ typedef struct hmc_random_args {
 } hmc_random_args;
 
 int hmc_random_run(const hmc_random_args* args, void* cuda_stream);
-/* bytes of hmc_random_args.workspace the large-D path needs for this configuration (0 when it does not apply) */
+/* bytes of hmc_random_args.workspace the large-D path needs for this configuration: non-zero exactly for the runs it covers
+   (float32, identity metric, 128 <= D <= 8192), whatever kernel is asked for; 0 otherwise.  Depends on Nchain and D only. */
 int64_t hmc_random_workspace_bytes(const hmc_random_args* args);
 
 /*

@@ -64,10 +64,12 @@ extern "C" int hmc_random_run(const hmc_random_args* args, void* cuda_stream) {
     const char* why = "";
     // tensor-core kernel where it applies and pays (its 100-wide tile does the work of D = 100 whatever D is: ~6.4e9
     // gradient-evals/s; the FFMA kernel's rate grows as 1/D^2 and overtakes it below D ~ 50), then the large-D GEMM path, then
-    // the FFMA kernel, then the generic one
+    // the FFMA kernel, then the generic one.  The large-D path covers every 128 <= D <= 8192; AUTO takes it for D % 256 == 0
+    // (unpadded tiles) and for D > 1024 (beyond the generic kernel), and leaves 128 < D <= 1024 otherwise to the generic kernel
+    // (HMC_KERNEL_BIGD reaches the padded path there)
     if (kernel == HMC_KERNEL_AUTO)
         kernel = (a.target.D >= 52 && hmc_random_tc_supported(a, &why)) ? HMC_KERNEL_TC
-                 : (a.workspace && hmc_random_bigd_supported(a, &why)) ? HMC_KERNEL_BIGD
+                 : (a.workspace && hmc_random_bigd_supported(a, &why) && (a.target.D % 256 == 0 || a.target.D > 1024)) ? HMC_KERNEL_BIGD
                  : hmc_random_fast_supported(a, &why) ? HMC_KERNEL_FAST : HMC_KERNEL_GENERIC;
     if (kernel == HMC_KERNEL_BIGD) {
         if (!hmc_random_bigd_supported(a, &why)) {

@@ -4,6 +4,11 @@
 //
 // Follows HMC_sampler.gen_sample_random + leap_frog (/root/reference/samplers.py:387-491, 831-839).
 //
+// Any 128 <= D <= 8192: the GEMM works on Dp = D rounded up to 32 (one K stage).  Every operand, state row and the force matrix
+// are Dp wide and zero in the padded dimensions (no force, no momentum, dt = 0 there), so those stay zero and add nothing to the
+// energies; K = Dp, and the last column tile is Dp - (NT - 1) BN wide when BN does not divide Dp.  For D % 256 == 0, Dp = D
+// and nothing changes.  Only the caller's rows (start points, stored samples, state_q, the chain-0 trace) are exactly D wide.
+//
 // One PASS = one gradient evaluation for every chain (SURVEY H9: per-step GEMM with the leapfrog update fused in):
 //   bigd_gemm_step   persistent CTAs (clusters of two row blocks) over (128 chains x 256 dimensions) tiles, K = D.  Warp 0 issues
 //                    the TMA loads (cp.async.bulk.tensor, 64-byte swizzle, 3 stages of K = 32; the B tile multicast to the
@@ -38,7 +43,8 @@
 namespace {
 
 constexpr int BM = 128;            // chains per tile (UMMA M)
-constexpr int BN_MAX = 256;        // dimensions per tile (UMMA N; fp32 accumulator columns): 256 for the two-part split, 128 for the three-part one (shared memory)
+// dimensions per tile (UMMA N; fp32 accumulator columns) is a template parameter BN: 256 for the two-part split, 128 for the
+// three-part one (shared memory)
 // K per stage is a template parameter BK in {64, 32, 16} (one swizzle row of 128 / 64 / 32 bytes) with 128 / BK stages: the bytes
 // of operand memory are the same, the pipeline is finer -- a stage can only be refilled after its MMAs are done, so with two
 // 96 KB stages one load is in flight while the other stage is consumed and the tensor pipe waits for most of a load's latency.
@@ -146,17 +152,19 @@ __device__ __forceinline__ void split_pair(float x0, float x1, uint32_t (&h)[3])
 }
 
 struct BigdWs {                      // workspace carved by the host (all device pointers)
-    uint16_t* xp;                    // [2][NPART][Ncp][D]  split position = A operand: pass n reads buffer n & 1 and writes the other one
+    uint16_t* xp;                    // [2][NPART][Ncp][Dp]  split position = A operand: pass n reads buffer n & 1 and writes the other one
                                      // (the column tiles of a row block read ALL its columns while one of them already writes its own)
     int wr;                          // buffer the parts of the next pass go to (set per launch)
     int* perm;                       // [Ncp] row -> local chain index (-1: padding row).  Rows are chains SORTED by the number of passes
                                      // their run needs (the trajectory lengths are a pure function of (seed, chain, iteration)), so the
                                      // 128 chains of a row block end together and finished blocks drop out of the GEMM early
     int* plan;                       // [Ncp] passes a chain needs: sum over its iterations of L + 1
-    uint16_t* bp;                    // [NPART][D][D]    split force matrix (x 2^s for the fp16 split) = B operand
-    float* x;                        // [Ncp][D] shifted position q - mu
-    float* x0;                       // [Ncp][D] position at the start of the running trajectory
-    float* p;                        // [Ncp][D] momentum
+    uint16_t* bp;                    // [NPART][Dp][Dp]  split force matrix (x 2^s for the fp16 split) = B operand, zero outside D x D
+    float* x;                        // [Ncp][Dp] shifted position q - mu
+    float* x0;                       // [Ncp][Dp] position at the start of the running trajectory
+    float* p;                        // [Ncp][Dp] momentum
+    float* mu;                       // [Dp] target mean, zero from D on
+    float* dt;                       // [Dp] step sizes, zero from D on (the padded dimensions never move)
     float* red;                      // [Ncp][NT][2][2] partial (q.g, p.p) per column tile and epilogue warp of the last pass
     int* mode;                       // [Ncp] MD_*
     int* l;                          // [Ncp] leapfrog steps done in the running trajectory
@@ -173,6 +181,8 @@ struct BigdWs {                      // workspace carved by the host (all device
     int* counters;                   // [0..1] list length by pass parity, [2] running chains after the last events kernel
     float binv;                      // 2^-s
     int Ncp, NT, npart;
+    int Dp;                          // D rounded up to whole K stages (32): the width of every row and matrix above.  The padded
+                                     // dimensions hold zeros throughout: no force, no momentum, no step
 };
 
 // CL = CTAs per cluster (launch attribute): the CL row blocks of a cluster work on the SAME column block at the same time, each
@@ -186,7 +196,7 @@ template <int NPART, int BN, int CL, int BK, int STAGES>
 __global__ void __launch_bounds__(NTHREADS, 1) bigd_gemm_step(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                                                               const __grid_constant__ CUtensorMap mapP, const __grid_constant__ CUtensorMap mapX,
                                                               const __grid_constant__ CUtensorMap mapS,
-                                                              BigdWs w, int Nchain, int D, const float* __restrict__ dtv) {
+                                                              BigdWs w, int Nchain, int Dp, const float* __restrict__ dtv) {
     extern __shared__ __align__(1024) unsigned char smem[];
     constexpr int A_BYTES = BM * BK * 2, B_BYTES = BN * BK * 2;                 // one part of one stage
     constexpr int STAGE_BYTES = NPART * (A_BYTES + B_BYTES);
@@ -217,9 +227,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) bigd_gemm_step(const __grid_const
     if constexpr (CL > 1) cluster_sync_all();              // barriers of every CTA initialised before anybody signals them
     asm volatile("tcgen05.fence::after_thread_sync;");
     const uint32_t tmem = *tmem_slot;
-    const int NT = w.NT, KB = D / BK;
+    const int NT = w.NT, KB = Dp / BK;
+    // the last column tile is narrow when BN does not divide Dp: its MMAs run at N = n_last (a multiple of 32) and its epilogue
+    // takes n_last / CW chunks.  Its B loads keep the full box: the rows past n_last are loaded (the next part's first rows, or
+    // the TMA's zero fill past the last part) but no MMA reads them, so the stage's transaction bytes stay STAGE_BYTES
+    const int n_last = Dp - (NT - 1) * BN;
     const int ntiles = (w.Ncp / (BM * CL)) * NT;            // work items of a cluster: (CL row blocks, one column block)
-    const size_t part_rows_a = (size_t)w.Ncp, part_rows_b = (size_t)D;
+    const size_t part_rows_a = (size_t)w.Ncp, part_rows_b = (size_t)Dp;
     const int crank = (CL > 1) ? (int)cluster_ctarank() : 0;
     const int cid = blockIdx.x / CL, ncl = gridDim.x / CL;
     constexpr uint16_t cmask = (uint16_t)((1u << CL) - 1u);
@@ -264,10 +278,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) bigd_gemm_step(const __grid_const
         // ===== MMA issuer =====
         if (lane == 0) {
             constexpr uint32_t fmt = (NPART == 2) ? 0u : 1u;       // 0 = f16, 1 = bf16
-            const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+            const uint32_t idesc0 = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(BM >> 4) << 24);
+            const uint32_t idesc_full = idesc0 | ((uint32_t)(BN >> 3) << 17), idesc_last = idesc0 | ((uint32_t)(n_last >> 3) << 17);
             uint32_t n = 0, nt_done = 0;
             for (int t = cid; t < ntiles; t += ncl) {
                 if (!item_active(t / NT)) continue;
+                const uint32_t idesc = (t % NT == NT - 1) ? idesc_last : idesc_full;
                 const int as = nt_done & 1;
                 mbar_wait(tempty + as, ((nt_done >> 1) & 1) ^ 1);
                 asm volatile("tcgen05.fence::after_thread_sync;");
@@ -308,7 +324,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) bigd_gemm_step(const __grid_const
         const int quarter = warp & 3, ew = warp - 2, half = ew >> 2;    // (two warps of a quarter take alternating chunks)
         unsigned char* ebase = epi + ew * EPI_WARP_BYTES;
         uint64_t* ef = efull + ew * NBUF;
-        constexpr int NCH = BN / CW;                        // chunks of a tile
+        auto nch = [&](int tt) { return ((tt % NT) == NT - 1 ? n_last : BN) / CW; };    // chunks of a tile
         // a tile is LIVE for this warp when one of its 32 chains takes part in the pass; only live tiles enter the chunk stream
         auto tile_md = [&](int tt) { const long ch = (long)((tt / NT) * CL + crank) * BM + quarter * 32 + lane;
                                      return (ch < Nchain) ? w.mode[ch] : (int)MD_IDLE; };
@@ -333,7 +349,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) bigd_gemm_step(const __grid_const
             if (pf_t >= ntiles) return;
             issue_chunk(pf_t, pf_c, pf_g);
             ++pf_g;
-            if ((pf_c += NHALF) >= NCH) { pf_c = half; pf_t = next_live(pf_t); }
+            if ((pf_c += NHALF) >= nch(pf_t)) { pf_c = half; pf_t = next_live(pf_t); }
         };
         prefetch_one();
         prefetch_one();
@@ -355,6 +371,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) bigd_gemm_step(const __grid_const
             asm volatile("tcgen05.fence::after_thread_sync;");
             float hv = 0.f, hk = 0.f;
             if (live) {
+                const int NCH = nch(t);
                 for (int c = half; c < NCH; c += NHALF, ++g) {
                     const int buf = g % NBUF;
                     unsigned char* bp = ebase + buf * EPI_BUF_BYTES;
@@ -434,20 +451,33 @@ __global__ void __launch_bounds__(NTHREADS, 1) bigd_gemm_step(const __grid_const
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// momentum draw for one chain by one warp: p row, 0.5 |p|^2, and (iteration >= 1) trajectory length and log-uniform
-// (same Philox keying as every other kernel: hmc_normal4 / hmc_scalar_draws)
+// momentum draw for one chain by one warp: p row (Dp wide, zero from D on), 0.5 |p|^2 of the D real dimensions, and
+// (iteration >= 1) trajectory length and log-uniform (same Philox keying as every other kernel: hmc_normal4 / hmc_scalar_draws;
+// when D % 4 != 0 only the first D % 4 normals of the last slot are used)
 // ---------------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float bigd_draw(const hmc_random_args& a, long m, int iter, int lane, float* prow, int* L, float* lnu) {
+__device__ __forceinline__ float bigd_draw(const hmc_random_args& a, int Dp, long m, int iter, int lane, float* prow, int* L, float* lnu) {
     const int D = a.target.D;
     const uint64_t gid = (uint64_t)(a.chain_id0 + m);
     float s = 0.f;
     if (a.p_tape) {
         const double* src = a.p_tape + ((size_t)m * (a.Niter + 1) + iter) * D;
         for (int j = lane; j < D; j += 32) { const float v = (float)src[j]; if (prow) prow[j] = v; s = fmaf(v, v, s); }
+        if (prow) for (int j = D + lane; j < Dp; j += 32) prow[j] = 0.f;
         if (iter >= 1) { *L = a.L_tape[(size_t)m * a.Niter + iter - 1]; *lnu = (float)log(a.u_tape[(size_t)m * a.Niter + iter - 1]); }
     } else {
         for (int sl = lane; sl < D / 4; sl += 32) {
             const float4 z = hmc_normal4(a.seed, gid, (uint32_t)iter, (uint32_t)sl);
+            if (prow) *reinterpret_cast<float4*>(prow + 4 * sl) = z;
+            s += z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w;
+        }
+        for (int sl = D / 4 + lane; sl < Dp / 4; sl += 32) {             // the partly used last slot, then the padding
+            float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (4 * sl < D) {
+                z = hmc_normal4(a.seed, gid, (uint32_t)iter, (uint32_t)sl);
+                z.w = 0.f;
+                if (4 * sl + 2 >= D) z.z = 0.f;
+                if (4 * sl + 1 >= D) z.y = 0.f;
+            }
             if (prow) *reinterpret_cast<float4*>(prow + 4 * sl) = z;
             s += z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w;
         }
@@ -457,12 +487,13 @@ __device__ __forceinline__ float bigd_draw(const hmc_random_args& a, long m, int
 }
 
 template <int NPART>
-__device__ __forceinline__ void bigd_write_parts(const BigdWs& w, long m, int D, int lane, const float* xrow) {
-    for (int j = 2 * lane; j < D; j += 64) {
+__device__ __forceinline__ void bigd_write_parts(const BigdWs& w, long m, int lane, const float* xrow) {
+    const int Dp = w.Dp;
+    for (int j = 2 * lane; j < Dp; j += 64) {
         uint32_t h[3];
         split_pair<NPART>(xrow[j], xrow[j + 1], h);
 #pragma unroll
-        for (int pt = 0; pt < NPART; ++pt) reinterpret_cast<uint32_t*>(w.xp + (((size_t)w.wr * NPART + pt) * w.Ncp + m) * D)[j >> 1] = h[pt];
+        for (int pt = 0; pt < NPART; ++pt) reinterpret_cast<uint32_t*>(w.xp + (((size_t)w.wr * NPART + pt) * w.Ncp + m) * Dp)[j >> 1] = h[pt];
     }
 }
 
@@ -484,22 +515,22 @@ __global__ void __launch_bounds__(256) bigd_plan(hmc_random_args a, int* __restr
 // chain start (samplers.py:411-420) or resume from state_q: one warp per chain
 template <int NPART>
 __global__ void __launch_bounds__(128) bigd_init(hmc_random_args a, BigdWs w) {
-    const int lane = threadIdx.x & 31, D = a.target.D;
+    const int lane = threadIdx.x & 31, D = a.target.D, Dp = w.Dp;
     const long m = (long)blockIdx.x * 4 + (threadIdx.x >> 5);            // row of the workspace
     if (m >= w.Ncp) return;
-    float* xr = w.x + (size_t)m * D;
-    float* x0r = w.x0 + (size_t)m * D;
-    float* pr = w.p + (size_t)m * D;
+    float* xr = w.x + (size_t)m * Dp;
+    float* x0r = w.x0 + (size_t)m * Dp;
+    float* pr = w.p + (size_t)m * Dp;
     const long c = w.perm[m];                                            // the chain that lives in this row
     if (c < 0) {                                             // padding rows of the last tile
-        for (int j = lane; j < D; j += 32) { xr[j] = 0.f; x0r[j] = 0.f; pr[j] = 0.f; }
-        bigd_write_parts<NPART>(w, m, D, lane, xr);
+        for (int j = lane; j < Dp; j += 32) { xr[j] = 0.f; x0r[j] = 0.f; pr[j] = 0.f; }
+        bigd_write_parts<NPART>(w, m, lane, xr);
         if (lane == 0) { w.mode[m] = MD_IDLE; w.it[m] = a.iter_end + 1; }
         return;
     }
     const bool fresh = a.iter_begin == 0;
     const float* src = (fresh ? (const float*)a.q_start : (const float*)a.state_q) + (size_t)c * D;
-    const float* mu = (const float*)a.target.mu;
+    const float* mu = w.mu;
     const long Lc = 1 + (a.Niter - a.warm_up_num) / a.thin_rate;
     const long Lrow = a.store_ring > 0 ? a.store_ring : Lc;
     for (int j = lane; j < D; j += 32) {
@@ -507,13 +538,14 @@ __global__ void __launch_bounds__(128) bigd_init(hmc_random_args a, BigdWs w) {
         if (fresh) ((float*)a.q_chain)[(size_t)c * Lrow * D + j] = v;              // samplers.py:413
         xr[j] = v - mu[j]; x0r[j] = v - mu[j];
     }
+    for (int j = D + lane; j < Dp; j += 32) { xr[j] = 0.f; x0r[j] = 0.f; }
     __syncwarp();
-    bigd_write_parts<NPART>(w, m, D, lane, xr);
+    bigd_write_parts<NPART>(w, m, lane, xr);
     int L = 1; float lnu = 0.f;
     float K0 = 0.f;
-    if (fresh) K0 = bigd_draw(a, c, 0, lane, nullptr, &L, &lnu);                   // samplers.py:415 (K only)
+    if (fresh) K0 = bigd_draw(a, Dp, c, 0, lane, nullptr, &L, &lnu);               // samplers.py:415 (K only)
     const int it = a.iter_begin + 1;
-    const float Kn = bigd_draw(a, c, it, lane, pr, &L, &lnu);                      // samplers.py:431, 441, 461
+    const float Kn = bigd_draw(a, Dp, c, it, lane, pr, &L, &lnu);                  // samplers.py:431, 441, 461
     if (lane == 0) {
         w.mode[m] = (it <= a.iter_end) ? MD_FIRST : MD_IDLE;
         w.l[m] = 0; w.L[m] = L; w.it[m] = it; w.init[m] = fresh ? 1 : 0;
@@ -526,7 +558,7 @@ __global__ void __launch_bounds__(128) bigd_init(hmc_random_args a, BigdWs w) {
 // per-chain bookkeeping after a pass (one thread per chain, one block per 128-chain tile)
 __global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, int pass) {
     const long m = (long)blockIdx.x * BM + threadIdx.x;                              // row (the grid covers the Ncp rows exactly)
-    const int D = a.target.D;
+    const int Dp = w.Dp;
     const long Lc = 1 + (a.Niter - a.warm_up_num) / a.thin_rate;
     const long Lrow = a.store_ring > 0 ? a.store_ring : Lc;
     if (blockIdx.x == 0 && threadIdx.x == 0) w.counters[(pass + 1) & 1] = 0;       // list length of the NEXT pass
@@ -539,7 +571,7 @@ __global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, i
         const float V = fmaf(0.5f * w.binv, hv, (float)a.target.v_const);           // V(q) at the point the gradient was taken
         const int it = w.it[m];
         const bool tr = a.phi_q && (a.chain_id0 + c) == 0 && it <= a.N_save_chain0;
-        const float* mu = (const float*)a.target.mu;
+        const float* mu = w.mu;
         if (md == MD_FIRST) {
             const int L = w.L[m];
             sL = (unsigned long long)L; sL2 = (unsigned long long)L * L;
@@ -558,8 +590,8 @@ __global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, i
             if (tr) {                                                               // samplers.py:442-452
                 a.phi_len[it - 1] = L + 1;
                 double* phi = a.phi_q + (size_t)(it - 1) * a.L_high * 2;
-                phi[0] = (double)(w.x0[(size_t)m * D] + mu[0]); phi[1] = (double)(w.x0[(size_t)m * D + 1] + mu[1]);
-                phi[2] = (double)(w.x[(size_t)m * D] + mu[0]); phi[3] = (double)(w.x[(size_t)m * D + 1] + mu[1]);
+                phi[0] = (double)(w.x0[(size_t)m * Dp] + mu[0]); phi[1] = (double)(w.x0[(size_t)m * Dp + 1] + mu[1]);
+                phi[2] = (double)(w.x[(size_t)m * Dp] + mu[0]); phi[3] = (double)(w.x[(size_t)m * Dp + 1] + mu[1]);
             }
             w.l[m] = 1;
             md = (L == 1) ? MD_LAST : MD_MID;
@@ -567,7 +599,7 @@ __global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, i
             const int l = w.l[m] + 1;
             if (tr) {
                 double* phi = a.phi_q + (size_t)(it - 1) * a.L_high * 2;
-                phi[2 * l] = (double)(w.x[(size_t)m * D] + mu[0]); phi[2 * l + 1] = (double)(w.x[(size_t)m * D + 1] + mu[1]);
+                phi[2 * l] = (double)(w.x[(size_t)m * Dp] + mu[0]); phi[2 * l + 1] = (double)(w.x[(size_t)m * Dp + 1] + mu[1]);
             }
             w.l[m] = l;
             if (l == w.L[m]) md = MD_LAST;
@@ -603,65 +635,72 @@ __global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, i
 // trajectory ends: one warp per listed chain
 template <int NPART>
 __global__ void __launch_bounds__(256) bigd_trajectory_end(hmc_random_args a, BigdWs w, int pass) {
-    const int lane = threadIdx.x & 31, D = a.target.D;
+    const int lane = threadIdx.x & 31, D = a.target.D, Dp = w.Dp;
     const int n = w.counters[pass & 1];
     const long Lc = 1 + (a.Niter - a.warm_up_num) / a.thin_rate;
     const long Lrow = a.store_ring > 0 ? a.store_ring : Lc;
-    const float* mu = (const float*)a.target.mu;
+    const float* mu = w.mu;
+    const bool ext4 = (D & 3) == 0;             // the external rows (stored samples, state_q) are D wide: 16-byte aligned only then
     for (int e = blockIdx.x * 8 + (threadIdx.x >> 5); e < n; e += gridDim.x * 8) {
         const int ent = w.list[e];
         const long m = ent & 0x7fffffff;                                            // row
         const long c = w.perm[m];                                                   // its chain
         const bool accepted = ent < 0;
-        float* xr = w.x + (size_t)m * D;
-        float* x0r = w.x0 + (size_t)m * D;
+        float* xr = w.x + (size_t)m * Dp;
+        float* x0r = w.x0 + (size_t)m * Dp;
         int it = w.it[m];
         const bool keep = it >= a.warm_up_num;
         float* dst = keep ? (float*)a.q_chain + ((size_t)c * Lrow + ((it - a.warm_up_num) / a.thin_rate) % Lrow) * D : nullptr;
         const bool last = it >= a.iter_end;
         float* sq = last ? (float*)a.state_q + (size_t)c * D : nullptr;
-        if (accepted) {                                                             // samplers.py:463-469
-            for (int j = 4 * lane; j < D; j += 128) {
-                const float4 v = *reinterpret_cast<const float4*>(xr + j);
-                *reinterpret_cast<float4*>(x0r + j) = v;
+        // accepted: start point <- proposal (samplers.py:463-469); rejected: proposal <- start point (samplers.py:470-472)
+        const float* from = accepted ? xr : x0r;
+        float* to = accepted ? x0r : xr;
+        for (int j = 4 * lane; j < Dp; j += 128) {
+            const float4 v = *reinterpret_cast<const float4*>(from + j);
+            *reinterpret_cast<float4*>(to + j) = v;
+            if (ext4 && j < D) {
                 const float4 mu4 = *reinterpret_cast<const float4*>(mu + j);
                 const float4 q = make_float4(v.x + mu4.x, v.y + mu4.y, v.z + mu4.z, v.w + mu4.w);
                 if (dst) *reinterpret_cast<float4*>(dst + j) = q;
                 if (sq) *reinterpret_cast<float4*>(sq + j) = q;
             }
-        } else {                                                                    // samplers.py:470-472
-            for (int j = 4 * lane; j < D; j += 128) {
-                const float4 v = *reinterpret_cast<const float4*>(x0r + j);
-                *reinterpret_cast<float4*>(xr + j) = v;
-                const float4 mu4 = *reinterpret_cast<const float4*>(mu + j);
-                const float4 q = make_float4(v.x + mu4.x, v.y + mu4.y, v.z + mu4.z, v.w + mu4.w);
-                if (dst) *reinterpret_cast<float4*>(dst + j) = q;
-                if (sq) *reinterpret_cast<float4*>(sq + j) = q;
+        }
+        if (!ext4) {
+            for (int j = lane; j < D; j += 32) {
+                const float q = from[j] + mu[j];
+                if (dst) dst[j] = q;
+                if (sq) sq[j] = q;
             }
+        }
+        if (!accepted) {
             __syncwarp();
-            bigd_write_parts<NPART>(w, m, D, lane, x0r);
+            bigd_write_parts<NPART>(w, m, lane, x0r);
         }
         if (last) {
             if (lane == 0) { w.mode[m] = MD_IDLE; w.it[m] = it + 1; a.state_eprev[c] = (double)w.E_prev[m]; }
         } else {
             it += 1;
             int L = 1; float lnu = 0.f;
-            const float Kn = bigd_draw(a, c, it, lane, w.p + (size_t)m * D, &L, &lnu);      // samplers.py:431, 441, 461
+            const float Kn = bigd_draw(a, Dp, c, it, lane, w.p + (size_t)m * Dp, &L, &lnu);  // samplers.py:431, 441, 461
             if (lane == 0) { w.K_new[m] = Kn; w.L[m] = L; w.lnu[m] = lnu; w.l[m] = 0; w.it[m] = it; w.mode[m] = MD_FIRST; }
         }
     }
 }
 
-// force matrix -> split 16-bit parts, K-major rows: bp[part][n][k] = part(F[n][k] * scale); Ft[k][n] = F[n][k]
+// force matrix -> split 16-bit parts, K-major rows: bp[part][n][k] = part(F[n][k] * scale) for n, k < D, zero up to Dp;
+// Ft[k][n] = F[n][k] (row stride Dpad)
 template <int NPART>
-__global__ void bigd_split_matrix(const float* __restrict__ Ft, int D, int Dpad, float scale, uint16_t* __restrict__ bp) {
-    const long total = (long)D * (D / 2);
+__global__ void bigd_split_matrix(const float* __restrict__ Ft, int D, int Dpad, int Dp, float scale, uint16_t* __restrict__ bp) {
+    const long total = (long)Dp * (Dp / 2);
     for (long t = blockIdx.x * (long)blockDim.x + threadIdx.x; t < total; t += (long)gridDim.x * blockDim.x) {
-        const int n = (int)(t / (D / 2)), k = 2 * (int)(t % (D / 2));
+        const int n = (int)(t / (Dp / 2)), k = 2 * (int)(t % (Dp / 2));
+        const float f0 = (n < D && k < D) ? Ft[(size_t)k * Dpad + n] * scale : 0.f;
+        const float f1 = (n < D && k + 1 < D) ? Ft[(size_t)(k + 1) * Dpad + n] * scale : 0.f;
         uint32_t h[3];
-        split_pair<NPART>(Ft[(size_t)k * Dpad + n] * scale, Ft[(size_t)(k + 1) * Dpad + n] * scale, h);
+        split_pair<NPART>(f0, f1, h);
 #pragma unroll
-        for (int pt = 0; pt < NPART; ++pt) reinterpret_cast<uint32_t*>(bp + ((size_t)pt * D + n) * D)[k >> 1] = h[pt];
+        for (int pt = 0; pt < NPART; ++pt) reinterpret_cast<uint32_t*>(bp + ((size_t)pt * Dp + n) * Dp)[k >> 1] = h[pt];
     }
 }
 
@@ -710,15 +749,18 @@ size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // carve the workspace; returns the bytes needed (ws may be NULL to only size it)
 size_t carve(BigdWs& w, unsigned char* ws, long Nchain, int D, int npart, int bn) {
     const long Ncp = (Nchain + BM * kMaxCluster - 1) / (BM * kMaxCluster) * (BM * kMaxCluster);   // whole clusters of row blocks
-    const int NT = D / bn;
+    const int Dp = (D + 31) / 32 * 32;
+    const int NT = (Dp + bn - 1) / bn;
     size_t off = 0;
     auto take = [&](size_t bytes) { unsigned char* p = ws ? ws + off : nullptr; off = align_up(off + bytes, 1024); return p; };
-    w.Ncp = (int)Ncp; w.NT = NT; w.npart = npart;
-    w.xp = (uint16_t*)take((size_t)2 * npart * Ncp * D * 2);
-    w.bp = (uint16_t*)take((size_t)npart * D * D * 2);
-    w.x = (float*)take((size_t)Ncp * D * 4);
-    w.x0 = (float*)take((size_t)Ncp * D * 4);
-    w.p = (float*)take((size_t)Ncp * D * 4);
+    w.Ncp = (int)Ncp; w.NT = NT; w.npart = npart; w.Dp = Dp;
+    w.xp = (uint16_t*)take((size_t)2 * npart * Ncp * Dp * 2);
+    w.bp = (uint16_t*)take((size_t)npart * Dp * Dp * 2);
+    w.x = (float*)take((size_t)Ncp * Dp * 4);
+    w.x0 = (float*)take((size_t)Ncp * Dp * 4);
+    w.p = (float*)take((size_t)Ncp * Dp * 4);
+    w.mu = (float*)take((size_t)Dp * 4);
+    w.dt = (float*)take((size_t)Dp * 4);
     w.red = (float*)take((size_t)Ncp * NT * 2 * 2 * 4);
     w.mode = (int*)take(Ncp * 4); w.l = (int*)take(Ncp * 4); w.L = (int*)take(Ncp * 4); w.it = (int*)take(Ncp * 4); w.init = (int*)take(Ncp * 4);
     w.K_new = (float*)take(Ncp * 4); w.K0 = (float*)take(Ncp * 4); w.lnu = (float*)take(Ncp * 4); w.E_init = (float*)take(Ncp * 4);
@@ -751,8 +793,14 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
     HMC_CUDA_CHECK(cudaGetDevice(&dev));
     HMC_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     // force matrix parts (scaled to the top of the fp16 range for the fp16 split)
+    const int Dp = w.Dp;
     float scale = 1.f;
     HMC_CUDA_CHECK(cudaMemsetAsync(w.counters, 0, 64, stream));
+    // mean and step sizes, zero-padded to Dp (the caller's arrays are D_pad <= Dp long)
+    HMC_CUDA_CHECK(cudaMemsetAsync(w.mu, 0, (size_t)Dp * 4, stream));
+    HMC_CUDA_CHECK(cudaMemsetAsync(w.dt, 0, (size_t)Dp * 4, stream));
+    HMC_CUDA_CHECK(cudaMemcpyAsync(w.mu, a.target.mu, (size_t)D * 4, cudaMemcpyDeviceToDevice, stream));
+    HMC_CUDA_CHECK(cudaMemcpyAsync(w.dt, a.target.dt, (size_t)D * 4, cudaMemcpyDeviceToDevice, stream));
     if (NPART == 2) {
         unsigned int* mxd = (unsigned int*)(w.counters + 8);
         bigd_absmax<<<sms * 4, 256, 0, stream>>>((const float*)a.target.Ft, D, a.target.D_pad, mxd);
@@ -765,17 +813,17 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
         scale = ldexpf(1.f, sft);
     }
     w.binv = 1.f / scale;
-    bigd_split_matrix<NPART><<<sms * 8, 256, 0, stream>>>((const float*)a.target.Ft, D, a.target.D_pad, scale, w.bp);
+    bigd_split_matrix<NPART><<<sms * 8, 256, 0, stream>>>((const float*)a.target.Ft, D, a.target.D_pad, Dp, scale, w.bp);
     CUtensorMap mapA[2], mapS[2], mapB, mapP, mapX;
     const CUtensorMapDataType dt16 = NPART == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
     for (int b = 0; b < 2; ++b) {
-        uint16_t* xb = w.xp + (size_t)b * NPART * w.Ncp * D;
-        if (int rc = make_map(&mapA[b], dt16, 2, xb, (uint64_t)NPART * w.Ncp, D, BK, BM)) return rc;       // operand loads
-        if (int rc = make_map(&mapS[b], dt16, 2, xb, (uint64_t)NPART * w.Ncp, D, CW, 32)) return rc;       // epilogue stores
+        uint16_t* xb = w.xp + (size_t)b * NPART * w.Ncp * Dp;
+        if (int rc = make_map(&mapA[b], dt16, 2, xb, (uint64_t)NPART * w.Ncp, Dp, BK, BM)) return rc;      // operand loads
+        if (int rc = make_map(&mapS[b], dt16, 2, xb, (uint64_t)NPART * w.Ncp, Dp, CW, 32)) return rc;      // epilogue stores
     }
-    if (int rc = make_map(&mapB, dt16, 2, w.bp, (uint64_t)NPART * D, D, BK, BN / CL)) return rc;           // each CTA of a cluster loads 1 / CL of a B tile
-    if (int rc = make_map(&mapP, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.p, (uint64_t)w.Ncp, D, CW, 32)) return rc;
-    if (int rc = make_map(&mapX, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.x, (uint64_t)w.Ncp, D, CW, 32)) return rc;
+    if (int rc = make_map(&mapB, dt16, 2, w.bp, (uint64_t)NPART * Dp, Dp, BK, BN / CL)) return rc;         // each CTA of a cluster loads 1 / CL of a B tile
+    if (int rc = make_map(&mapP, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.p, (uint64_t)w.Ncp, Dp, CW, 32)) return rc;
+    if (int rc = make_map(&mapX, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.x, (uint64_t)w.Ncp, Dp, CW, 32)) return rc;
     w.wr = 0;                                                    // pass 0 reads buffer 0
     try {   // rows = chains sorted by planned passes, longest first (stable: equal plans keep the chain order); padding rows last
         bigd_plan<<<(a.Nchain + 255) / 256, 256, 0, stream>>>(a, w.plan);
@@ -815,11 +863,11 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
     const int nclusters = ntiles < max_clusters ? ntiles : max_clusters;
     const int grid = nclusters * CL;
     cfg.gridDim = dim3(grid);
-    const float* dtv = (const float*)a.target.dt;
+    const float* dtv = w.dt;
     const int Nch = a.Nchain;
     // pass n: operands from buffer n & 1, the epilogue (and the trajectory ends after it) write buffer (n + 1) & 1
     auto launch_gemm = [&](long pass) { w.wr = (int)((pass + 1) & 1);
-                                        return cudaLaunchKernelEx(&cfg, kern, mapA[pass & 1], mapB, mapP, mapX, mapS[(pass + 1) & 1], w, Nch, D, dtv); };
+                                        return cudaLaunchKernelEx(&cfg, kern, mapA[pass & 1], mapB, mapP, mapX, mapS[(pass + 1) & 1], w, Nch, Dp, dtv); };
     int* running_h = nullptr;
     HMC_CUDA_CHECK(cudaMallocHost(&running_h, 4));
     const long max_pass = (long)(a.iter_end - a.iter_begin) * (a.L_high + 1) + 8;
@@ -869,7 +917,7 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
 bool hmc_random_bigd_supported(const hmc_random_args& a, const char** why) {
     if (a.dtype != HMC_F32) { *why = "float32 only"; return false; }
     if (a.target.Mit || a.target.Pt || a.target.Lct) { *why = "identity momentum metric only"; return false; }
-    if (a.target.D < BN_MAX || (a.target.D % BN_MAX) != 0 || a.target.D > 8192) { *why = "D must be a multiple of 256 in [256, 8192]"; return false; }
+    if (a.target.D < 128 || a.target.D > 8192) { *why = "D must be in [128, 8192]"; return false; }
     if (a.iter_end <= a.iter_begin) { *why = "needs at least one iteration"; return false; }
     return true;
 }

@@ -7,7 +7,7 @@ diagnostics (utils.py:77-179) run in libhmc_b200.so through the C-ABI of include
 fallback: a target that is not a multivariate normal, or a missing CUDA library, raises.
 
 Extra keyword-only constructor arguments (defaults keep the reference behaviour):
-  dtype="float32"|"float64", seed=0 (Philox key), kernel="auto"|"generic"|"fast"|"tc", draws=None (the reference's
+  dtype="float32"|"float64", seed=0 (Philox key), kernel="auto"|"generic"|"fast"|"tc"|"bigd", draws=None (the reference's
   own draws as structured tapes, see tests/golden/make_golden.py), on_dmax="assert"|"stop" (NUTS, SURVEY H6),
   chain_id0=0 / distributed=False (chains sharded over ranks; counters and moments are all-reduced),
   iter_block=None (iterations per kernel launch), target=None (explicit ``MVNSpec`` instead of probing V/dVdq),
@@ -195,7 +195,14 @@ class sampler(object):
 
 
 class HMC_sampler(sampler):
-    """HMC sampler for multivariate-normal targets (samplers.py:297-384), CUDA backed."""
+    """HMC sampler for multivariate-normal targets (samplers.py:297-384), CUDA backed.
+
+    ``kernel`` of the random-trajectory sampler (float32, ``cov_p = I`` unless noted; "auto" picks as csrc/api.cu does):
+      "tc"       tensor-core kernel, D % 4 == 0, D <= 100 (zero-padded 100-wide tile); auto for 52 <= D <= 100
+      "bigd"     large-D GEMM path, any 128 <= D <= 8192 (padded to D rounded up to 32); auto for D % 256 == 0 and D > 1024
+      "fast"     FFMA2 kernel, 20 < D <= 128; auto where neither of the above applies
+      "generic"  warp-per-chain kernel, D <= 1024, float64 and dense ``cov_p`` too; auto for the rest
+    """
 
     def __init__(self, D, V, dVdq, Nchain=2, Niter=1000, thin_rate=1, warm_up_num=0,
                  cov_p=None, sampler_type="Fixed", L=None, global_dt=True, dt=None,
@@ -381,7 +388,8 @@ class HMC_sampler(sampler):
         a.seed = self.seed
         a.target = tgt
         a.flags = _L.FLAG_UNIFORM_DT if np.ndim(self.dt) == 0 or np.all(np.asarray(self.dt) == np.asarray(self.dt).flat[0]) else 0
-        bigd = self.dtype == "float32" and self._cov_p_identity and D >= 256 and D % 256 == 0 and self.kernel in ("auto", "bigd")
+        bigd = self.dtype == "float32" and self._cov_p_identity and 128 <= D <= 8192 and \
+            (self.kernel == "bigd" or (self.kernel == "auto" and (D % 256 == 0 or D > 1024)))     # csrc/api.cu AUTO rule
         if self.tc_precision is None:
             self.tc_precision = "fp16x2" if bigd else "bf16x3"
         if self.tc_precision == "fp16x2":
