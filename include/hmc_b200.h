@@ -42,20 +42,22 @@ enum { HMC_F32 = 0, HMC_F64 = 1 };
 /* which kernel implements the run */
 enum {
     HMC_KERNEL_AUTO = 0,    /* tensor-core kernel if it covers the run, else the large-D GEMM path (when a workspace is given and
-                               D % 256 == 0 or D > 1024), else the FFMA2 kernel, else the generic one */
-    HMC_KERNEL_GENERIC = 1, /* one warp per chain, any D <= 1024, float or double (parity workhorse) */
+                               D % 256 == 0 or D > 1024), else the FFMA2 kernel, else the generic one.  NUTS: the tensor-core kernel,
+                               else the large-D path when a workspace is given, it covers the run and D > 256, else the generic one */
+    HMC_KERNEL_GENERIC = 1, /* one warp per chain, any D <= 1024 (NUTS: D <= 256), float or double (parity workhorse) */
     HMC_KERNEL_FAST = 2,    /* FP32 FFMA2 register-tile kernel, 20 < D <= 128, identity momentum metric */
     HMC_KERNEL_TC = 3,      /* tcgen05 tensor-core kernel (bf16x3 / fp16x2 split, fp32 accumulate in TMEM), D <= 100 and a multiple of 4
                                (smaller targets run zero padded in the 100-wide tile; AUTO picks it from D = 52), identity metric */
     HMC_KERNEL_BIGD = 4     /* large D, any 128 <= D <= 8192, float32, identity metric: one tcgen05 GEMM over all chains per leapfrog
                                step, operands by TMA, the leapfrog update fused into the epilogue; works on D rounded up to 32 (the
-                               padded dimensions stay zero); needs hmc_random_args.workspace */
+                               padded dimensions stay zero); needs hmc_random_args.workspace.  NUTS too (hmc_nuts_args.workspace):
+                               the same GEMM writes the gradient rows and a step kernel advances every chain's tree by one point */
 };
 
-/* hmc_random_args.flags */
+/* hmc_random_args.flags, hmc_nuts_args.flags */
 enum {
     HMC_FLAG_UNIFORM_DT = 1, /* every entry of target.dt is equal (lets the fused kernels fold dt into constants) */
-    HMC_FLAG_TC_FP16X2 = 2   /* tensor-core kernel: the caller vouches that |q - mu| stays below ~1.6e4 and that the target's
+    HMC_FLAG_TC_FP16X2 = 2   /* tensor-core kernels (NUTS: the large-D path only): the caller vouches that |q - mu| stays below ~1.6e4 and that the target's
                                 scale is not far below 1 (no component of interest under 2^-14), which lets the gradient
                                 product use the two-part fp16 split (3 tensor passes, FP32-grade) instead of the three-part
                                 bf16 split (6 passes); a trajectory that leaves the fp16 range ends in a rejection */
@@ -157,6 +159,8 @@ int64_t hmc_random_workspace_bytes(const hmc_random_args* args);
  * find_next / retrieve_save_index / check_points / release_fast (utils.py:222-304, 367-385; closed forms).
  * Draw order per chain: one momentum per iteration; one direction coin per doubling (samplers.py:608); one
  * uniform per surviving inner step (samplers.py:748) and one per completed doubling (samplers.py:773).
+ * Kernels: the generic one (D <= 256, float or double, any metric), the tensor-core one (D = 100, float32, identity metric,
+ * d_max <= 12), the large-D path (any 128 <= D <= 8192, float32, identity metric; needs `workspace`).
  */
 typedef struct hmc_nuts_args {
     int32_t dtype;
@@ -192,9 +196,16 @@ typedef struct hmc_nuts_args {
     unsigned long long* counters; /* [4]: leapfrog steps, doublings, energy-instability rejections, d_max hits */
     int32_t* status;        /* [Nchain] bit0: d_max exceeded; may be NULL */
     int64_t* n_leapfrog;    /* [Nchain] leapfrog steps per chain (accumulated); may be NULL */
+    int32_t flags;          /* HMC_FLAG_TC_FP16X2 selects the two-part fp16 split on the large-D path (default: bf16x3) */
+    int32_t reserved0;
+    void* workspace;        /* scratch of hmc_nuts_workspace_bytes(args) bytes for HMC_KERNEL_BIGD (1024-byte aligned); NULL otherwise */
+    int64_t workspace_bytes;
 } hmc_nuts_args;
 
 int hmc_nuts_run(const hmc_nuts_args* args, void* cuda_stream);
+/* bytes of hmc_nuts_args.workspace the large-D path needs for this configuration: non-zero exactly for the runs it covers
+   (float32, identity metric, 128 <= D <= 8192), whatever kernel is asked for; 0 otherwise.  Depends on Nchain and D only. */
+int64_t hmc_nuts_workspace_bytes(const hmc_nuts_args* args);
 
 /*
  * Diagnostics: replace utils.convergence_stats / utils.variogram (utils.py:77-179) as two HBM-bound

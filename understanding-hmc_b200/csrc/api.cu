@@ -24,6 +24,9 @@ size_t hmc_random_bigd_workspace(const hmc_random_args& a);
 int hmc_nuts_run_generic(const hmc_nuts_args& a, cudaStream_t stream);
 int hmc_nuts_run_tc(const hmc_nuts_args& a, cudaStream_t stream);
 bool hmc_nuts_tc_supported(const hmc_nuts_args& a, const char** why);
+int hmc_nuts_run_bigd(const hmc_nuts_args& a, cudaStream_t stream);
+bool hmc_nuts_bigd_supported(const hmc_nuts_args& a, const char** why);
+size_t hmc_nuts_bigd_workspace(const hmc_nuts_args& a);
 
 extern "C" int hmc_version(void) { return HMC_B200_VERSION; }
 extern "C" const char* hmc_last_error_string(void) { return g_err; }
@@ -125,7 +128,27 @@ extern "C" int hmc_nuts_run(const hmc_nuts_args* args, void* cuda_stream) {
                 "dense momentum metric: target.Pt, Mit and Lct must be given together");
     const char* why = "";
     int kernel = a.kernel;
-    if (kernel == HMC_KERNEL_AUTO) kernel = hmc_nuts_tc_supported(a, &why) ? HMC_KERNEL_TC : HMC_KERNEL_GENERIC;
+    // tensor-core kernel where it applies, else the large-D GEMM path above the generic kernel's D <= 256, else the generic kernel
+    if (kernel == HMC_KERNEL_AUTO)
+        kernel = hmc_nuts_tc_supported(a, &why) ? HMC_KERNEL_TC
+                 : (a.target.D > 256 && a.workspace && hmc_nuts_bigd_supported(a, &why)) ? HMC_KERNEL_BIGD : HMC_KERNEL_GENERIC;
+    if (kernel == HMC_KERNEL_BIGD) {
+        if (!hmc_nuts_bigd_supported(a, &why)) {
+            hmc_set_error("large-D NUTS kernel does not cover this configuration: %s", why);
+            return HMC_E_UNSUPPORTED;
+        }
+        return hmc_nuts_run_bigd(a, (cudaStream_t)cuda_stream);
+    }
+    if (kernel == HMC_KERNEL_GENERIC && a.target.D > 256) {
+        // (the generic kernel stops at D = 256; above it only the large-D path runs NUTS)
+        if (!hmc_nuts_bigd_supported(a, &why)) {
+            hmc_set_error("NUTS above D = 256 runs on the large-D path only, which does not cover this configuration: %s (got D = %d)",
+                          why, a.target.D);
+            return HMC_E_UNSUPPORTED;
+        }
+        hmc_set_error("NUTS above D = 256 runs on the large-D path only: it needs hmc_nuts_args.workspace (hmc_nuts_workspace_bytes)");
+        return HMC_E_UNSUPPORTED;
+    }
     if (kernel == HMC_KERNEL_TC) {
         if (!hmc_nuts_tc_supported(a, &why)) {
             hmc_set_error("tensor-core NUTS kernel does not cover this configuration: %s", why);
@@ -134,10 +157,19 @@ extern "C" int hmc_nuts_run(const hmc_nuts_args* args, void* cuda_stream) {
         return hmc_nuts_run_tc(a, (cudaStream_t)cuda_stream);
     }
     if (kernel != HMC_KERNEL_GENERIC) {
-        hmc_set_error("NUTS: kernel must be auto, generic or tc");
+        hmc_set_error("NUTS: kernel must be auto, generic, tc or bigd");
         return HMC_E_BADARG;
     }
     return hmc_nuts_run_generic(a, (cudaStream_t)cuda_stream);
+}
+
+extern "C" int64_t hmc_nuts_workspace_bytes(const hmc_nuts_args* args) {
+    const char* why = "";
+    if (!args) return 0;
+    hmc_nuts_args a = *args;                        // (the iteration range of the launch does not matter for the size)
+    a.iter_begin = 0; a.iter_end = 1;
+    if (!hmc_nuts_bigd_supported(a, &why)) return 0;
+    return (int64_t)hmc_nuts_bigd_workspace(a);
 }
 
 // ---------------------------------------------------------------------------------------------------------

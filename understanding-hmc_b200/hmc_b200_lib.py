@@ -19,7 +19,8 @@ HMC_OK, HMC_E_BADARG, HMC_E_UNSUPPORTED, HMC_E_CUDA, HMC_E_DMAX = 0, 1, 2, 3, 4
 
 EXPORTS = ["hmc_random_run", "hmc_nuts_run", "hmc_diag_moments", "hmc_diag_variogram", "hmc_diag_short_series", "hmc_philox_draws",
            "hmc_ffma_peak", "hmc_version", "hmc_last_error_string", "hmc_start_pts", "hmc_summary_moments", "hmc_summary_hist",
-           "hmc_summary_select", "hmc_random_workspace_bytes", "hmc_diag_variogram_all", "hmc_diag_variogram_all_workspace_bytes", "hmc_leap_frog"]
+           "hmc_summary_select", "hmc_random_workspace_bytes", "hmc_diag_variogram_all", "hmc_diag_variogram_all_workspace_bytes", "hmc_leap_frog",
+           "hmc_nuts_workspace_bytes"]
 
 
 class Target(C.Structure):
@@ -48,7 +49,8 @@ class NutsArgs(C.Structure):
                 ("u_tape", C.c_void_p), ("tape_dir_stride", C.c_int32), ("tape_u_stride", C.c_int32),
                 ("q_chain", C.c_void_p), ("E_chain", C.c_void_p), ("dE_chain", C.c_void_p), ("state_q", C.c_void_p),
                 ("state_eprev", C.c_void_p), ("scratch", C.c_void_p), ("counters", C.c_void_p), ("status", C.c_void_p),
-                ("n_leapfrog", C.c_void_p)]
+                ("n_leapfrog", C.c_void_p), ("flags", C.c_int32), ("reserved0", C.c_int32), ("workspace", C.c_void_p),
+                ("workspace_bytes", C.c_int64)]
 
 
 _lib = None
@@ -70,6 +72,8 @@ def load():
     lib.hmc_random_workspace_bytes.restype = C.c_int64
     lib.hmc_nuts_run.argtypes = [C.POINTER(NutsArgs), C.c_void_p]
     lib.hmc_nuts_run.restype = C.c_int
+    lib.hmc_nuts_workspace_bytes.argtypes = [C.POINTER(NutsArgs)]
+    lib.hmc_nuts_workspace_bytes.restype = C.c_int64
     lib.hmc_diag_moments.argtypes = [C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int64, C.c_void_p,
                                      C.c_void_p]
     lib.hmc_diag_moments.restype = C.c_int

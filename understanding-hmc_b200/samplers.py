@@ -12,9 +12,9 @@ Extra keyword-only constructor arguments (defaults keep the reference behaviour)
   chain_id0=0 / distributed=False (chains sharded over ranks; counters and moments are all-reduced),
   iter_block=None (iterations per kernel launch), target=None (explicit ``MVNSpec`` instead of probing V/dVdq),
   tc_precision="bf16x3"|"fp16x2" (split of the tensor-core gradient product: three bf16 parts / six tensor passes -- the
-  default of the D = 100 kernel -- or two fp16 parts / three passes -- the default of the large-D GEMM path; at D = 100,
-  rho = 0.95 fp16x2 is 10 % faster at 3x the trajectory error, see DESIGN 4.0; a D = 100 run whose start points leave the
-  fp16 range repeats itself with bf16x3).
+  default of the D = 100 kernel and of NUTS on the large-D path -- or two fp16 parts / three passes -- the default of the
+  large-D GEMM path of the random-trajectory sampler; at D = 100, rho = 0.95 fp16x2 is 10 % faster at 3x the trajectory error,
+  see DESIGN 4.0; a D = 100 run whose start points leave the fp16 range repeats itself with bf16x3).
 """
 import os
 
@@ -202,6 +202,12 @@ class HMC_sampler(sampler):
       "bigd"     large-D GEMM path, any 128 <= D <= 8192 (padded to D rounded up to 32); auto for D % 256 == 0 and D > 1024
       "fast"     FFMA2 kernel, 20 < D <= 128; auto where neither of the above applies
       "generic"  warp-per-chain kernel, D <= 1024, float64 and dense ``cov_p`` too; auto for the rest
+
+    ``kernel`` of the NUTS sampler (reported as ``nuts_kernel``):
+      "tc"       tensor-core kernel, D = 100, float32, ``cov_p = I``, d_max <= 12; auto there
+      "bigd"     large-D GEMM path, any 128 <= D <= 8192, float32, ``cov_p = I`` (bf16x3 split unless tc_precision="fp16x2");
+                 auto for D > 256
+      "generic"  warp-per-chain kernel, D <= 256, float64 and dense ``cov_p`` too; auto for the rest
     """
 
     def __init__(self, D, V, dVdq, Nchain=2, Niter=1000, thin_rate=1, warm_up_num=0,
@@ -508,8 +514,13 @@ class HMC_sampler(sampler):
         a.dtype = _L.HMC_F32 if self.dtype == "float32" else _L.HMC_F64
         a.kernel = _L.KERNELS[self.kernel]
         # (mirror of the library's AUTO rule, for reports: csrc/api.cu hmc_nuts_run)
-        self.nuts_kernel = "tc" if (self.kernel in ("auto", "tc") and self.dtype == "float32" and D == 100 and self.d_max <= 12) \
-            else "generic"
+        bigd_ok = self.dtype == "float32" and self._cov_p_identity and 128 <= D <= 8192
+        if self.kernel in ("auto", "tc") and self.dtype == "float32" and D == 100 and self.d_max <= 12:
+            self.nuts_kernel = "tc"
+        elif bigd_ok and (self.kernel == "bigd" or (self.kernel == "auto" and D > 256)):
+            self.nuts_kernel = "bigd"
+        else:
+            self.nuts_kernel = "generic"
         a.Nchain, a.d_max, a.chain_id0 = Nc, int(self.d_max), self.chain_id0
         a.Niter, a.warm_up_num, a.thin_rate = self.Niter, self.warm_up_num, self.thin_rate
         a.on_dmax = 0 if self.on_dmax == "assert" else 1
@@ -527,11 +538,24 @@ class HMC_sampler(sampler):
         a.state_q, a.state_eprev = state_q.data_ptr(), state_e.data_ptr()
         a.scratch, a.counters, a.status, a.n_leapfrog = scratch.data_ptr(), counters.data_ptr(), status.data_ptr(), \
             nleap.data_ptr()
+        if self.nuts_kernel == "bigd":            # large-D GEMM path: its scratch (split operands, x / p / gradient rows, chain states)
+            if self.tc_precision is None:
+                self.tc_precision = "bf16x3"      # tree decisions are sign tests and near-ties: the split without fp16's V bias
+            if self.tc_precision == "fp16x2":
+                # two-part fp16 split; needs a target whose scale is not far below 1 (fp16 subnormals), as for Random
+                if float(np.min(1.0 / np.sqrt(np.abs(np.diag(self.target.P))))) < 2.0 ** -10:
+                    self.tc_precision = "bf16x3"
+                else:
+                    a.flags |= _L.FLAG_TC_FP16X2
+            nbytes = int(lib.hmc_nuts_workspace_bytes(a))
+            ws = torch.empty((nbytes + 1024,), dtype=torch.uint8, device=dev)
+            a.workspace = (ws.data_ptr() + 1023) // 1024 * 1024
+            a.workspace_bytes = nbytes
         stream = _L.current_stream_ptr()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         if verbose:
-            print("Running %d NUTS chains x %d iterations on %s (%s)" %
-                  (Nc, self.Niter, torch.cuda.get_device_name(dev), self.dtype))
+            print("Running %d NUTS chains x %d iterations on %s (%s, kernel=%s)" %
+                  (Nc, self.Niter, torch.cuda.get_device_name(dev), self.dtype, self.nuts_kernel))
         ev0.record()
         for (b, e) in self._blocks():
             a.iter_begin, a.iter_end = b, e
