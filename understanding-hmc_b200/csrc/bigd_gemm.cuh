@@ -5,12 +5,16 @@
 //   EPI_GRAD      the gradient rows themselves, G[Ncp][Dp] float32 by TMA store (the NUTS step runs as its own kernel)
 // W is the caller's workspace: it provides tile_active (row blocks with a chain that takes part), mode (per row: MD_IDLE rows
 // need no gradient), Ncp, NT and binv (2^-s of the fp16 split's matrix scaling); the leapfrog epilogue also uses red.
-// Also here: the split of a pair of floats into 16-bit parts, the split of the force matrix, the tensor-map helper.
+// Also here: the split of a pair of floats into 16-bit parts, the split of the force matrix, the tensor-map helper, and what the
+// two samplers do alike around the GEMM (bottom of the file): coverage, workspace geometry and carving, the target as GEMM
+// operands, the launch configuration, the choice of split and cluster, the look at the running chains, and the momentum-row and
+// split-position helpers of their own kernels.
 #pragma once
 #include "hmc_common.cuh"
 #include <cuda.h>
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
+#include <cstdlib>
 
 namespace {
 
@@ -499,5 +503,175 @@ constexpr size_t gemm_smem_bytes() {
 }
 static_assert(gemm_smem_bytes<2, 256, 32, (NEPI == 4 ? 3 : 2)>() <= 232448 && gemm_smem_bytes<3, 128, 32, 2>() <= 232448,
               "shared memory of the large-D GEMM exceeds 227 KB");
+
+// =====================================================================================================================
+// What the two samplers do alike around the GEMM.  Each keeps its own workspace struct (the fields the GEMM reads are named
+// alike), kernels and pass loop; `name` is the path's name in error messages.
+// =====================================================================================================================
+
+// the runs the large-D path covers (the `why` strings end up in error messages)
+bool bigd_covers(int dtype, const hmc_target& t, int iter_begin, int iter_end, const char** why) {
+    if (dtype != HMC_F32) { *why = "float32 only"; return false; }
+    if (t.Mit || t.Pt || t.Lct) { *why = "identity momentum metric only"; return false; }
+    if (t.D < 128 || t.D > 8192) { *why = "D must be in [128, 8192]"; return false; }
+    if (iter_end <= iter_begin) { *why = "needs at least one iteration"; return false; }
+    return true;
+}
+
+// Workspace geometry and carving: Ncp rows (the chains padded to whole clusters of row blocks), Dp = D rounded up to whole K
+// stages (32) columns in NT column tiles of width bn; take() hands out the arrays one after the other, 1024-byte aligned (with a
+// NULL base it only sizes them)
+struct BigdCarve {
+    unsigned char* base;
+    long Ncp;
+    int Dp, NT;
+    size_t off = 0;
+    BigdCarve(unsigned char* ws, long Nchain, int D, int bn)
+        : base(ws), Ncp((Nchain + BM * kMaxCluster - 1) / (BM * kMaxCluster) * (BM * kMaxCluster)), Dp((D + 31) / 32 * 32),
+          NT((Dp + bn - 1) / bn) {}
+    void* take(size_t bytes) { unsigned char* p = base ? base + off : nullptr; off = align_up(off + bytes, 1024); return p; }
+};
+
+int bigd_check_workspace(const void* ws, int64_t bytes, size_t need, const char* name, const char* sizer) {
+    if (ws && (size_t)bytes >= need) return HMC_OK;
+    hmc_set_error("%s needs a workspace of %zu bytes (%s)", name, need, sizer);
+    return HMC_E_BADARG;
+}
+
+template <int NPART>
+constexpr CUtensorMapDataType bigd_dt16() { return NPART == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16; }
+
+// The target as the GEMM's inputs: clears w.counters (word 8 is the abs-max scratch), mu and dt zero-padded to Dp (the caller's
+// arrays are D_pad <= Dp long), the force matrix split into w.bp -- for the fp16 split scaled by 2^s to the top of the fp16 range,
+// which needs the matrix's abs-max on the host (the one wait for the device here) -- w.binv = 2^-s, and the map of the B operand
+// (each CTA of a cluster loads 1 / CL of a B tile)
+template <int NPART, int BN, int CL, int BK, class W>
+int bigd_target_operands(const hmc_target& t, W& w, int sms, cudaStream_t stream, CUtensorMap* mapB) {
+    const int D = t.D, Dp = w.Dp;
+    HMC_CUDA_CHECK(cudaMemsetAsync(w.counters, 0, 64, stream));
+    HMC_CUDA_CHECK(cudaMemsetAsync(w.mu, 0, (size_t)Dp * 4, stream));
+    HMC_CUDA_CHECK(cudaMemsetAsync(w.dt, 0, (size_t)Dp * 4, stream));
+    HMC_CUDA_CHECK(cudaMemcpyAsync(w.mu, t.mu, (size_t)D * 4, cudaMemcpyDeviceToDevice, stream));
+    HMC_CUDA_CHECK(cudaMemcpyAsync(w.dt, t.dt, (size_t)D * 4, cudaMemcpyDeviceToDevice, stream));
+    float scale = 1.f;
+    if (NPART == 2) {
+        unsigned int* mxd = (unsigned int*)(w.counters + 8);
+        bigd_absmax<<<sms * 4, 256, 0, stream>>>((const float*)t.Ft, D, t.D_pad, mxd);
+        unsigned int mx = 0;
+        HMC_CUDA_CHECK(cudaMemcpyAsync(&mx, mxd, 4, cudaMemcpyDeviceToHost, stream));
+        HMC_CUDA_CHECK(cudaStreamSynchronize(stream));
+        const int e = (int)(mx >> 23) - 127;
+        int sft = (mx == 0u || e < -100) ? 0 : 14 - e;
+        sft = sft > 100 ? 100 : (sft < -100 ? -100 : sft);
+        scale = ldexpf(1.f, sft);
+    }
+    w.binv = 1.f / scale;
+    bigd_split_matrix<NPART><<<sms * 8, 256, 0, stream>>>((const float*)t.Ft, D, t.D_pad, Dp, scale, w.bp);
+    return make_map(mapB, bigd_dt16<NPART>(), 2, w.bp, (uint64_t)NPART * Dp, Dp, BK, BN / CL);
+}
+
+// Launch configuration of the GEMM kernel: persistent clusters of CL CTAs, as many as are resident at once (a GPC holds whole
+// clusters only), never more than the nwork work items.  cfg points to attr for the cluster attribute.
+template <class K>
+int bigd_launch_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute& attr, K kern, int CL, int nwork, size_t smem, int sms,
+                       cudaStream_t stream, const char* name) {
+    HMC_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attr.id = cudaLaunchAttributeClusterDimension;
+    attr.val.clusterDim.x = CL; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+    cfg = {};
+    cfg.gridDim = dim3(sms / CL * CL); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+    cfg.attrs = &attr; cfg.numAttrs = 1;
+    int max_clusters = sms / CL;
+    if (CL > 1) {
+        int nc = 0;
+        HMC_CUDA_CHECK(cudaOccupancyMaxActiveClusters(&nc, kern, &cfg));
+        if (nc < 1) { hmc_set_error("%s: no cluster of %d CTAs fits on this device", name, CL); return HMC_E_CUDA; }
+        if (nc < max_clusters) max_clusters = nc;
+    }
+    cfg.gridDim = dim3((nwork < max_clusters ? nwork : max_clusters) * CL);
+    return HMC_OK;
+}
+
+template <int NPART_, int BN_, int CL_, int BK_, int STAGES_>
+struct BigdVariant { static constexpr int NPART = NPART_, BN = BN_, CL = CL_, BK = BK_, STAGES = STAGES_; };
+
+// The GEMM variant of a run, handed to the path's runner as run(BigdVariant<...>{}): the two-part fp16 split on 256-column tiles
+// when the caller sets HMC_FLAG_TC_FP16X2, else the three-part bf16 split on 128-column tiles (shared memory); HMC_B200_TC_PREC
+// overrides the flag ('f...': fp16x2, else bf16x3).  Clusters of two row blocks share the column block's B tile by TMA multicast
+// (HMC_B200_BIGD_CLUSTER=1: plain CTAs).  With the first epilogue the cluster changed nothing (the kernel was bound by its
+// epilogue); with the TMA epilogue it is worth 8 % of a full pass at fp16x2 and 19 % of a bf16x3 run (DESIGN 4.5).
+template <class Run>
+int bigd_run_variant(int flags, Run run) {
+    bool fp16 = (flags & HMC_FLAG_TC_FP16X2) != 0;
+    if (const char* e = getenv("HMC_B200_TC_PREC")) fp16 = (e[0] == 'f');
+    int cl = 2;
+    if (const char* e = getenv("HMC_B200_BIGD_CLUSTER")) cl = atoi(e);
+    constexpr int ST2 = NEPI == 4 ? 3 : 2;           // operand stages that fit beside the epilogue buffers
+    if (fp16) return cl == 2 ? run(BigdVariant<2, 256, 2, 32, ST2>{}) : run(BigdVariant<2, 256, 1, 32, ST2>{});
+    return cl == 2 ? run(BigdVariant<3, 128, 2, 32, 2>{}) : run(BigdVariant<3, 128, 1, 32, 2>{});
+}
+
+// The host's look at the running chains: counters[2] (running chains after the last pass) read through a pinned word
+struct BigdRunning {
+    int* h = nullptr;
+    int alloc() { HMC_CUDA_CHECK(cudaMallocHost(&h, 4)); return HMC_OK; }
+    ~BigdRunning() { if (h) cudaFreeHost(h); }
+    int read(const int* counters, cudaStream_t stream) {          // -1 on a CUDA error
+        if (cudaMemcpyAsync(h, counters + 2, 4, cudaMemcpyDeviceToHost, stream) != cudaSuccess ||
+            cudaStreamSynchronize(stream) != cudaSuccess) return -1;
+        return *h;
+    }
+};
+
+// the result of a pass loop: rc as the loop left it (HMC_E_CUDA: a launch or a look failed), else a launch error since
+int bigd_loop_result(int rc, const char* name) {
+    if (rc == HMC_OK) HMC_CUDA_CHECK(cudaGetLastError());
+    else hmc_set_error("%s: CUDA error in the pass loop: %s", name, cudaGetErrorString(cudaGetLastError()));
+    return rc;
+}
+
+// Momentum row of one chain and iteration, by one warp: normal j is component j & 3 of hmc_normal4(seed, gid, iter, j >> 2) -- or
+// element j of the injected tape row when one is given -- for j < D, zero from D on; stored to the Dp-wide row prow when one is
+// given.  Returns this lane's sum of the squares.  Lane l takes the tape elements l, l + 32, ..., and the Philox slots l, l + 32,
+// ... below `wrap`, then from `wrap` on (the partly used last slot when D % 4 != 0, then the padding) wrap + l, wrap + l + 32, ...
+// That order decides the last bit of the float sums: Random passes wrap = D / 4, NUTS 0, as their results have always had it.
+__device__ __forceinline__ float bigd_momentum(const double* tape, uint64_t seed, uint64_t gid, int iter, int D, int Dp, int lane,
+                                               float* prow, int wrap) {
+    float s = 0.f;
+    if (tape) {
+        for (int j = lane; j < Dp; j += 32) { const float v = j < D ? (float)tape[j] : 0.f; if (prow) prow[j] = v; s = fmaf(v, v, s); }
+    } else {
+        for (int sl = lane; sl < wrap; sl += 32) {
+            const float4 z = hmc_normal4(seed, gid, (uint32_t)iter, (uint32_t)sl);
+            if (prow) *reinterpret_cast<float4*>(prow + 4 * sl) = z;
+            s += z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w;
+        }
+        for (int sl = wrap + lane; sl < Dp / 4; sl += 32) {
+            float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (4 * sl < D) {
+                z = hmc_normal4(seed, gid, (uint32_t)iter, (uint32_t)sl);
+                if (4 * sl + 3 >= D) z.w = 0.f;
+                if (4 * sl + 2 >= D) z.z = 0.f;
+                if (4 * sl + 1 >= D) z.y = 0.f;
+            }
+            if (prow) *reinterpret_cast<float4*>(prow + 4 * sl) = z;
+            s += z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w;
+        }
+    }
+    __syncwarp();                              // (the row is read with other lane-to-element maps afterwards)
+    return s;
+}
+
+// the split position of row m (Dp wide) as the NPART 16-bit parts of the A operand: xp[part][Ncp][Dp] from the buffer base xp
+template <int NPART>
+__device__ __forceinline__ void bigd_write_parts(uint16_t* xp, int Ncp, int Dp, long m, int lane, const float* xr) {
+    __syncwarp();                              // xr was written with another lane-to-element map
+    for (int j = 2 * lane; j < Dp; j += 64) {
+        uint32_t h[3];
+        split_pair<NPART>(xr[j], xr[j + 1], h);
+#pragma unroll
+        for (int pt = 0; pt < NPART; ++pt) reinterpret_cast<uint32_t*>(xp + ((size_t)pt * Ncp + m) * Dp)[j >> 1] = h[pt];
+    }
+}
 
 }  // namespace

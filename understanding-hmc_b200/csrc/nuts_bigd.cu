@@ -21,7 +21,8 @@
 //                  sampling, live and boundary rows, end of a doubling, next coin, then the first half kick and drift of the next
 //                  step; writes x, p and the split position (the next pass's A operand)
 // Rows are chains in their own order (tree sizes are not known in advance, so there is no sort); a row block whose chains have
-// all finished leaves the GEMM through tile_active.  The host looks at the number of running chains every 8 passes.
+// all finished leaves the GEMM through tile_active.  The host looks at the number of running chains every 8 passes.  The set-up
+// around the GEMM and the momentum-row / split-position helpers are shared with random_bigd.cu (bigd_gemm.cuh).
 //
 // State: the check-point stack and the live / boundary rows are the caller's scratch ([Nchain + 128][2 (d_max+1) + 7][D_pad],
 // the layout of nuts_generic.cu, cursors of the injected streams in row R + 6).  Everything the GEMM touches is in the workspace,
@@ -71,38 +72,8 @@ __device__ __forceinline__ double nb_unif(uint32_t w) { return ((double)(w >> 8)
 // nuts_generic.cu: normal j of the row is component j & 3 of hmc_normal4(seed, chain, iteration, j >> 2).
 __device__ float nb_draw(const hmc_nuts_args& a, int Dp, long m, int iter, int lane, float* pr) {
     const int D = a.target.D;
-    float s = 0.f;
-    if (a.p_tape) {
-        const double* src = a.p_tape + ((size_t)m * (a.Niter + 1) + iter) * D;
-        for (int j = lane; j < Dp; j += 32) { const float v = j < D ? (float)src[j] : 0.f; pr[j] = v; s = fmaf(v, v, s); }
-    } else {
-        const uint64_t gid = (uint64_t)(a.chain_id0 + m);
-        for (int sl = lane; sl < Dp / 4; sl += 32) {
-            float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (4 * sl < D) {
-                z = hmc_normal4(a.seed, gid, (uint32_t)iter, (uint32_t)sl);
-                if (4 * sl + 3 >= D) z.w = 0.f;
-                if (4 * sl + 2 >= D) z.z = 0.f;
-                if (4 * sl + 1 >= D) z.y = 0.f;
-            }
-            *reinterpret_cast<float4*>(pr + 4 * sl) = z;
-            s += z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w;
-        }
-    }
-    __syncwarp();                              // (the row is read with other lane-to-element maps afterwards)
-    return warp_sum<float>(s);
-}
-
-template <int NPART>
-__device__ __forceinline__ void nb_write_parts(const NbWs& w, long m, int lane, const float* xr) {
-    const int Dp = w.Dp;
-    __syncwarp();                              // xr was written with another lane-to-element map
-    for (int j = 2 * lane; j < Dp; j += 64) {
-        uint32_t h[3];
-        split_pair<NPART>(xr[j], xr[j + 1], h);
-#pragma unroll
-        for (int pt = 0; pt < NPART; ++pt) reinterpret_cast<uint32_t*>(w.xp + ((size_t)pt * w.Ncp + m) * Dp)[j >> 1] = h[pt];
-    }
+    const double* tape = a.p_tape ? a.p_tape + ((size_t)m * (a.Niter + 1) + iter) * D : nullptr;
+    return warp_sum<float>(bigd_momentum(tape, a.seed, (uint64_t)(a.chain_id0 + m), iter, D, Dp, lane, pr, 0));
 }
 
 // chain start (samplers.py:548-555) or resume from state_q / state_eprev / the cursors: one warp per row
@@ -115,7 +86,7 @@ __global__ void __launch_bounds__(128) nuts_bigd_init(hmc_nuts_args a, NbWs w) {
     float* pr = w.p + (size_t)m * Dp;
     if (m >= a.Nchain) {                                                    // padding rows of the last row blocks
         for (int j = lane; j < Dp; j += 32) { xr[j] = 0.f; pr[j] = 0.f; }
-        nb_write_parts<NPART>(w, m, lane, xr);
+        bigd_write_parts<NPART>(w.xp, w.Ncp, Dp, m, lane, xr);
         if (lane == 0) { w.mode[m] = MD_IDLE; w.ch[m].ph = NB_IDLE; }
         return;
     }
@@ -127,8 +98,7 @@ __global__ void __launch_bounds__(128) nuts_bigd_init(hmc_nuts_args a, NbWs w) {
         if (fresh && j < D) ((float*)a.q_chain)[(size_t)m * Lc * D + j] = v;           // samplers.py:548
         xr[j] = v - w.mu[j];
     }
-    __syncwarp();
-    nb_write_parts<NPART>(w, m, lane, xr);
+    bigd_write_parts<NPART>(w.xp, w.Ncp, Dp, m, lane, xr);
     const int R = 2 * (a.d_max + 1);
     const long long* cur = reinterpret_cast<const long long*>((const float*)a.scratch + ((size_t)m * (R + 7) + R + 6) * Dpad);
     nb_draw(a, Dp, m, fresh ? 0 : a.iter_begin + 1, lane, pr);                      // samplers.py:549 / 565
@@ -421,7 +391,7 @@ __global__ void __launch_bounds__(32 * NB_WARPS) nuts_bigd_step(hmc_nuts_args a,
             }
             new_x = true;
         }
-        if (new_x) nb_write_parts<NPART>(w, m, lane, xr);
+        if (new_x) bigd_write_parts<NPART>(w.xp, w.Ncp, Dp, m, lane, xr);
         c.ph = next_ph;
         if (lane == 0) { w.ch[m] = c; w.mode[m] = next_ph == NB_IDLE ? MD_IDLE : MD_MID; }
         alive += next_ph != NB_IDLE;
@@ -439,93 +409,54 @@ __global__ void __launch_bounds__(32 * NB_WARPS) nuts_bigd_step(hmc_nuts_args a,
 }
 
 size_t carve(NbWs& w, unsigned char* ws, long Nchain, int D, int npart, int bn) {
-    const long Ncp = (Nchain + BM * kMaxCluster - 1) / (BM * kMaxCluster) * (BM * kMaxCluster);   // whole clusters of row blocks
-    const int Dp = (D + 31) / 32 * 32;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { unsigned char* p = ws ? ws + off : nullptr; off = align_up(off + bytes, 1024); return p; };
-    w.Ncp = (int)Ncp; w.NT = (Dp + bn - 1) / bn; w.Dp = Dp;
-    w.xp = (uint16_t*)take((size_t)npart * Ncp * Dp * 2);
-    w.bp = (uint16_t*)take((size_t)npart * Dp * Dp * 2);
-    w.x = (float*)take((size_t)Ncp * Dp * 4);
-    w.p = (float*)take((size_t)Ncp * Dp * 4);
-    w.g = (float*)take((size_t)Ncp * Dp * 4);
-    w.mu = (float*)take((size_t)Dp * 4);
-    w.dt = (float*)take((size_t)Dp * 4);
-    w.ch = (NbChain*)take((size_t)Ncp * sizeof(NbChain));
-    w.mode = (int*)take(Ncp * 4);
-    w.tile_active = (int*)take((Ncp / BM) * 4);
-    w.counters = (int*)take(64);
-    w.grads = (unsigned long long*)take(8);
-    return off;
+    BigdCarve c(ws, Nchain, D, bn);
+    const long Ncp = c.Ncp;
+    const int Dp = c.Dp;
+    w.Ncp = (int)Ncp; w.NT = c.NT; w.Dp = Dp;
+    w.xp = (uint16_t*)c.take((size_t)npart * Ncp * Dp * 2);
+    w.bp = (uint16_t*)c.take((size_t)npart * Dp * Dp * 2);
+    w.x = (float*)c.take((size_t)Ncp * Dp * 4);
+    w.p = (float*)c.take((size_t)Ncp * Dp * 4);
+    w.g = (float*)c.take((size_t)Ncp * Dp * 4);
+    w.mu = (float*)c.take((size_t)Dp * 4);
+    w.dt = (float*)c.take((size_t)Dp * 4);
+    w.ch = (NbChain*)c.take((size_t)Ncp * sizeof(NbChain));
+    w.mode = (int*)c.take(Ncp * 4);
+    w.tile_active = (int*)c.take((Ncp / BM) * 4);
+    w.counters = (int*)c.take(64);
+    w.grads = (unsigned long long*)c.take(8);
+    return c.off;
 }
+
+constexpr const char* kName = "large-D NUTS kernel";
 
 template <int NPART, int BN, int CL, int BK, int STAGES>
 int run_nuts_bigd(const hmc_nuts_args& a, cudaStream_t stream) {
     const int D = a.target.D;
     NbWs w;
     const size_t need = carve(w, (unsigned char*)a.workspace, a.Nchain, D, NPART, BN);
-    if (!a.workspace || (size_t)a.workspace_bytes < need) {
-        hmc_set_error("large-D NUTS kernel needs a workspace of %zu bytes (hmc_nuts_workspace_bytes)", need);
-        return HMC_E_BADARG;
-    }
+    if (int rc = bigd_check_workspace(a.workspace, a.workspace_bytes, need, kName, "hmc_nuts_workspace_bytes")) return rc;
     int dev = 0, sms = 0;
     HMC_CUDA_CHECK(cudaGetDevice(&dev));
     HMC_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const int Dp = w.Dp;
-    HMC_CUDA_CHECK(cudaMemsetAsync(w.counters, 0, 64, stream));
     HMC_CUDA_CHECK(cudaMemsetAsync(w.grads, 0, 8, stream));
-    // mean and step sizes, zero-padded to Dp (the caller's arrays are D_pad <= Dp long)
-    HMC_CUDA_CHECK(cudaMemsetAsync(w.mu, 0, (size_t)Dp * 4, stream));
-    HMC_CUDA_CHECK(cudaMemsetAsync(w.dt, 0, (size_t)Dp * 4, stream));
-    HMC_CUDA_CHECK(cudaMemcpyAsync(w.mu, a.target.mu, (size_t)D * 4, cudaMemcpyDeviceToDevice, stream));
-    HMC_CUDA_CHECK(cudaMemcpyAsync(w.dt, a.target.dt, (size_t)D * 4, cudaMemcpyDeviceToDevice, stream));
-    // force matrix parts (scaled to the top of the fp16 range for the fp16 split), as random_bigd.cu
-    float scale = 1.f;
-    if (NPART == 2) {
-        unsigned int* mxd = (unsigned int*)(w.counters + 8);
-        bigd_absmax<<<sms * 4, 256, 0, stream>>>((const float*)a.target.Ft, D, a.target.D_pad, mxd);
-        unsigned int mx = 0;
-        HMC_CUDA_CHECK(cudaMemcpyAsync(&mx, mxd, 4, cudaMemcpyDeviceToHost, stream));
-        HMC_CUDA_CHECK(cudaStreamSynchronize(stream));
-        const int e = (int)(mx >> 23) - 127;
-        int sft = (mx == 0u || e < -100) ? 0 : 14 - e;
-        sft = sft > 100 ? 100 : (sft < -100 ? -100 : sft);
-        scale = ldexpf(1.f, sft);
-    }
-    w.binv = 1.f / scale;
-    bigd_split_matrix<NPART><<<sms * 8, 256, 0, stream>>>((const float*)a.target.Ft, D, a.target.D_pad, Dp, scale, w.bp);
     CUtensorMap mapA, mapB, mapG;
-    const CUtensorMapDataType dt16 = NPART == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    if (int rc = make_map(&mapA, dt16, 2, w.xp, (uint64_t)NPART * w.Ncp, Dp, BK, BM)) return rc;          // operand loads
-    if (int rc = make_map(&mapB, dt16, 2, w.bp, (uint64_t)NPART * Dp, Dp, BK, BN / CL)) return rc;        // 1 / CL of a B tile per CTA
+    if (int rc = bigd_target_operands<NPART, BN, CL, BK>(a.target, w, sms, stream, &mapB)) return rc;
+    if (int rc = make_map(&mapA, bigd_dt16<NPART>(), 2, w.xp, (uint64_t)NPART * w.Ncp, Dp, BK, BM)) return rc;          // operand loads
     if (int rc = make_map(&mapG, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.g, (uint64_t)w.Ncp, Dp, CW, 32)) return rc;   // gradient stores
     nuts_bigd_init<NPART><<<(w.Ncp + 3) / 4, 128, 0, stream>>>(a, w);
     const int ntile_rows = w.Ncp / BM;
     HMC_CUDA_CHECK(cudaMemsetAsync(w.tile_active, 0xff, (size_t)ntile_rows * 4, stream));
-    const size_t smem = gemm_smem_bytes<NPART, BN, BK, STAGES>();
     auto kern = bigd_gemm_step<NbWs, EPI_GRAD, NPART, BN, CL, BK, STAGES>;
-    HMC_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int ntiles = (ntile_rows / CL) * w.NT;                 // work items of a cluster
-    cudaLaunchConfig_t cfg = {};
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.gridDim = dim3(sms / CL * CL); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    int max_clusters = sms / CL;
-    if (CL > 1) {
-        int nc = 0;
-        HMC_CUDA_CHECK(cudaOccupancyMaxActiveClusters(&nc, kern, &cfg));
-        if (nc < 1) { hmc_set_error("large-D NUTS kernel: no cluster of %d CTAs fits on this device", CL); return HMC_E_CUDA; }
-        if (nc < max_clusters) max_clusters = nc;
-    }
-    const int nclusters = ntiles < max_clusters ? ntiles : max_clusters;
-    const int grid = nclusters * CL;
-    cfg.gridDim = dim3(grid);
+    cudaLaunchConfig_t cfg;
+    cudaLaunchAttribute attr;
+    if (int rc = bigd_launch_config(cfg, attr, kern, CL, (ntile_rows / CL) * w.NT, gemm_smem_bytes<NPART, BN, BK, STAGES>(), sms, stream,
+                                    kName)) return rc;
     const int Nch = a.Nchain;
     auto launch_gemm = [&]() { return cudaLaunchKernelEx(&cfg, kern, mapA, mapB, mapG, mapG, mapG, w, Nch, Dp, (const float*)w.dt); };
-    int* running_h = nullptr;
-    HMC_CUDA_CHECK(cudaMallocHost(&running_h, 16));
+    BigdRunning running;
+    if (int rc = running.alloc()) return rc;
     // a chain needs at most 1 + d_max gradient-only passes and 2^d_max - 1 steps per iteration, plus its chain start
     const long max_pass = (long)(a.iter_end - a.iter_begin) * ((1L << a.d_max) + a.d_max + 2) + 8;
     int rc = HMC_OK;
@@ -551,17 +482,16 @@ int run_nuts_bigd(const hmc_nuts_args& a, cudaStream_t stream) {
                                     NPART, BN, CL, a.Nchain, D, tsum[0] / 8, tsum[1] / 8);
         }
         if ((pass & 7) == 7) {
-            if (cudaMemcpyAsync(running_h, w.counters + 2, 4, cudaMemcpyDeviceToHost, stream) != cudaSuccess ||
-                cudaStreamSynchronize(stream) != cudaSuccess) { rc = HMC_E_CUDA; break; }
-            if (*running_h == 0) { ++pass; break; }
+            const int n = running.read(w.counters, stream);
+            if (n < 0) { rc = HMC_E_CUDA; break; }
+            if (n == 0) { ++pass; break; }
         }
     }
     if (rc == HMC_OK && pass >= max_pass) {                       // the bound holds every chain's passes: this look finds none running
-        if (cudaMemcpyAsync(running_h, w.counters + 2, 4, cudaMemcpyDeviceToHost, stream) != cudaSuccess ||
-            cudaStreamSynchronize(stream) != cudaSuccess) rc = HMC_E_CUDA;
-        else if (*running_h != 0) {
-            hmc_set_error("large-D NUTS kernel: %d chains still running after %ld passes", *running_h, max_pass);
-            cudaFreeHost(running_h);
+        const int n = running.read(w.counters, stream);
+        if (n < 0) rc = HMC_E_CUDA;
+        else if (n != 0) {
+            hmc_set_error("large-D NUTS kernel: %d chains still running after %ld passes", n, max_pass);
             return HMC_E_CUDA;
         }
     }
@@ -572,20 +502,13 @@ int run_nuts_bigd(const hmc_nuts_args& a, cudaStream_t stream) {
         fprintf(stderr, "[nuts bigd passes] passes=%ld gradient_rows=%llu chains=%d\n", pass, ng, a.Nchain);
         for (int i = 0; i < 3; ++i) cudaEventDestroy(ev[i]);
     }
-    cudaFreeHost(running_h);
-    if (rc == HMC_OK) HMC_CUDA_CHECK(cudaGetLastError());
-    else hmc_set_error("large-D NUTS kernel: CUDA error in the pass loop: %s", cudaGetErrorString(cudaGetLastError()));
-    return rc;
+    return bigd_loop_result(rc, kName);
 }
 
 }  // namespace
 
 bool hmc_nuts_bigd_supported(const hmc_nuts_args& a, const char** why) {
-    if (a.dtype != HMC_F32) { *why = "float32 only"; return false; }
-    if (a.target.Mit || a.target.Pt || a.target.Lct) { *why = "identity momentum metric only"; return false; }
-    if (a.target.D < 128 || a.target.D > 8192) { *why = "D must be in [128, 8192]"; return false; }
-    if (a.iter_end <= a.iter_begin) { *why = "needs at least one iteration"; return false; }
-    return true;
+    return bigd_covers(a.dtype, a.target, a.iter_begin, a.iter_end, why);
 }
 
 size_t hmc_nuts_bigd_workspace(const hmc_nuts_args& a) {
@@ -593,13 +516,10 @@ size_t hmc_nuts_bigd_workspace(const hmc_nuts_args& a) {
     return carve(w, nullptr, a.Nchain, a.target.D, 3, 128);
 }
 
+// bf16x3 unless the caller asks for fp16x2 (tree decisions are sign tests and near-ties; DESIGN 4.0 / 4.7)
 int hmc_nuts_run_bigd(const hmc_nuts_args& a, cudaStream_t stream) {
-    // bf16x3 unless the caller asks for fp16x2 (tree decisions are sign tests and near-ties; DESIGN 4.0 / 4.7)
-    bool fp16 = (a.flags & HMC_FLAG_TC_FP16X2) != 0;
-    if (const char* e = getenv("HMC_B200_TC_PREC")) fp16 = (e[0] == 'f');
-    int cl = 2;
-    if (const char* e = getenv("HMC_B200_BIGD_CLUSTER")) cl = atoi(e);
-    constexpr int ST2 = NEPI == 4 ? 3 : 2;
-    if (fp16) return cl == 2 ? run_nuts_bigd<2, 256, 2, 32, ST2>(a, stream) : run_nuts_bigd<2, 256, 1, 32, ST2>(a, stream);
-    return cl == 2 ? run_nuts_bigd<3, 128, 2, 32, 2>(a, stream) : run_nuts_bigd<3, 128, 1, 32, 2>(a, stream);
+    return bigd_run_variant(a.flags, [&](auto v) {
+        using V = decltype(v);
+        return run_nuts_bigd<V::NPART, V::BN, V::CL, V::BK, V::STAGES>(a, stream);
+    });
 }

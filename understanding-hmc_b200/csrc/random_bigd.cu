@@ -28,6 +28,7 @@
 //                    461-472), next iteration or chain end.
 // Chains advance asynchronously (SURVEY H3): every chain has its own phase, the GEMM never waits for a trajectory end.
 // All three kernels of a pass are enqueued back to back; the host looks at the number of running chains every 8 passes.
+// The set-up around the GEMM and the momentum-row / split-position helpers are shared with nuts_bigd.cu (bigd_gemm.cuh).
 //
 // HBM per chain and pass: p and q read + written (16 B / dimension), split position written (4 or 6 B) and read by TMA
 // (4 or 6 B; the four column tiles of a row block re-read it from L2): ~24 B x D vs 2 D^2 x 3 tensor flop.
@@ -75,51 +76,18 @@ struct BigdWs {                      // workspace carved by the host (all device
 };
 
 
-// ---------------------------------------------------------------------------------------------------------------------
-// momentum draw for one chain by one warp: p row (Dp wide, zero from D on), 0.5 |p|^2 of the D real dimensions, and
-// (iteration >= 1) trajectory length and log-uniform (same Philox keying as every other kernel: hmc_normal4 / hmc_scalar_draws;
-// when D % 4 != 0 only the first D % 4 normals of the last slot are used)
-// ---------------------------------------------------------------------------------------------------------------------
+// momentum draw for one chain by one warp: p row (bigd_momentum; prow may be NULL), 0.5 |p|^2 of the D real dimensions, and
+// (iteration >= 1) trajectory length and log-uniform (same Philox keying as every other kernel: hmc_scalar_draws)
 __device__ __forceinline__ float bigd_draw(const hmc_random_args& a, int Dp, long m, int iter, int lane, float* prow, int* L, float* lnu) {
     const int D = a.target.D;
     const uint64_t gid = (uint64_t)(a.chain_id0 + m);
-    float s = 0.f;
-    if (a.p_tape) {
-        const double* src = a.p_tape + ((size_t)m * (a.Niter + 1) + iter) * D;
-        for (int j = lane; j < D; j += 32) { const float v = (float)src[j]; if (prow) prow[j] = v; s = fmaf(v, v, s); }
-        if (prow) for (int j = D + lane; j < Dp; j += 32) prow[j] = 0.f;
-        if (iter >= 1) { *L = a.L_tape[(size_t)m * a.Niter + iter - 1]; *lnu = (float)log(a.u_tape[(size_t)m * a.Niter + iter - 1]); }
-    } else {
-        for (int sl = lane; sl < D / 4; sl += 32) {
-            const float4 z = hmc_normal4(a.seed, gid, (uint32_t)iter, (uint32_t)sl);
-            if (prow) *reinterpret_cast<float4*>(prow + 4 * sl) = z;
-            s += z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w;
-        }
-        for (int sl = D / 4 + lane; sl < Dp / 4; sl += 32) {             // the partly used last slot, then the padding
-            float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (4 * sl < D) {
-                z = hmc_normal4(a.seed, gid, (uint32_t)iter, (uint32_t)sl);
-                z.w = 0.f;
-                if (4 * sl + 2 >= D) z.z = 0.f;
-                if (4 * sl + 1 >= D) z.y = 0.f;
-            }
-            if (prow) *reinterpret_cast<float4*>(prow + 4 * sl) = z;
-            s += z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w;
-        }
-        if (iter >= 1) { double u; hmc_scalar_draws(a.seed, gid, (uint32_t)iter, a.L_low, a.L_high, L, &u); *lnu = (float)log(u); }
+    const double* tape = a.p_tape ? a.p_tape + ((size_t)m * (a.Niter + 1) + iter) * D : nullptr;
+    const float s = bigd_momentum(tape, a.seed, gid, iter, D, Dp, lane, prow, D / 4);
+    if (iter >= 1) {
+        if (a.p_tape) { *L = a.L_tape[(size_t)m * a.Niter + iter - 1]; *lnu = (float)log(a.u_tape[(size_t)m * a.Niter + iter - 1]); }
+        else { double u; hmc_scalar_draws(a.seed, gid, (uint32_t)iter, a.L_low, a.L_high, L, &u); *lnu = (float)log(u); }
     }
     return 0.5f * warp_sum<float>(s);
-}
-
-template <int NPART>
-__device__ __forceinline__ void bigd_write_parts(const BigdWs& w, long m, int lane, const float* xrow) {
-    const int Dp = w.Dp;
-    for (int j = 2 * lane; j < Dp; j += 64) {
-        uint32_t h[3];
-        split_pair<NPART>(xrow[j], xrow[j + 1], h);
-#pragma unroll
-        for (int pt = 0; pt < NPART; ++pt) reinterpret_cast<uint32_t*>(w.xp + (((size_t)w.wr * NPART + pt) * w.Ncp + m) * Dp)[j >> 1] = h[pt];
-    }
 }
 
 // passes the run of a chain needs (one per leapfrog point: L + 1 per iteration; rejections add a few): the key the rows are sorted by
@@ -146,10 +114,11 @@ __global__ void __launch_bounds__(128) bigd_init(hmc_random_args a, BigdWs w) {
     float* xr = w.x + (size_t)m * Dp;
     float* x0r = w.x0 + (size_t)m * Dp;
     float* pr = w.p + (size_t)m * Dp;
+    uint16_t* const xw = w.xp + (size_t)w.wr * NPART * w.Ncp * Dp;      // the operand buffer the next pass reads
     const long c = w.perm[m];                                            // the chain that lives in this row
     if (c < 0) {                                             // padding rows of the last tile
         for (int j = lane; j < Dp; j += 32) { xr[j] = 0.f; x0r[j] = 0.f; pr[j] = 0.f; }
-        bigd_write_parts<NPART>(w, m, lane, xr);
+        bigd_write_parts<NPART>(xw, w.Ncp, Dp, m, lane, xr);
         if (lane == 0) { w.mode[m] = MD_IDLE; w.it[m] = a.iter_end + 1; }
         return;
     }
@@ -164,8 +133,7 @@ __global__ void __launch_bounds__(128) bigd_init(hmc_random_args a, BigdWs w) {
         xr[j] = v - mu[j]; x0r[j] = v - mu[j];
     }
     for (int j = D + lane; j < Dp; j += 32) { xr[j] = 0.f; x0r[j] = 0.f; }
-    __syncwarp();
-    bigd_write_parts<NPART>(w, m, lane, xr);
+    bigd_write_parts<NPART>(xw, w.Ncp, Dp, m, lane, xr);
     int L = 1; float lnu = 0.f;
     float K0 = 0.f;
     if (fresh) K0 = bigd_draw(a, Dp, c, 0, lane, nullptr, &L, &lnu);               // samplers.py:415 (K only)
@@ -298,10 +266,7 @@ __global__ void __launch_bounds__(256) bigd_trajectory_end(hmc_random_args a, Bi
                 if (sq) sq[j] = q;
             }
         }
-        if (!accepted) {
-            __syncwarp();
-            bigd_write_parts<NPART>(w, m, lane, x0r);
-        }
+        if (!accepted) bigd_write_parts<NPART>(w.xp + (size_t)w.wr * NPART * w.Ncp * Dp, w.Ncp, Dp, m, lane, x0r);   // next pass's buffer
         if (last) {
             if (lane == 0) { w.mode[m] = MD_IDLE; w.it[m] = it + 1; a.state_eprev[c] = (double)w.E_prev[m]; }
         } else {
@@ -316,74 +281,48 @@ __global__ void __launch_bounds__(256) bigd_trajectory_end(hmc_random_args a, Bi
 
 // carve the workspace; returns the bytes needed (ws may be NULL to only size it)
 size_t carve(BigdWs& w, unsigned char* ws, long Nchain, int D, int npart, int bn) {
-    const long Ncp = (Nchain + BM * kMaxCluster - 1) / (BM * kMaxCluster) * (BM * kMaxCluster);   // whole clusters of row blocks
-    const int Dp = (D + 31) / 32 * 32;
-    const int NT = (Dp + bn - 1) / bn;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { unsigned char* p = ws ? ws + off : nullptr; off = align_up(off + bytes, 1024); return p; };
+    BigdCarve c(ws, Nchain, D, bn);
+    const long Ncp = c.Ncp;
+    const int Dp = c.Dp, NT = c.NT;
     w.Ncp = (int)Ncp; w.NT = NT; w.npart = npart; w.Dp = Dp;
-    w.xp = (uint16_t*)take((size_t)2 * npart * Ncp * Dp * 2);
-    w.bp = (uint16_t*)take((size_t)npart * Dp * Dp * 2);
-    w.x = (float*)take((size_t)Ncp * Dp * 4);
-    w.x0 = (float*)take((size_t)Ncp * Dp * 4);
-    w.p = (float*)take((size_t)Ncp * Dp * 4);
-    w.mu = (float*)take((size_t)Dp * 4);
-    w.dt = (float*)take((size_t)Dp * 4);
-    w.red = (float*)take((size_t)Ncp * NT * 2 * 2 * 4);
-    w.mode = (int*)take(Ncp * 4); w.l = (int*)take(Ncp * 4); w.L = (int*)take(Ncp * 4); w.it = (int*)take(Ncp * 4); w.init = (int*)take(Ncp * 4);
-    w.K_new = (float*)take(Ncp * 4); w.K0 = (float*)take(Ncp * 4); w.lnu = (float*)take(Ncp * 4); w.E_init = (float*)take(Ncp * 4);
-    w.E_prev = (float*)take(Ncp * 4);
-    w.tile_active = (int*)take((Ncp / BM) * 4);
-    w.list = (int*)take(Ncp * 4);
-    w.counters = (int*)take(64);
-    w.perm = (int*)take(Ncp * 4);
-    w.plan = (int*)take(Ncp * 4);
-    return off;
+    w.xp = (uint16_t*)c.take((size_t)2 * npart * Ncp * Dp * 2);
+    w.bp = (uint16_t*)c.take((size_t)npart * Dp * Dp * 2);
+    w.x = (float*)c.take((size_t)Ncp * Dp * 4);
+    w.x0 = (float*)c.take((size_t)Ncp * Dp * 4);
+    w.p = (float*)c.take((size_t)Ncp * Dp * 4);
+    w.mu = (float*)c.take((size_t)Dp * 4);
+    w.dt = (float*)c.take((size_t)Dp * 4);
+    w.red = (float*)c.take((size_t)Ncp * NT * 2 * 2 * 4);
+    w.mode = (int*)c.take(Ncp * 4); w.l = (int*)c.take(Ncp * 4); w.L = (int*)c.take(Ncp * 4); w.it = (int*)c.take(Ncp * 4); w.init = (int*)c.take(Ncp * 4);
+    w.K_new = (float*)c.take(Ncp * 4); w.K0 = (float*)c.take(Ncp * 4); w.lnu = (float*)c.take(Ncp * 4); w.E_init = (float*)c.take(Ncp * 4);
+    w.E_prev = (float*)c.take(Ncp * 4);
+    w.tile_active = (int*)c.take((Ncp / BM) * 4);
+    w.list = (int*)c.take(Ncp * 4);
+    w.counters = (int*)c.take(64);
+    w.perm = (int*)c.take(Ncp * 4);
+    w.plan = (int*)c.take(Ncp * 4);
+    return c.off;
 }
 
+constexpr const char* kName = "large-D kernel";
 
 template <int NPART, int BN, int CL, int BK, int STAGES>
 int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
     const int D = a.target.D;
     BigdWs w;
     const size_t need = carve(w, (unsigned char*)a.workspace, a.Nchain, D, NPART, BN);
-    if (!a.workspace || (size_t)a.workspace_bytes < need) {
-        hmc_set_error("large-D kernel needs a workspace of %zu bytes (hmc_random_workspace_bytes)", need);
-        return HMC_E_BADARG;
-    }
+    if (int rc = bigd_check_workspace(a.workspace, a.workspace_bytes, need, kName, "hmc_random_workspace_bytes")) return rc;
     int dev = 0, sms = 0;
     HMC_CUDA_CHECK(cudaGetDevice(&dev));
     HMC_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    // force matrix parts (scaled to the top of the fp16 range for the fp16 split)
     const int Dp = w.Dp;
-    float scale = 1.f;
-    HMC_CUDA_CHECK(cudaMemsetAsync(w.counters, 0, 64, stream));
-    // mean and step sizes, zero-padded to Dp (the caller's arrays are D_pad <= Dp long)
-    HMC_CUDA_CHECK(cudaMemsetAsync(w.mu, 0, (size_t)Dp * 4, stream));
-    HMC_CUDA_CHECK(cudaMemsetAsync(w.dt, 0, (size_t)Dp * 4, stream));
-    HMC_CUDA_CHECK(cudaMemcpyAsync(w.mu, a.target.mu, (size_t)D * 4, cudaMemcpyDeviceToDevice, stream));
-    HMC_CUDA_CHECK(cudaMemcpyAsync(w.dt, a.target.dt, (size_t)D * 4, cudaMemcpyDeviceToDevice, stream));
-    if (NPART == 2) {
-        unsigned int* mxd = (unsigned int*)(w.counters + 8);
-        bigd_absmax<<<sms * 4, 256, 0, stream>>>((const float*)a.target.Ft, D, a.target.D_pad, mxd);
-        unsigned int mx = 0;
-        HMC_CUDA_CHECK(cudaMemcpyAsync(&mx, mxd, 4, cudaMemcpyDeviceToHost, stream));
-        HMC_CUDA_CHECK(cudaStreamSynchronize(stream));
-        const int e = (int)(mx >> 23) - 127;
-        int sft = (mx == 0u || e < -100) ? 0 : 14 - e;
-        sft = sft > 100 ? 100 : (sft < -100 ? -100 : sft);
-        scale = ldexpf(1.f, sft);
-    }
-    w.binv = 1.f / scale;
-    bigd_split_matrix<NPART><<<sms * 8, 256, 0, stream>>>((const float*)a.target.Ft, D, a.target.D_pad, Dp, scale, w.bp);
     CUtensorMap mapA[2], mapS[2], mapB, mapP, mapX;
-    const CUtensorMapDataType dt16 = NPART == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    if (int rc = bigd_target_operands<NPART, BN, CL, BK>(a.target, w, sms, stream, &mapB)) return rc;
     for (int b = 0; b < 2; ++b) {
         uint16_t* xb = w.xp + (size_t)b * NPART * w.Ncp * Dp;
-        if (int rc = make_map(&mapA[b], dt16, 2, xb, (uint64_t)NPART * w.Ncp, Dp, BK, BM)) return rc;      // operand loads
-        if (int rc = make_map(&mapS[b], dt16, 2, xb, (uint64_t)NPART * w.Ncp, Dp, CW, 32)) return rc;      // epilogue stores
+        if (int rc = make_map(&mapA[b], bigd_dt16<NPART>(), 2, xb, (uint64_t)NPART * w.Ncp, Dp, BK, BM)) return rc;      // operand loads
+        if (int rc = make_map(&mapS[b], bigd_dt16<NPART>(), 2, xb, (uint64_t)NPART * w.Ncp, Dp, CW, 32)) return rc;      // epilogue stores
     }
-    if (int rc = make_map(&mapB, dt16, 2, w.bp, (uint64_t)NPART * Dp, Dp, BK, BN / CL)) return rc;         // each CTA of a cluster loads 1 / CL of a B tile
     if (int rc = make_map(&mapP, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.p, (uint64_t)w.Ncp, Dp, CW, 32)) return rc;
     if (int rc = make_map(&mapX, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.x, (uint64_t)w.Ncp, Dp, CW, 32)) return rc;
     w.wr = 0;                                                    // pass 0 reads buffer 0
@@ -404,34 +343,18 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
     bigd_init<NPART><<<(w.Ncp + 3) / 4, 128, 0, stream>>>(a, w);
     const int ntile_rows = w.Ncp / BM;
     HMC_CUDA_CHECK(cudaMemsetAsync(w.tile_active, 0xff, (size_t)ntile_rows * 4, stream));
-    const size_t smem = gemm_smem_bytes<NPART, BN, BK, STAGES>();
     auto kern = bigd_gemm_step<BigdWs, EPI_LEAPFROG, NPART, BN, CL, BK, STAGES>;
-    HMC_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int ntiles = (ntile_rows / CL) * w.NT;                 // work items of a cluster
-    // persistent clusters: as many as are resident at once (a GPC holds whole clusters only), never more than there is work
-    cudaLaunchConfig_t cfg = {};
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.gridDim = dim3(sms / CL * CL); cfg.blockDim = dim3(NTHREADS); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    int max_clusters = sms / CL;
-    if (CL > 1) {
-        int nc = 0;
-        HMC_CUDA_CHECK(cudaOccupancyMaxActiveClusters(&nc, kern, &cfg));
-        if (nc < 1) { hmc_set_error("large-D kernel: no cluster of %d CTAs fits on this device", CL); return HMC_E_CUDA; }
-        if (nc < max_clusters) max_clusters = nc;
-    }
-    const int nclusters = ntiles < max_clusters ? ntiles : max_clusters;
-    const int grid = nclusters * CL;
-    cfg.gridDim = dim3(grid);
+    cudaLaunchConfig_t cfg;
+    cudaLaunchAttribute attr;
+    if (int rc = bigd_launch_config(cfg, attr, kern, CL, ntiles, gemm_smem_bytes<NPART, BN, BK, STAGES>(), sms, stream, kName)) return rc;
     const float* dtv = w.dt;
     const int Nch = a.Nchain;
     // pass n: operands from buffer n & 1, the epilogue (and the trajectory ends after it) write buffer (n + 1) & 1
     auto launch_gemm = [&](long pass) { w.wr = (int)((pass + 1) & 1);
                                         return cudaLaunchKernelEx(&cfg, kern, mapA[pass & 1], mapB, mapP, mapX, mapS[(pass + 1) & 1], w, Nch, Dp, dtv); };
-    int* running_h = nullptr;
-    HMC_CUDA_CHECK(cudaMallocHost(&running_h, 4));
+    BigdRunning running;
+    if (int rc = running.alloc()) return rc;
     const long max_pass = (long)(a.iter_end - a.iter_begin) * (a.L_high + 1) + 8;
     int rc = HMC_OK;
     // HMC_B200_BIGD_TIMING=1: CUDA-event times of the three kernels of passes 4..11 on stderr (measurement aid)
@@ -440,48 +363,37 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
     float tsum[3] = {0.f, 0.f, 0.f};
     if (timing) for (int i = 0; i < 4; ++i) cudaEventCreate(&ev[i]);
     for (long pass = 0; pass < max_pass; ++pass) {
-        if (timing && pass >= 4 && pass < 12) {
-            cudaEventRecord(ev[0], stream);
-            launch_gemm(pass);
-            cudaEventRecord(ev[1], stream);
-            cudaMemsetAsync(w.counters + 2, 0, 4, stream);
-            bigd_events<<<ntile_rows, BM, 0, stream>>>(a, w, (int)pass);
-            cudaEventRecord(ev[2], stream);
-            bigd_trajectory_end<NPART><<<sms * 2, 256, 0, stream>>>(a, w, (int)pass);
+        const bool timed = timing && pass >= 4 && pass < 12;
+        if (timed) cudaEventRecord(ev[0], stream);
+        if (launch_gemm(pass) != cudaSuccess) { rc = HMC_E_CUDA; break; }
+        if (timed) cudaEventRecord(ev[1], stream);
+        cudaMemsetAsync(w.counters + 2, 0, 4, stream);
+        bigd_events<<<ntile_rows, BM, 0, stream>>>(a, w, (int)pass);
+        if (timed) cudaEventRecord(ev[2], stream);
+        bigd_trajectory_end<NPART><<<sms * 2, 256, 0, stream>>>(a, w, (int)pass);
+        if (timed) {
             cudaEventRecord(ev[3], stream);
             cudaEventSynchronize(ev[3]);
             for (int i = 0; i < 3; ++i) { float ms = 0.f; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); tsum[i] += ms; }
             if (pass == 11) fprintf(stderr, "[bigd timing] NPART=%d BN=%d BK=%d cluster=%d chains=%d D=%d: gemm_step %.3f ms, events %.3f ms, trajectory_end %.3f ms per pass (%d work items on %d CTAs)\n",
-                                    NPART, BN, BK, CL, a.Nchain, D, tsum[0] / 8, tsum[1] / 8, tsum[2] / 8, ntiles, grid);
-            continue;
+                                    NPART, BN, BK, CL, a.Nchain, D, tsum[0] / 8, tsum[1] / 8, tsum[2] / 8, ntiles, (int)cfg.gridDim.x);
         }
-        if (launch_gemm(pass) != cudaSuccess) { rc = HMC_E_CUDA; break; }
-        cudaMemsetAsync(w.counters + 2, 0, 4, stream);
-        bigd_events<<<ntile_rows, BM, 0, stream>>>(a, w, (int)pass);
-        bigd_trajectory_end<NPART><<<sms * 2, 256, 0, stream>>>(a, w, (int)pass);
         if ((pass & 7) == 7) {
             // chains that ended their last trajectory in this pass are still MD_PENDING for the events kernel's count: they are
             // counted as running and found idle at the next look
-            if (cudaMemcpyAsync(running_h, w.counters + 2, 4, cudaMemcpyDeviceToHost, stream) != cudaSuccess ||
-                cudaStreamSynchronize(stream) != cudaSuccess) { rc = HMC_E_CUDA; break; }
-            if (*running_h == 0) break;
+            const int n = running.read(w.counters, stream);
+            if (n < 0) { rc = HMC_E_CUDA; break; }
+            if (n == 0) break;
         }
     }
     if (timing) for (int i = 0; i < 4; ++i) cudaEventDestroy(ev[i]);
-    cudaFreeHost(running_h);
-    if (rc == HMC_OK) HMC_CUDA_CHECK(cudaGetLastError());
-    else hmc_set_error("large-D kernel: CUDA error in the pass loop: %s", cudaGetErrorString(cudaGetLastError()));
-    return rc;
+    return bigd_loop_result(rc, kName);
 }
 
 }  // namespace
 
 bool hmc_random_bigd_supported(const hmc_random_args& a, const char** why) {
-    if (a.dtype != HMC_F32) { *why = "float32 only"; return false; }
-    if (a.target.Mit || a.target.Pt || a.target.Lct) { *why = "identity momentum metric only"; return false; }
-    if (a.target.D < 128 || a.target.D > 8192) { *why = "D must be in [128, 8192]"; return false; }
-    if (a.iter_end <= a.iter_begin) { *why = "needs at least one iteration"; return false; }
-    return true;
+    return bigd_covers(a.dtype, a.target, a.iter_begin, a.iter_end, why);
 }
 
 size_t hmc_random_bigd_workspace(const hmc_random_args& a) {
@@ -490,14 +402,8 @@ size_t hmc_random_bigd_workspace(const hmc_random_args& a) {
 }
 
 int hmc_random_run_bigd(const hmc_random_args& a, cudaStream_t stream) {
-    bool fp16 = (a.flags & HMC_FLAG_TC_FP16X2) != 0;
-    if (const char* e = getenv("HMC_B200_TC_PREC")) fp16 = (e[0] == 'f');
-    // Clusters of two row blocks share the column block's B tile by TMA multicast (HMC_B200_BIGD_CLUSTER=1: plain CTAs).  With the
-    // first epilogue the cluster changed nothing (the kernel was bound by its epilogue); with the TMA epilogue it is worth 8 % of a
-    // full pass at fp16x2 and 19 % of a bf16x3 run (DESIGN 4.5).
-    int cl = 2;
-    if (const char* e = getenv("HMC_B200_BIGD_CLUSTER")) cl = atoi(e);
-    constexpr int ST2 = NEPI == 4 ? 3 : 2;           // operand stages that fit beside the epilogue buffers
-    if (fp16) return cl == 2 ? run_bigd<2, 256, 2, 32, ST2>(a, stream) : run_bigd<2, 256, 1, 32, ST2>(a, stream);
-    return cl == 2 ? run_bigd<3, 128, 2, 32, 2>(a, stream) : run_bigd<3, 128, 1, 32, 2>(a, stream);
+    return bigd_run_variant(a.flags, [&](auto v) {
+        using V = decltype(v);
+        return run_bigd<V::NPART, V::BN, V::CL, V::BK, V::STAGES>(a, stream);
+    });
 }

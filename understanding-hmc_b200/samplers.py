@@ -363,6 +363,25 @@ class HMC_sampler(sampler):
             return q_start.to(device=dev, dtype=tdt, non_blocking=True).contiguous()
         return torch.from_numpy(np.ascontiguousarray(np.asarray(q_start), dtype=float)).to(device=dev, dtype=tdt).contiguous()
 
+    def _fp16x2_flag(self):
+        """FLAG_TC_FP16X2 when tc_precision asks for the two-part fp16 split of the tensor-core gradient product and the target
+        allows it, else 0.  The split needs a target whose scale is not far below 1 (fp16 subnormals); otherwise tc_precision
+        falls back to bf16x3."""
+        if self.tc_precision != "fp16x2":
+            return 0
+        if float(np.min(1.0 / np.sqrt(np.abs(np.diag(self.target.P))))) < 2.0 ** -10:
+            self.tc_precision = "bf16x3"
+            return 0
+        return _L.FLAG_TC_FP16X2
+
+    @staticmethod
+    def _set_workspace(torch, dev, a, nbytes):
+        """Point the launch arguments a at a new 1024-byte aligned device workspace of nbytes; returns the tensor that owns it."""
+        buf = torch.empty((nbytes + 1024,), dtype=torch.uint8, device=dev)
+        a.workspace = (buf.data_ptr() + 1023) // 1024 * 1024
+        a.workspace_bytes = nbytes
+        return buf
+
     def prepare_random(self, q_start, N_save_chain0=0):
         """Allocate the device-resident outputs/state and build the C-ABI argument block (hmc_random_args) of
         the random-trajectory sampler; the caller launches iteration blocks with hmc_random_run."""
@@ -398,13 +417,8 @@ class HMC_sampler(sampler):
             (self.kernel == "bigd" or (self.kernel == "auto" and (D % 256 == 0 or D > 1024)))     # csrc/api.cu AUTO rule
         if self.tc_precision is None:
             self.tc_precision = "fp16x2" if bigd else "bf16x3"
-        if self.tc_precision == "fp16x2":
-            # two-part fp16 split of the tensor-core gradient product; needs |q - mu| < 16384 (checked by the kernel, word
-            # 16 + Nchain of state_g) and a target whose scale is not far below 1 (fp16 subnormals)
-            if float(np.min(1.0 / np.sqrt(np.abs(np.diag(self.target.P))))) < 2.0 ** -10:
-                self.tc_precision = "bf16x3"
-            else:
-                a.flags |= _L.FLAG_TC_FP16X2
+        # (the fp16 split also needs |q - mu| < 16384: the tensor-core kernel checks it, word 16 + Nchain of state_g)
+        a.flags |= self._fp16x2_flag()
         a.flags |= (int(os.environ.get("HMC_B200_TILE_VARIANT", "0")) & 0xff) << 8      # tuning knob
         a.q_start = keep["qs"].data_ptr()
         if self.draws is not None:
@@ -419,11 +433,7 @@ class HMC_sampler(sampler):
             keep["state_e"].data_ptr()
         a.counters = counters.data_ptr()
         if bigd:                                  # large-D GEMM path: its scratch (split operands, state, per-chain scalars)
-            nbytes = int(_L.load().hmc_random_workspace_bytes(a))
-            keep["workspace"] = torch.empty((nbytes + 1024,), dtype=torch.uint8, device=dev)
-            base = keep["workspace"].data_ptr()
-            a.workspace = (base + 1023) // 1024 * 1024
-            a.workspace_bytes = nbytes
+            keep["workspace"] = self._set_workspace(torch, dev, a, int(_L.load().hmc_random_workspace_bytes(a)))
         if save_chain and owns0:
             keep["phi"] = torch.zeros((N_save_chain0, int(self.L_high), 2), dtype=f64, device=dev)
             keep["phi_len"] = torch.zeros((N_save_chain0,), dtype=torch.int32, device=dev)
@@ -541,16 +551,8 @@ class HMC_sampler(sampler):
         if self.nuts_kernel == "bigd":            # large-D GEMM path: its scratch (split operands, x / p / gradient rows, chain states)
             if self.tc_precision is None:
                 self.tc_precision = "bf16x3"      # tree decisions are sign tests and near-ties: the split without fp16's V bias
-            if self.tc_precision == "fp16x2":
-                # two-part fp16 split; needs a target whose scale is not far below 1 (fp16 subnormals), as for Random
-                if float(np.min(1.0 / np.sqrt(np.abs(np.diag(self.target.P))))) < 2.0 ** -10:
-                    self.tc_precision = "bf16x3"
-                else:
-                    a.flags |= _L.FLAG_TC_FP16X2
-            nbytes = int(lib.hmc_nuts_workspace_bytes(a))
-            ws = torch.empty((nbytes + 1024,), dtype=torch.uint8, device=dev)
-            a.workspace = (ws.data_ptr() + 1023) // 1024 * 1024
-            a.workspace_bytes = nbytes
+            a.flags |= self._fp16x2_flag()
+            keep["workspace"] = self._set_workspace(torch, dev, a, int(lib.hmc_nuts_workspace_bytes(a)))
         stream = _L.current_stream_ptr()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         if verbose:
