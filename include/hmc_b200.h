@@ -92,10 +92,24 @@ typedef struct hmc_target {
  * HMC_sampler.leap_frog (samplers.py:831-839) for B independent (p, q) pairs, rows of [B][D] arrays in `dtype`:
  *   p' = p - dt F (q - mu) / 2,  q' = q + dt p',  p'' = p' - dt F (q' - mu) / 2      (F = M^-1 P; q moves by p, not M^-1 p: quirk Q9)
  * `nsteps` >= 1 repetitions.  The public primitive of the path (the samplers fuse it into their trajectory kernels, one gradient
- * per step); D <= 1024.
+ * per step); D <= 1024 (hmc_leap_frog_bigd: float32 up to D = 8192).
  */
 int hmc_leap_frog(int32_t dtype, const hmc_target* target, int64_t B, const void* p_old, const void* q_old, void* p_new, void* q_new,
                   int32_t nsteps, void* cuda_stream);
+
+/*
+ * hmc_leap_frog for float32 and any 128 <= D <= 8192, on the tcgen05 GEMM of the large-D path (csrc/bigd_primitives.cu): any
+ * metric (only target.Ft, mu and dt enter), B rows of [B][D] arrays.  The nsteps steps run as nsteps + 1 gradient products: the
+ * closing half kick of a step and the opening half kick of the next are merged into one full kick, so with nsteps > 1 the result
+ * differs from nsteps separate calls in the last bits.  flags: HMC_FLAG_TC_FP16X2 selects the two-part fp16 split (default: the
+ * three-part bf16 split), with the same range condition as for the samplers.  `workspace`: device scratch of at least
+ * hmc_leap_frog_workspace_bytes(target, B, flags) bytes, 1024-byte aligned; a missing or short one is HMC_E_BADARG.  float64 or D
+ * outside [128, 8192] is HMC_E_UNSUPPORTED.  The size is non-zero exactly for 128 <= D <= 8192 and 1 <= B <= 2^30 (it depends on
+ * target->D and B only and covers both splits); 0 otherwise.
+ */
+int64_t hmc_leap_frog_workspace_bytes(const hmc_target* target, int64_t B, int32_t flags);
+int hmc_leap_frog_bigd(int32_t dtype, const hmc_target* target, int64_t B, const void* p_old, const void* q_old, void* p_new,
+                       void* q_new, int32_t nsteps, int32_t flags, void* workspace, int64_t workspace_bytes, void* cuda_stream);
 
 /*
  * Random-trajectory-length sampler: replaces HMC_sampler.gen_sample_random (samplers.py:387-491) together
@@ -253,6 +267,19 @@ int hmc_diag_variogram_all(int32_t dtype, const void* q, int64_t Nchain, int64_t
  */
 int hmc_start_pts(int32_t dtype, uint64_t seed, int64_t chain_id0, int64_t Nchain, int32_t D, const double* q0,
                   const double* Lc, const double* sd, void* out, void* cuda_stream);
+
+/*
+ * q_m = q0 + Lc z_m on the tensor cores (csrc/bigd_primitives.cu), float32 out, 128 <= D <= 8192: the same Philox normals as
+ * hmc_start_pts (seed, global chain id, HMC_STREAM_START, full-precision Box-Muller), so for the same (seed, chain_id0) the two
+ * entry points draw the same z.  Lc: row-major lower-triangular float64 [D][D] (the lower triangle is read), rounded to float32
+ * and split into three bf16 parts, fp32 accumulation; or NULL with sd [D] (diagonal cov0: elementwise, no GEMM, the same rows as
+ * hmc_start_pts).  `workspace` (used with Lc only): device scratch of at least hmc_start_pts_workspace_bytes(Nchain, D) bytes,
+ * 1024-byte aligned; a missing or short one is HMC_E_BADARG.  float64 or D outside [128, 8192] is HMC_E_UNSUPPORTED.  The size
+ * is non-zero exactly for 128 <= D <= 8192 and 1 <= Nchain <= 2^30, 0 otherwise.
+ */
+int64_t hmc_start_pts_workspace_bytes(int64_t Nchain, int32_t D);
+int hmc_start_pts_bigd(int32_t dtype, uint64_t seed, int64_t chain_id0, int64_t Nchain, int32_t D, const double* q0,
+                       const double* Lc, const double* sd, void* out, void* workspace, int64_t workspace_bytes, void* cuda_stream);
 
 /*
  * Sample summaries: the inputs of sampler.plot_samples (samplers.py:84-113, 160-186, 209-250) as HBM-bound reductions over

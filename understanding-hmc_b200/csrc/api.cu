@@ -27,6 +27,14 @@ bool hmc_nuts_tc_supported(const hmc_nuts_args& a, const char** why);
 int hmc_nuts_run_bigd(const hmc_nuts_args& a, cudaStream_t stream);
 bool hmc_nuts_bigd_supported(const hmc_nuts_args& a, const char** why);
 size_t hmc_nuts_bigd_workspace(const hmc_nuts_args& a);
+bool hmc_start_pts_bigd_supported(int dtype, int D, const char** why);
+size_t hmc_start_pts_bigd_workspace(long Nchain, int D);
+int hmc_start_pts_bigd_run(uint64_t seed, int64_t chain_id0, long Nchain, int D, const double* q0, const double* Lc, const double* sd,
+                           float* out, void* ws, int64_t ws_bytes, cudaStream_t stream);
+bool hmc_leap_frog_bigd_supported(int dtype, int D, const char** why);
+size_t hmc_leap_frog_bigd_workspace(long B, int D);
+int hmc_leap_frog_bigd_run(const hmc_target& t, long B, const float* p_old, const float* q_old, float* p_new, float* q_new, int nsteps,
+                           int flags, void* ws, int64_t ws_bytes, cudaStream_t stream);
 
 extern "C" int hmc_version(void) { return HMC_B200_VERSION; }
 extern "C" const char* hmc_last_error_string(void) { return g_err; }
@@ -170,6 +178,52 @@ extern "C" int64_t hmc_nuts_workspace_bytes(const hmc_nuts_args* args) {
     a.iter_begin = 0; a.iter_end = 1;
     if (!hmc_nuts_bigd_supported(a, &why)) return 0;
     return (int64_t)hmc_nuts_bigd_workspace(a);
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Large-D primitives (csrc/bigd_primitives.cu): start points and leap_frog on the tcgen05 GEMM, 128 <= D <= 8192, float32
+// ---------------------------------------------------------------------------------------------------------
+static constexpr int64_t kBigdMaxRows = (int64_t)1 << 30;       // chains / rows of one call (the GEMM indexes rows with int)
+
+extern "C" int64_t hmc_start_pts_workspace_bytes(int64_t Nchain, int32_t D) {
+    const char* why = "";
+    if (Nchain < 1 || Nchain > kBigdMaxRows || !hmc_start_pts_bigd_supported(HMC_F32, D, &why)) return 0;
+    return (int64_t)hmc_start_pts_bigd_workspace((long)Nchain, D);
+}
+
+extern "C" int hmc_start_pts_bigd(int32_t dtype, uint64_t seed, int64_t chain_id0, int64_t Nchain, int32_t D, const double* q0,
+                                  const double* Lc, const double* sd, void* out, void* workspace, int64_t workspace_bytes,
+                                  void* cuda_stream) {
+    HMC_REQUIRE(Nchain >= 1 && Nchain <= kBigdMaxRows && q0 && out && (Lc || sd),
+                "hmc_start_pts_bigd: need 1 <= Nchain <= 2^30, q0, out and Lc or sd");
+    const char* why = "";
+    if (!hmc_start_pts_bigd_supported(dtype, D, &why)) {
+        hmc_set_error("hmc_start_pts_bigd does not cover this configuration: %s", why);
+        return HMC_E_UNSUPPORTED;
+    }
+    return hmc_start_pts_bigd_run(seed, chain_id0, (long)Nchain, D, q0, Lc, sd, (float*)out, workspace, workspace_bytes,
+                                  (cudaStream_t)cuda_stream);
+}
+
+extern "C" int64_t hmc_leap_frog_workspace_bytes(const hmc_target* target, int64_t B, int32_t flags) {
+    (void)flags;                                    // (sized for the larger of the two splits)
+    const char* why = "";
+    if (!target || B < 1 || B > kBigdMaxRows || !hmc_leap_frog_bigd_supported(HMC_F32, target->D, &why)) return 0;
+    return (int64_t)hmc_leap_frog_bigd_workspace((long)B, target->D);
+}
+
+extern "C" int hmc_leap_frog_bigd(int32_t dtype, const hmc_target* target, int64_t B, const void* p_old, const void* q_old, void* p_new,
+                                  void* q_new, int32_t nsteps, int32_t flags, void* workspace, int64_t workspace_bytes, void* cuda_stream) {
+    HMC_REQUIRE(target && p_old && q_old && p_new && q_new, "hmc_leap_frog_bigd: NULL buffer");
+    if (int rc = check_target(*target)) return rc;
+    HMC_REQUIRE(B >= 1 && B <= kBigdMaxRows && nsteps >= 1, "hmc_leap_frog_bigd: need 1 <= B <= 2^30 and nsteps >= 1");
+    const char* why = "";
+    if (!hmc_leap_frog_bigd_supported(dtype, target->D, &why)) {
+        hmc_set_error("hmc_leap_frog_bigd does not cover this configuration: %s", why);
+        return HMC_E_UNSUPPORTED;
+    }
+    return hmc_leap_frog_bigd_run(*target, (long)B, (const float*)p_old, (const float*)q_old, (float*)p_new, (float*)q_new, nsteps, flags,
+                                  workspace, workspace_bytes, (cudaStream_t)cuda_stream);
 }
 
 // ---------------------------------------------------------------------------------------------------------

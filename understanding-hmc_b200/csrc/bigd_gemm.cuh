@@ -1,4 +1,5 @@
-// The large-D tcgen05 GEMM shared by the large-D samplers (random_bigd.cu, nuts_bigd.cu): G = X F^T for all chains of a pass,
+// The large-D tcgen05 GEMM shared by the large-D samplers (random_bigd.cu, nuts_bigd.cu) and primitives (bigd_primitives.cu:
+// start points, leap_frog): G = X F^T for all chains of a pass,
 // X = the split positions [Ncp][Dp] (A operand, by TMA), F = the split force matrix [Dp][Dp] (B operand, by TMA, multicast to a
 // cluster of row blocks), fp32 accumulators in tensor memory.  The epilogue is a template parameter:
 //   EPI_LEAPFROG  the leapfrog update of the random-trajectory sampler fused into the epilogue (random_bigd.cu explains it)
@@ -515,6 +516,14 @@ bool bigd_covers(int dtype, const hmc_target& t, int iter_begin, int iter_end, c
     if (t.Mit || t.Pt || t.Lct) { *why = "identity momentum metric only"; return false; }
     if (t.D < 128 || t.D > 8192) { *why = "D must be in [128, 8192]"; return false; }
     if (iter_end <= iter_begin) { *why = "needs at least one iteration"; return false; }
+    return true;
+}
+
+// the dtype and sizes the GEMM itself covers, whatever the metric: the large-D primitives (bigd_primitives.cu) take any metric,
+// their caller having folded it into the one matrix they multiply by
+bool bigd_covers_gemm(int dtype, int D, const char** why) {
+    if (dtype != HMC_F32) { *why = "float32 only"; return false; }
+    if (D < 128 || D > 8192) { *why = "D must be in [128, 8192]"; return false; }
     return true;
 }
 

@@ -52,7 +52,22 @@ __device__ __forceinline__ long hmc_store_index(int it, int warm_up_num, int thi
     return (long)idx;
 }
 
-enum { HMC_STREAM_MOMENTUM = 0, HMC_STREAM_SCALAR = 1, HMC_STREAM_NUTS = 2 };
+enum { HMC_STREAM_MOMENTUM = 0, HMC_STREAM_SCALAR = 1, HMC_STREAM_NUTS = 2, HMC_STREAM_START = 4 };
+
+// 4 standard normals for dims 4*slot .. 4*slot+3 of a start point (hmc_start_pts, hmc_start_pts_bigd: both draw the same z)
+__device__ __forceinline__ float4 hmc_start_normal4(uint64_t seed, uint64_t gid, uint32_t slot) {
+    const Philox4 r = philox4x32_10((uint32_t)gid, 0u, slot, HMC_STREAM_START | ((uint32_t)(gid >> 32) << 8),
+                                    (uint32_t)seed, (uint32_t)(seed >> 32));
+    // Box-Muller, full-precision logf / sincosf (not on a hot path)
+    const float u1 = ((float)(r.x >> 8) + 0.5f) * 5.9604644775390625e-08f, u2 = ((float)(r.z >> 8) + 0.5f) * 5.9604644775390625e-08f;
+    const float r1 = sqrtf(-2.0f * logf(u1)), r2 = sqrtf(-2.0f * logf(u2));
+    const float a1 = ((float)(r.y >> 8) * 5.9604644775390625e-08f - 0.5f) * 6.283185307179586f;
+    const float a2 = ((float)(r.w >> 8) * 5.9604644775390625e-08f - 0.5f) * 6.283185307179586f;
+    float s1, c1, s2, c2;
+    sincosf(a1, &s1, &c1);
+    sincosf(a2, &s2, &c2);
+    return make_float4(r1 * c1, r1 * s1, r2 * c2, r2 * s2);
+}
 
 // 4 standard normals for dims 4*slot .. 4*slot+3 of (chain, iteration): float32 Box-Muller.
 __device__ __forceinline__ float4 hmc_normal4(uint64_t seed, uint64_t chain, uint32_t iter, uint32_t slot) {

@@ -12,8 +12,6 @@
 
 namespace {
 
-enum { HMC_STREAM_START = 4 };
-
 // one warp per chain: z staged in shared memory, lane j computes rows j, j+32, ... of q0 + Lc z (Lc lower triangular,
 // row-major) or q0 + sd .* z
 template <typename T>
@@ -25,19 +23,7 @@ __global__ void __launch_bounds__(128) start_pts_kernel(uint64_t seed, int64_t c
     float* zs = zs_all + (size_t)warp * Dp;
     for (long m = (long)blockIdx.x * (blockDim.x >> 5) + warp; m < Nchain; m += (long)gridDim.x * (blockDim.x >> 5)) {
         const uint64_t gid = (uint64_t)(chain_id0 + m);
-        for (int s = lane; s < Dp / 4; s += 32) {
-            const Philox4 r = philox4x32_10((uint32_t)gid, 0u, (uint32_t)s, HMC_STREAM_START | ((uint32_t)(gid >> 32) << 8),
-                                            (uint32_t)seed, (uint32_t)(seed >> 32));
-            // Box-Muller, full-precision logf / sincosf (not on a hot path)
-            const float u1 = ((float)(r.x >> 8) + 0.5f) * 5.9604644775390625e-08f, u2 = ((float)(r.z >> 8) + 0.5f) * 5.9604644775390625e-08f;
-            const float r1 = sqrtf(-2.0f * logf(u1)), r2 = sqrtf(-2.0f * logf(u2));
-            const float a1 = ((float)(r.y >> 8) * 5.9604644775390625e-08f - 0.5f) * 6.283185307179586f;
-            const float a2 = ((float)(r.w >> 8) * 5.9604644775390625e-08f - 0.5f) * 6.283185307179586f;
-            float s1, c1, s2, c2;
-            sincosf(a1, &s1, &c1);
-            sincosf(a2, &s2, &c2);
-            *reinterpret_cast<float4*>(zs + 4 * s) = make_float4(r1 * c1, r1 * s1, r2 * c2, r2 * s2);
-        }
+        for (int s = lane; s < Dp / 4; s += 32) *reinterpret_cast<float4*>(zs + 4 * s) = hmc_start_normal4(seed, gid, (uint32_t)s);
         __syncwarp();
         for (int j = lane; j < D; j += 32) {
             double v = q0[j];
@@ -222,6 +208,10 @@ extern "C" int hmc_start_pts(int32_t dtype, uint64_t seed, int64_t chain_id0, in
     long blocks = (Nchain + warps - 1) / warps;
     const long cap = (long)sm_count() * 16;
     if (blocks > cap) blocks = cap;
+    if (smem > 48 * 1024) {                          // (above D = 3072 the z rows need the opt-in to more than 48 KB)
+        HMC_CUDA_CHECK(cudaFuncSetAttribute(start_pts_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        HMC_CUDA_CHECK(cudaFuncSetAttribute(start_pts_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    }
     if (dtype == HMC_F32) start_pts_kernel<float><<<(int)blocks, warps * 32, smem, stream>>>(seed, chain_id0, Nchain, D, q0, Lc, sd, (float*)out);
     else start_pts_kernel<double><<<(int)blocks, warps * 32, smem, stream>>>(seed, chain_id0, Nchain, D, q0, Lc, sd, (double*)out);
     HMC_CUDA_CHECK(cudaGetLastError());

@@ -20,7 +20,8 @@ HMC_OK, HMC_E_BADARG, HMC_E_UNSUPPORTED, HMC_E_CUDA, HMC_E_DMAX = 0, 1, 2, 3, 4
 EXPORTS = ["hmc_random_run", "hmc_nuts_run", "hmc_diag_moments", "hmc_diag_variogram", "hmc_diag_short_series", "hmc_philox_draws",
            "hmc_ffma_peak", "hmc_version", "hmc_last_error_string", "hmc_start_pts", "hmc_summary_moments", "hmc_summary_hist",
            "hmc_summary_select", "hmc_random_workspace_bytes", "hmc_diag_variogram_all", "hmc_diag_variogram_all_workspace_bytes", "hmc_leap_frog",
-           "hmc_nuts_workspace_bytes"]
+           "hmc_nuts_workspace_bytes", "hmc_start_pts_workspace_bytes", "hmc_start_pts_bigd", "hmc_leap_frog_workspace_bytes",
+           "hmc_leap_frog_bigd"]
 
 
 class Target(C.Structure):
@@ -91,12 +92,22 @@ def load():
     lib.hmc_leap_frog.argtypes = [C.c_int32, C.POINTER(Target), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                   C.c_void_p]
     lib.hmc_leap_frog.restype = C.c_int
+    lib.hmc_leap_frog_workspace_bytes.argtypes = [C.POINTER(Target), C.c_int64, C.c_int32]
+    lib.hmc_leap_frog_workspace_bytes.restype = C.c_int64
+    lib.hmc_leap_frog_bigd.argtypes = [C.c_int32, C.POINTER(Target), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.hmc_leap_frog_bigd.restype = C.c_int
     lib.hmc_philox_draws.argtypes = [C.c_uint64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.hmc_philox_draws.restype = C.c_int
     lib.hmc_start_pts.argtypes = [C.c_int32, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.c_void_p]
     lib.hmc_start_pts.restype = C.c_int
+    lib.hmc_start_pts_workspace_bytes.argtypes = [C.c_int64, C.c_int32]
+    lib.hmc_start_pts_workspace_bytes.restype = C.c_int64
+    lib.hmc_start_pts_bigd.argtypes = [C.c_int32, C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.hmc_start_pts_bigd.restype = C.c_int
     lib.hmc_summary_moments.argtypes = [C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int64, C.c_int64,
                                         C.c_void_p, C.c_void_p]
     lib.hmc_summary_moments.restype = C.c_int
@@ -131,6 +142,12 @@ def check(rc):
 def ptr(t):
     """Device pointer of a torch tensor (or None)."""
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def aligned_workspace(torch, dev, nbytes):
+    """A new device workspace of nbytes, 1024-byte aligned (as the large-D entry points want it): (tensor that owns it, address)."""
+    buf = torch.empty((nbytes + 1024,), dtype=torch.uint8, device=dev)
+    return buf, (buf.data_ptr() + 1023) // 1024 * 1024
 
 
 def current_stream_ptr():

@@ -42,6 +42,12 @@ class MVNSpec(object):
         return cls(q0, np.linalg.inv(cov0), 0.5 * (D * np.log(2 * np.pi) + logdet))
 
 
+def leap_frog_entry(D):
+    """The library entry point ``HMC_sampler.leap_frog`` calls for dimension D: ``hmc_leap_frog`` (one warp per pair) up to
+    D = 1024, ``hmc_leap_frog_bigd`` (the large-D tensor-core GEMM, float32, D <= 8192) above."""
+    return "hmc_leap_frog" if D <= 1024 else "hmc_leap_frog_bigd"
+
+
 def equicorrelated_cov(D, rho):
     """cov0 of the reference's drivers: (1 - rho) I + rho 1 1^T (case3-script.py:31-33)."""
     return (1.0 - rho) * np.eye(D) + rho * np.ones((D, D))
@@ -377,8 +383,7 @@ class HMC_sampler(sampler):
     @staticmethod
     def _set_workspace(torch, dev, a, nbytes):
         """Point the launch arguments a at a new 1024-byte aligned device workspace of nbytes; returns the tensor that owns it."""
-        buf = torch.empty((nbytes + 1024,), dtype=torch.uint8, device=dev)
-        a.workspace = (buf.data_ptr() + 1023) // 1024 * 1024
+        buf, a.workspace = _L.aligned_workspace(torch, dev, nbytes)
         a.workspace_bytes = nbytes
         return buf
 
@@ -601,10 +606,12 @@ class HMC_sampler(sampler):
         return np.random.multivariate_normal(np.zeros(self.D), self.cov_p, size=1)
 
     def leap_frog(self, p_old, q_old, nsteps=1):
-        """One leapfrog step (samplers.py:831-839) -- on the GPU (``hmc_leap_frog``), for a single (p, q) pair or a batch of rows:
+        """One leapfrog step (samplers.py:831-839) -- on the GPU, for a single (p, q) pair or a batch of rows:
         p' = p - dt M^-1 dVdq(q) / 2, q' = q + dt p', p'' = p' - dt M^-1 dVdq(q') / 2, as the reference writes it (force times
         M^-1, q moved by p: Q9).  Returns (p_new, q_new) as float64 numpy arrays of the input's shape.  ``nsteps`` > 1 repeats the
-        step (this repo's extension)."""
+        step (this repo's extension).  D <= 1024 runs ``hmc_leap_frog``; above, float32 runs ``hmc_leap_frog_bigd`` on the large-D
+        GEMM (up to D = 8192, bf16x3 split unless tc_precision="fp16x2"; there nsteps > 1 merges the half kicks between steps, which
+        changes the last bits)."""
         import torch
         lib = _L.load()
         dev = torch.device("cuda", torch.cuda.current_device())
@@ -617,8 +624,16 @@ class HMC_sampler(sampler):
         pd = torch.from_numpy(np.ascontiguousarray(p2)).to(device=dev, dtype=tdt)
         qd = torch.from_numpy(np.ascontiguousarray(q2)).to(device=dev, dtype=tdt)
         pn, qn = torch.empty_like(pd), torch.empty_like(qd)
-        _L.check(lib.hmc_leap_frog(_L.HMC_F32 if self.dtype == "float32" else _L.HMC_F64, t, q2.shape[0], _L.ptr(pd), _L.ptr(qd),
-                                   _L.ptr(pn), _L.ptr(qn), int(nsteps), _L.current_stream_ptr()))
+        dtype = _L.HMC_F32 if self.dtype == "float32" else _L.HMC_F64
+        if leap_frog_entry(self.D) == "hmc_leap_frog":
+            _L.check(lib.hmc_leap_frog(dtype, t, q2.shape[0], _L.ptr(pd), _L.ptr(qd), _L.ptr(pn), _L.ptr(qn), int(nsteps),
+                                       _L.current_stream_ptr()))
+        else:
+            flags = self._fp16x2_flag()
+            nbytes = int(lib.hmc_leap_frog_workspace_bytes(t, q2.shape[0], flags)) if self.dtype == "float32" else 0
+            ws, ws_ptr = _L.aligned_workspace(torch, dev, nbytes) if nbytes else (None, None)
+            _L.check(lib.hmc_leap_frog_bigd(dtype, t, q2.shape[0], _L.ptr(pd), _L.ptr(qd), _L.ptr(pn), _L.ptr(qn), int(nsteps), flags,
+                                            ws_ptr, nbytes, _L.current_stream_ptr()))
         return pn.double().cpu().numpy().reshape(shape), qn.double().cpu().numpy().reshape(shape)
 
     def make_movie(self, title_prefix, q0=None, cov0=None, plot_cov=True, qmin=-3, qmax=3):

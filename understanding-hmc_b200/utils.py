@@ -284,13 +284,20 @@ def acceptance_rate(decision_chain, start=None, end=None):
     raise NotImplementedError("acceptance_rate is not part of the B200 hot-path build; use HMC_sampler.accept_R")
 
 
+def start_pts_entry(D):
+    """The library entry point ``start_pts(device=...)`` calls for dimension D: ``hmc_start_pts`` (one warp per chain) up to
+    D = 4096, ``hmc_start_pts_bigd`` (the large-D tensor-core GEMM, float32, D <= 8192) above."""
+    return "hmc_start_pts" if D <= 4096 else "hmc_start_pts_bigd"
+
+
 def start_pts(q0, cov0, size, device=None, seed=0, chain_id0=0, dtype="float32"):
     """Starting points ~ N(q0, cov0) (utils.py:204-209).
 
     Default (``device=None``): the reference's own call on the host, consuming the global ``np.random`` stream, so the
-    drivers reproduce their start points.  ``device="cuda"``: generated on the GPU (csrc/summary.cu, Philox keyed by
-    (seed, global chain id): independent of how chains are sharded) and returned as a CUDA tensor that
-    ``HMC_sampler.gen_sample`` takes as is -- no host draws, no H2D copy of Nchain x D values."""
+    drivers reproduce their start points.  ``device="cuda"``: generated on the GPU (Philox keyed by (seed, global chain id):
+    independent of how chains are sharded) and returned as a CUDA tensor that ``HMC_sampler.gen_sample`` takes as is -- no
+    host draws, no H2D copy of Nchain x D values.  Up to D = 4096 ``hmc_start_pts`` (csrc/summary.cu) makes them; above, up to
+    D = 8192 and in float32 only, ``hmc_start_pts_bigd`` (csrc/bigd_primitives.cu) from the same normals (start_pts_entry)."""
     if device is None:
         return np.random.multivariate_normal(q0, cov0, size=size)
     import torch
@@ -306,9 +313,16 @@ def start_pts(q0, cov0, size, device=None, seed=0, chain_id0=0, dtype="float32")
         Lc_d, fac = torch.from_numpy(np.ascontiguousarray(np.linalg.cholesky(cov0))).to(dev), None
     tdt = torch.float32 if dtype == "float32" else torch.float64
     out = torch.empty((int(size), D), dtype=tdt, device=dev)
+    dt_id = _L.HMC_F32 if tdt == torch.float32 else _L.HMC_F64
     with torch.cuda.device(dev):
-        _L.check(lib.hmc_start_pts(_L.HMC_F32 if tdt == torch.float32 else _L.HMC_F64, int(seed), int(chain_id0), int(size), D,
-                                   _L.ptr(q0_d), _L.ptr(Lc_d), _L.ptr(fac), _L.ptr(out), _L.current_stream_ptr()))
+        if start_pts_entry(D) == "hmc_start_pts":
+            _L.check(lib.hmc_start_pts(dt_id, int(seed), int(chain_id0), int(size), D, _L.ptr(q0_d), _L.ptr(Lc_d), _L.ptr(fac),
+                                       _L.ptr(out), _L.current_stream_ptr()))
+        else:                                      # (the workspace holds the GEMM operands: dense cov0 in float32 only)
+            nbytes = int(lib.hmc_start_pts_workspace_bytes(int(size), D)) if Lc_d is not None and tdt == torch.float32 else 0
+            ws, ws_ptr = _L.aligned_workspace(torch, dev, nbytes) if nbytes else (None, None)
+            _L.check(lib.hmc_start_pts_bigd(dt_id, int(seed), int(chain_id0), int(size), D, _L.ptr(q0_d), _L.ptr(Lc_d), _L.ptr(fac),
+                                            _L.ptr(out), ws_ptr, nbytes, _L.current_stream_ptr()))
     return out
 
 
