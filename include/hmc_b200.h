@@ -42,7 +42,8 @@ enum { HMC_F32 = 0, HMC_F64 = 1 };
 /* which kernel implements the run */
 enum {
     HMC_KERNEL_AUTO = 0,    /* tensor-core kernel if it covers the run, else the large-D GEMM path (when a workspace is given and
-                               D % 256 == 0 or D > 1024), else the FFMA2 kernel, else the generic one.  NUTS: the tensor-core kernel,
+                               D % 256 == 0 or D > 1024; with a dense momentum metric for D > 1024 only), else the FFMA2 kernel, else
+                               the generic one.  NUTS: the tensor-core kernel,
                                else the large-D path when a workspace is given, it covers the run and D > 256, else the generic one */
     HMC_KERNEL_GENERIC = 1, /* one warp per chain, any D <= 1024 (NUTS: D <= 256), float or double (parity workhorse) */
     HMC_KERNEL_FAST = 2,    /* FP32 FFMA2 register-tile kernel, 20 < D <= 128, identity momentum metric */
@@ -50,14 +51,19 @@ enum {
                                (smaller targets run zero padded in the 100-wide tile; AUTO picks it from D = 52), identity metric */
     HMC_KERNEL_BIGD = 4     /* large D, any 128 <= D <= 8192, float32, identity metric: one tcgen05 GEMM over all chains per leapfrog
                                step, operands by TMA, the leapfrog update fused into the epilogue; works on D rounded up to 32 (the
-                               padded dimensions stay zero); needs hmc_random_args.workspace.  NUTS too (hmc_nuts_args.workspace):
-                               the same GEMM writes the gradient rows and a step kernel advances every chain's tree by one point */
+                               padded dimensions stay zero); needs hmc_random_args.workspace.  The Random sampler also takes a dense
+                               momentum metric (target.Pt, Mit and Lct) for 1024 < D <= 8192: the steps multiply by F = M^-1 P as
+                               always, and V, K and the momentum draw p = Lc z are batched tensor-core products (bf16x3) of the chains
+                               that end or start a trajectory in a pass.  Up to D = 1024 the generic kernel runs a dense metric, and
+                               this path refuses it there.  NUTS too (hmc_nuts_args.workspace, identity metric only): the same GEMM
+                               writes the gradient rows and a step kernel advances every chain's tree by one point */
 };
 
 /* hmc_random_args.flags, hmc_nuts_args.flags */
 enum {
     HMC_FLAG_UNIFORM_DT = 1, /* every entry of target.dt is equal (lets the fused kernels fold dt into constants) */
-    HMC_FLAG_TC_FP16X2 = 2   /* tensor-core kernels (NUTS: the large-D path only): the caller vouches that |q - mu| stays below ~1.6e4 and that the target's
+    HMC_FLAG_TC_FP16X2 = 2   /* tensor-core kernels (NUTS: the large-D path only; with a dense metric on the large-D path it selects the
+                                split of the gradient passes only -- V, K and Lc z always use bf16x3): the caller vouches that |q - mu| stays below ~1.6e4 and that the target's
                                 scale is not far below 1 (no component of interest under 2^-14), which lets the gradient
                                 product use the two-part fp16 split (3 tensor passes, FP32-grade) instead of the three-part
                                 bf16 split (6 passes); a trajectory that leaves the fp16 range ends in a rejection */
@@ -71,7 +77,8 @@ enum {
  *   Pt  [D][D_pad]  transpose of the precision matrix P, or NULL when M = I (then F == P)
  *   Mit [D][D_pad]  transpose of M^-1 = inv(cov_p), or NULL when M = I       (K, samplers.py:811-817)
  *   Lct [D][D_pad]  transpose of a factor Lc with Lc Lc^T = cov_p (p = Lc z), or NULL when M = I
- *                   (p_sample, samplers.py:825-829; only used when momenta come from Philox)
+ *                   (p_sample, samplers.py:825-829; only used when momenta come from Philox).  Mit must be inv(Lc Lc^T): the
+ *                   large-D path relies on it for K(p0) = p0^T M^-1 p0 / 2 = z^T z / 2 of a Philox draw (no product)
  *   mu  [D_pad]     target mean q0
  *   dt  [D_pad]     per-dimension time step (a scalar dt is broadcast by the host; samplers.py:333)
  *   v_const         0.5 (D ln 2pi + ln det cov0), the constant of -logpdf (utils.py:213-218)
@@ -165,7 +172,10 @@ typedef struct hmc_random_args {
 
 int hmc_random_run(const hmc_random_args* args, void* cuda_stream);
 /* bytes of hmc_random_args.workspace the large-D path needs for this configuration: non-zero exactly for the runs it covers
-   (float32, identity metric, 128 <= D <= 8192), whatever kernel is asked for; 0 otherwise.  Depends on Nchain and D only. */
+   (float32; identity metric and 128 <= D <= 8192, or a dense metric -- Pt, Mit and Lct all given -- and 1024 < D <= 8192), whatever
+   kernel is asked for; 0 otherwise.  Depends on Nchain, D and whether the metric is dense.  A dense metric adds the products'
+   operands and results: 9 Ncp Dp x 2 B of split rows, 9 Dp^2 x 2 B of split matrices, 3 Ncp Dp x 4 B of products (Ncp = Nchain
+   rounded up to 512, Dp = D rounded up to 32): about 33 GB on top of the identity size's ~26 GB at 131,072 chains and D = 8192. */
 int64_t hmc_random_workspace_bytes(const hmc_random_args* args);
 
 /*

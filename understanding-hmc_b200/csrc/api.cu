@@ -77,7 +77,8 @@ extern "C" int hmc_random_run(const hmc_random_args* args, void* cuda_stream) {
     // gradient-evals/s; the FFMA kernel's rate grows as 1/D^2 and overtakes it below D ~ 50), then the large-D GEMM path, then
     // the FFMA kernel, then the generic one.  The large-D path covers every 128 <= D <= 8192; AUTO takes it for D % 256 == 0
     // (unpadded tiles) and for D > 1024 (beyond the generic kernel), and leaves 128 < D <= 1024 otherwise to the generic kernel
-    // (HMC_KERNEL_BIGD reaches the padded path there)
+    // (HMC_KERNEL_BIGD reaches the padded path there).  A dense momentum metric is covered for D > 1024 only, so AUTO keeps it on
+    // the generic kernel up to D = 1024
     if (kernel == HMC_KERNEL_AUTO)
         kernel = (a.target.D >= 52 && hmc_random_tc_supported(a, &why)) ? HMC_KERNEL_TC
                  : (a.workspace && hmc_random_bigd_supported(a, &why) && (a.target.D % 256 == 0 || a.target.D > 1024)) ? HMC_KERNEL_BIGD

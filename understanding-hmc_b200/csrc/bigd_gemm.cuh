@@ -510,10 +510,18 @@ static_assert(gemm_smem_bytes<2, 256, 32, (NEPI == 4 ? 3 : 2)>() <= 232448 && ge
 // alike), kernels and pass loop; `name` is the path's name in error messages.
 // =====================================================================================================================
 
-// the runs the large-D path covers (the `why` strings end up in error messages)
-bool bigd_covers(int dtype, const hmc_target& t, int iter_begin, int iter_end, const char** why) {
+// the runs the large-D path covers (the `why` strings end up in error messages).  A dense momentum metric (target.Pt, Mit and
+// Lct, all three) only where the caller has it (`dense`: the Random sampler) and only for D > 1024: up to D = 1024 the generic
+// kernel runs it, and that stays so
+bool bigd_covers(int dtype, const hmc_target& t, int iter_begin, int iter_end, const char** why, bool dense = false) {
     if (dtype != HMC_F32) { *why = "float32 only"; return false; }
-    if (t.Mit || t.Pt || t.Lct) { *why = "identity momentum metric only"; return false; }
+    const bool metric = t.Mit || t.Pt || t.Lct;
+    if (metric && !dense) { *why = "identity momentum metric only"; return false; }
+    if (metric && t.D <= 1024) {
+        *why = "identity momentum metric only for D <= 1024 (the generic kernel runs a dense metric there)";
+        return false;
+    }
+    if (metric && !(t.Mit && t.Pt && t.Lct)) { *why = "a dense momentum metric needs target.Pt, Mit and Lct together"; return false; }
     if (t.D < 128 || t.D > 8192) { *why = "D must be in [128, 8192]"; return false; }
     if (iter_end <= iter_begin) { *why = "needs at least one iteration"; return false; }
     return true;

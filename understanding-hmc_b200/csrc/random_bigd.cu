@@ -148,8 +148,11 @@ __global__ void __launch_bounds__(128) bigd_init(hmc_random_args a, BigdWs w) {
     }
 }
 
-// per-chain bookkeeping after a pass (one thread per chain, one block per 128-chain tile)
-__global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, int pass) {
+// per-chain bookkeeping after a pass (one thread per chain, one block per 128-chain tile).  DENSE (a dense momentum metric): V at
+// a trajectory start is the carried V0 (V(x) != x.(F x) / 2 there), and a chain that ends its trajectory only goes on the list --
+// its energies need the metric products, and bigd_finish decides
+template <bool DENSE>
+__global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, int pass, const float* __restrict__ V0) {
     const long m = (long)blockIdx.x * BM + threadIdx.x;                              // row (the grid covers the Ncp rows exactly)
     const int Dp = w.Dp;
     const long Lc = 1 + (a.Niter - a.warm_up_num) / a.thin_rate;
@@ -159,9 +162,13 @@ __global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, i
     const long c = w.perm[m];                                                        // chain of this row: indexes the outputs
     unsigned long long acc_warm = 0, acc_post = 0, sL = 0, sL2 = 0;
     if (md == MD_FIRST || md == MD_MID || md == MD_LAST) {
-        float hv = 0.f, hk = 0.f;
-        for (int t = 0; t < 2 * w.NT; ++t) { hv += w.red[((size_t)m * 2 * w.NT + t) * 2]; hk += w.red[((size_t)m * 2 * w.NT + t) * 2 + 1]; }
-        const float V = fmaf(0.5f * w.binv, hv, (float)a.target.v_const);           // V(q) at the point the gradient was taken
+        float hv = 0.f, hk = 0.f, V;
+        if constexpr (DENSE) {
+            V = md == MD_FIRST ? V0[m] : 0.f;
+        } else {
+            for (int t = 0; t < 2 * w.NT; ++t) { hv += w.red[((size_t)m * 2 * w.NT + t) * 2]; hk += w.red[((size_t)m * 2 * w.NT + t) * 2 + 1]; }
+            V = fmaf(0.5f * w.binv, hv, (float)a.target.v_const);                   // V(q) at the point the gradient was taken
+        }
         const int it = w.it[m];
         const bool tr = a.phi_q && (a.chain_id0 + c) == 0 && it <= a.N_save_chain0;
         const float* mu = w.mu;
@@ -196,6 +203,9 @@ __global__ void __launch_bounds__(BM) bigd_events(hmc_random_args a, BigdWs w, i
             }
             w.l[m] = l;
             if (l == w.L[m]) md = MD_LAST;
+        } else if constexpr (DENSE) {
+            w.list[atomicAdd(&w.counters[pass & 1], 1)] = (int)m;
+            md = MD_PENDING;
         } else {                                                                    // Metropolis accept (samplers.py:455-472)
             const float Ei = w.E_init[m];
             const float dE = (V + 0.5f * hk) - Ei;
@@ -278,6 +288,167 @@ __global__ void __launch_bounds__(256) bigd_trajectory_end(hmc_random_args a, Bi
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------------
+// Dense momentum metric (target.Pt, Mit, Lct; 1024 < D <= 8192).  The passes do not change: the main GEMM multiplies by the force
+// matrix F = M^-1 P, which is all a leapfrog step needs (q moves by p: quirk Q9).  What a dense metric adds is at the ends of a
+// trajectory: V(x) = x.(P x) / 2 + v_const, K(p) = p.(M^-1 p) / 2 and the momentum draw p = Lc z.  They are three batched products on
+// the tensor cores (the EPI_GRAD GEMM, bf16x3 split whatever the pass split is: x, p and z are not bounded the way the fp16 split
+// needs), over the chains that ended a trajectory in the pass, gathered into compact rows:
+//   bigd_gather    one warp per listed chain: x = (x + mu) - mu (the x a resume from the stored float row sees, so that iteration
+//                  blocks equal one launch), its split row (segment 0, times P), the split p_L (segment 1, times M^-1), the split
+//                  next momentum (segment 2: z times Lc on Philox draws, the tape row times M^-1 on tapes); the row blocks below
+//                  the list length for the products
+//   3 x bigd_gemm_step<MetricWs, EPI_GRAD>  over the full capacity, idle row blocks skipped
+//   bigd_finish    one warp per listed chain: V(x_L), K(p_L), the Metropolis test, then bigd_trajectory_end's work; the next momentum
+//                  p0 = Lc z (or the tape row) with K(p0) = z.z / 2 on Philox draws (Lc Lc^T = cov_p = M, so p0.(M^-1 p0) = z.z
+//                  exactly) and p0.(M^-1 p0) / 2 on tapes.  V(x0) is carried: V(x_L) after an accept, the old V0 after a reject.
+// The chain start (or resume) runs the same three kernels once over every chain (`start`): V(x0), on tapes K of the iteration-0 row
+// and of the first momentum, and p0 = Lc z of the first iteration (bigd_init has drawn z, L and the uniform).
+// ---------------------------------------------------------------------------------------------------------------------------
+struct MetricWs {                    // the products' workspace (the fields the GEMM reads are named as in BigdWs)
+    uint16_t* xp;                    // [3 segments][3 parts][Ncp][Dp]  split rows, row e = list entry e (A operand)
+    uint16_t* bp;                    // [3 segments][3 parts][Dp][Dp]   split P, M^-1 and Lc (tapes: M^-1 again) (B operand)
+    float* g;                        // [3 segments][Ncp][Dp]           the products
+    int* mode;                       // [Ncp] MD_FIRST: every row of an active row block is stored (rows past the list are not read)
+    int* tile_active;                // [Ncp / 128] row blocks below the list length
+    float* V0;                       // [Ncp] by workspace row: V(x0) of the running trajectory
+    float binv;                      // 1: the bf16 split is not scaled
+    int Ncp, NT, Dp;
+};
+
+size_t carve_metric(MetricWs& mw, unsigned char* ws, size_t off, long Nchain, int D) {
+    BigdCarve c(ws, Nchain, D, 128);
+    c.off = off;
+    mw.Ncp = (int)c.Ncp; mw.NT = c.NT; mw.Dp = c.Dp; mw.binv = 1.f;
+    mw.xp = (uint16_t*)c.take((size_t)9 * c.Ncp * c.Dp * 2);
+    mw.bp = (uint16_t*)c.take((size_t)9 * c.Dp * c.Dp * 2);
+    mw.g = (float*)c.take((size_t)3 * c.Ncp * c.Dp * 4);
+    mw.mode = (int*)c.take(c.Ncp * 4);
+    mw.tile_active = (int*)c.take((c.Ncp / BM) * 4);
+    mw.V0 = (float*)c.take(c.Ncp * 4);
+    return c.off;
+}
+
+__device__ __forceinline__ float row_dot(const float* u, const float* v, int Dp, int lane) {
+    float s = 0.f;
+    for (int j = lane; j < Dp; j += 32) s = fmaf(u[j], v[j], s);
+    return warp_sum<float>(s);
+}
+
+__global__ void __launch_bounds__(256) bigd_gather(hmc_random_args a, BigdWs w, MetricWs mw, int pass, int start) {
+    const int lane = threadIdx.x & 31, D = a.target.D, Dp = w.Dp;
+    const int n = start ? a.Nchain : w.counters[pass & 1];
+    const long nthr = (long)gridDim.x * blockDim.x;
+    for (long t = (long)blockIdx.x * blockDim.x + threadIdx.x; t < mw.Ncp; t += nthr) {
+        if (start) mw.mode[t] = MD_FIRST;
+        if (t < mw.Ncp / BM) mw.tile_active[t] = t * BM < n;
+    }
+    const size_t seg = (size_t)3 * mw.Ncp * Dp;
+    for (int e = blockIdx.x * 8 + (threadIdx.x >> 5); e < n; e += gridDim.x * 8) {
+        const long m = start ? e : (w.list[e] & 0x7fffffff);
+        const long c = w.perm[m];
+        float* xr = w.x + (size_t)m * Dp;
+        float* pr = w.p + (size_t)m * Dp;
+        const int it = w.it[m];
+        if (!start)
+            for (int j = lane; j < Dp; j += 32) xr[j] = (xr[j] + w.mu[j]) - w.mu[j];
+        bigd_write_parts<3>(mw.xp, mw.Ncp, Dp, e, lane, xr);
+        // the momentum rows: at the start, the iteration-0 tape row (its K enters E_chain[., 0]) and p of the first iteration as
+        // bigd_init drew it; at a trajectory end, p_L and the draw of the next iteration (none after the last).  A drawn row is
+        // staged in the segment's product row, which the GEMM overwrites
+        const bool fresh_tape = start && a.iter_begin == 0 && a.p_tape;
+        if (!start || fresh_tape) {
+            float* g1 = mw.g + ((size_t)mw.Ncp + e) * Dp;
+            if (fresh_tape) bigd_momentum(a.p_tape + (size_t)c * (a.Niter + 1) * D, a.seed, 0, 0, D, Dp, lane, g1, D / 4);
+            bigd_write_parts<3>(mw.xp + seg, mw.Ncp, Dp, e, lane, start ? g1 : pr);
+        }
+        if (start) {
+            bigd_write_parts<3>(mw.xp + 2 * seg, mw.Ncp, Dp, e, lane, pr);
+        } else if (it < a.iter_end) {
+            float* g2 = mw.g + (2 * (size_t)mw.Ncp + e) * Dp;
+            const double* tape = a.p_tape ? a.p_tape + ((size_t)c * (a.Niter + 1) + it + 1) * D : nullptr;
+            bigd_momentum(tape, a.seed, (uint64_t)(a.chain_id0 + c), it + 1, D, Dp, lane, g2, D / 4);
+            bigd_write_parts<3>(mw.xp + 2 * seg, mw.Ncp, Dp, e, lane, g2);
+        }
+    }
+}
+
+template <int NPART>
+__global__ void __launch_bounds__(256) bigd_finish(hmc_random_args a, BigdWs w, MetricWs mw, int pass, int start) {
+    const int lane = threadIdx.x & 31, D = a.target.D, Dp = w.Dp;
+    const int n = start ? a.Nchain : w.counters[pass & 1];
+    const long Lc = 1 + (a.Niter - a.warm_up_num) / a.thin_rate;
+    const long Lrow = a.store_ring > 0 ? a.store_ring : Lc;
+    const float* mu = w.mu;
+    const float vc = (float)a.target.v_const;
+    for (int e = blockIdx.x * 8 + (threadIdx.x >> 5); e < n; e += gridDim.x * 8) {
+        const long m = start ? e : (w.list[e] & 0x7fffffff);
+        const long c = w.perm[m];
+        const float* gP = mw.g + (size_t)e * Dp;
+        const float* gM = mw.g + ((size_t)mw.Ncp + e) * Dp;
+        const float* gN = mw.g + (2 * (size_t)mw.Ncp + e) * Dp;
+        float* xr = w.x + (size_t)m * Dp;
+        float* x0r = w.x0 + (size_t)m * Dp;
+        float* pr = w.p + (size_t)m * Dp;
+        const float V = fmaf(0.5f, row_dot(xr, gP, Dp, lane), vc);                 // V(x_L), or V(x0) at the start
+        // p0 of a new trajectory: Lc z from its product on Philox draws (K = z.z / 2 given), the tape row in pr with K from M^-1 p0
+        auto momentum = [&](float Kz) {
+            if (a.p_tape) return 0.5f * row_dot(pr, gN, Dp, lane);
+            for (int j = lane; j < Dp; j += 32) pr[j] = gN[j];
+            return Kz;
+        };
+        if (start) {
+            float K0 = 0.f;
+            if (a.p_tape && a.iter_begin == 0) {                                    // K of the iteration-0 tape row (samplers.py:415)
+                const double* t0 = a.p_tape + (size_t)c * (a.Niter + 1) * D;
+                float s = 0.f;
+                for (int j = lane; j < D; j += 32) s = fmaf((float)t0[j], gM[j], s);
+                K0 = 0.5f * warp_sum<float>(s);
+            }
+            const float Kn = momentum(w.K_new[m]);
+            if (lane == 0) { mw.V0[m] = V; w.K_new[m] = Kn; if (a.p_tape && a.iter_begin == 0) w.K0[m] = K0; }
+            continue;
+        }
+        const float K = 0.5f * row_dot(pr, gM, Dp, lane);                          // samplers.py:455
+        int it = w.it[m];
+        const float Ei = w.E_init[m];
+        const float dE = (V + K) - Ei;
+        const bool accepted = (dE < 0.f) || (w.lnu[m] < -dE);                       // samplers.py:462
+        const bool keep = it >= a.warm_up_num;
+        const bool last = it >= a.iter_end;
+        if (lane == 0) {
+            w.E_prev[m] = Ei;                                                       // samplers.py:460
+            if (accepted) mw.V0[m] = V;
+            if (accepted && a.counters) atomicAdd(a.counters + (keep ? 1 : 0), 1ull);
+            if (a.phi_q && (a.chain_id0 + c) == 0 && it <= a.N_save_chain0) a.decision_chain[it - 1] = accepted ? 1 : 0;
+        }
+        float* dst = keep ? (float*)a.q_chain + ((size_t)c * Lrow + ((it - a.warm_up_num) / a.thin_rate) % Lrow) * D : nullptr;
+        float* sq = last ? (float*)a.state_q + (size_t)c * D : nullptr;
+        // accepted: start point <- proposal (samplers.py:463-469); rejected: proposal <- start point (samplers.py:470-472)
+        const float* from = accepted ? xr : x0r;
+        float* to = accepted ? x0r : xr;
+        for (int j = lane; j < Dp; j += 32) {
+            const float v = from[j];
+            to[j] = v;
+            if (j < D) {
+                if (dst) dst[j] = v + mu[j];
+                if (sq) sq[j] = v + mu[j];
+            }
+        }
+        // the next pass's operand: x0 (the pass wrote x_L before its re-derivation)
+        bigd_write_parts<NPART>(w.xp + (size_t)w.wr * NPART * w.Ncp * Dp, w.Ncp, Dp, m, lane, x0r);
+        if (last) {
+            if (lane == 0) { w.mode[m] = MD_IDLE; w.it[m] = it + 1; a.state_eprev[c] = (double)Ei; }
+        } else {
+            it += 1;
+            int L = 1; float lnu = 0.f;
+            const float Kz = bigd_draw(a, Dp, c, it, lane, a.p_tape ? pr : nullptr, &L, &lnu);   // samplers.py:431, 441, 461
+            const float Kn = momentum(Kz);
+            if (lane == 0) { w.K_new[m] = Kn; w.L[m] = L; w.lnu[m] = lnu; w.l[m] = 0; w.it[m] = it; w.mode[m] = MD_FIRST; }
+        }
+    }
+}
+
 
 // carve the workspace; returns the bytes needed (ws may be NULL to only size it)
 size_t carve(BigdWs& w, unsigned char* ws, long Nchain, int D, int npart, int bn) {
@@ -309,8 +480,11 @@ constexpr const char* kName = "large-D kernel";
 template <int NPART, int BN, int CL, int BK, int STAGES>
 int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
     const int D = a.target.D;
+    const bool dense = a.target.Pt != nullptr;                   // (with Mit and Lct: hmc_random_bigd_supported)
     BigdWs w;
-    const size_t need = carve(w, (unsigned char*)a.workspace, a.Nchain, D, NPART, BN);
+    MetricWs mw{};
+    size_t need = carve(w, (unsigned char*)a.workspace, a.Nchain, D, NPART, BN);
+    if (dense) need = carve_metric(mw, (unsigned char*)a.workspace, need, a.Nchain, D);
     if (int rc = bigd_check_workspace(a.workspace, a.workspace_bytes, need, kName, "hmc_random_workspace_bytes")) return rc;
     int dev = 0, sms = 0;
     HMC_CUDA_CHECK(cudaGetDevice(&dev));
@@ -325,6 +499,37 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
     }
     if (int rc = make_map(&mapP, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.p, (uint64_t)w.Ncp, Dp, CW, 32)) return rc;
     if (int rc = make_map(&mapX, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w.x, (uint64_t)w.Ncp, Dp, CW, 32)) return rc;
+    // dense metric: the three products' operands and GEMM (bf16x3, 128-column tiles, clusters of two row blocks)
+    constexpr int MCL = 2;
+    auto mkern = bigd_gemm_step<MetricWs, EPI_GRAD, 3, 128, MCL, 32, 2>;
+    CUtensorMap mapMA[3], mapMB[3], mapMG[3];
+    cudaLaunchConfig_t mcfg;
+    cudaLaunchAttribute mattr;
+    if (dense) {
+        const void* mats[3] = {a.target.Pt, a.target.Mit, a.p_tape ? a.target.Mit : a.target.Lct};
+        for (int sg = 0; sg < 3; ++sg) {
+            uint16_t* xs = mw.xp + (size_t)sg * 3 * mw.Ncp * Dp;
+            uint16_t* bs = mw.bp + (size_t)sg * 3 * Dp * Dp;
+            bigd_split_matrix<3><<<sms * 8, 256, 0, stream>>>((const float*)mats[sg], D, a.target.D_pad, Dp, 1.f, bs);
+            if (int rc = make_map(&mapMA[sg], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, xs, (uint64_t)3 * mw.Ncp, Dp, 32, BM)) return rc;
+            if (int rc = make_map(&mapMB[sg], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, bs, (uint64_t)3 * Dp, Dp, 32, 128 / MCL)) return rc;
+            if (int rc = make_map(&mapMG[sg], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, mw.g + (size_t)sg * mw.Ncp * Dp, (uint64_t)mw.Ncp, Dp, CW, 32))
+                return rc;
+        }
+        if (int rc = bigd_launch_config(mcfg, mattr, mkern, MCL, (mw.Ncp / BM / MCL) * mw.NT, gemm_smem_bytes<3, 128, 32, 2>(), sms, stream,
+                                        kName)) return rc;
+    }
+    // the list's per-trajectory products (`pass`: the list of that pass; start: every chain) up to the finish kernel, split in two
+    // by the timing event `mid`
+    auto metric_stage = [&](long pass, int start, cudaEvent_t mid) {
+        bigd_gather<<<sms * 2, 256, 0, stream>>>(a, w, mw, (int)pass, start);
+        for (int sg = 0; sg < 3; ++sg)
+            if (cudaLaunchKernelEx(&mcfg, mkern, mapMA[sg], mapMB[sg], mapMG[sg], mapMG[sg], mapMG[sg], mw, mw.Ncp, Dp, (const float*)nullptr) !=
+                cudaSuccess) return HMC_E_CUDA;
+        if (mid) cudaEventRecord(mid, stream);
+        bigd_finish<NPART><<<sms * 2, 256, 0, stream>>>(a, w, mw, (int)pass, start);
+        return HMC_OK;
+    };
     w.wr = 0;                                                    // pass 0 reads buffer 0
     try {   // rows = chains sorted by planned passes, longest first (stable: equal plans keep the chain order); padding rows last
         bigd_plan<<<(a.Nchain + 255) / 256, 256, 0, stream>>>(a, w.plan);
@@ -341,6 +546,7 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
         return HMC_E_CUDA;
     }
     bigd_init<NPART><<<(w.Ncp + 3) / 4, 128, 0, stream>>>(a, w);
+    if (dense) if (int rc = metric_stage(0, 1, nullptr)) return bigd_loop_result(rc, kName);
     const int ntile_rows = w.Ncp / BM;
     HMC_CUDA_CHECK(cudaMemsetAsync(w.tile_active, 0xff, (size_t)ntile_rows * 4, stream));
     auto kern = bigd_gemm_step<BigdWs, EPI_LEAPFROG, NPART, BN, CL, BK, STAGES>;
@@ -357,26 +563,36 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
     if (int rc = running.alloc()) return rc;
     const long max_pass = (long)(a.iter_end - a.iter_begin) * (a.L_high + 1) + 8;
     int rc = HMC_OK;
-    // HMC_B200_BIGD_TIMING=1: CUDA-event times of the three kernels of passes 4..11 on stderr (measurement aid)
+    // HMC_B200_BIGD_TIMING=1: CUDA-event times of the kernels of passes 4..11 on stderr (measurement aid); with a dense metric
+    // the trajectory end is split into the product stage (gather + three GEMMs) and the finish kernel
     const bool timing = getenv("HMC_B200_BIGD_TIMING") != nullptr;
-    cudaEvent_t ev[4];
-    float tsum[3] = {0.f, 0.f, 0.f};
-    if (timing) for (int i = 0; i < 4; ++i) cudaEventCreate(&ev[i]);
+    const int nst = dense ? 4 : 3;
+    cudaEvent_t ev[5];
+    float tsum[4] = {0.f, 0.f, 0.f, 0.f};
+    if (timing) for (int i = 0; i <= nst; ++i) cudaEventCreate(&ev[i]);
     for (long pass = 0; pass < max_pass; ++pass) {
         const bool timed = timing && pass >= 4 && pass < 12;
         if (timed) cudaEventRecord(ev[0], stream);
         if (launch_gemm(pass) != cudaSuccess) { rc = HMC_E_CUDA; break; }
         if (timed) cudaEventRecord(ev[1], stream);
         cudaMemsetAsync(w.counters + 2, 0, 4, stream);
-        bigd_events<<<ntile_rows, BM, 0, stream>>>(a, w, (int)pass);
-        if (timed) cudaEventRecord(ev[2], stream);
-        bigd_trajectory_end<NPART><<<sms * 2, 256, 0, stream>>>(a, w, (int)pass);
+        if (dense) {
+            bigd_events<true><<<ntile_rows, BM, 0, stream>>>(a, w, (int)pass, mw.V0);
+            if (timed) cudaEventRecord(ev[2], stream);
+            if ((rc = metric_stage(pass, 0, timed ? ev[3] : nullptr)) != HMC_OK) break;
+        } else {
+            bigd_events<false><<<ntile_rows, BM, 0, stream>>>(a, w, (int)pass, nullptr);
+            if (timed) cudaEventRecord(ev[2], stream);
+            bigd_trajectory_end<NPART><<<sms * 2, 256, 0, stream>>>(a, w, (int)pass);
+        }
         if (timed) {
-            cudaEventRecord(ev[3], stream);
-            cudaEventSynchronize(ev[3]);
-            for (int i = 0; i < 3; ++i) { float ms = 0.f; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); tsum[i] += ms; }
-            if (pass == 11) fprintf(stderr, "[bigd timing] NPART=%d BN=%d BK=%d cluster=%d chains=%d D=%d: gemm_step %.3f ms, events %.3f ms, trajectory_end %.3f ms per pass (%d work items on %d CTAs)\n",
+            cudaEventRecord(ev[nst], stream);
+            cudaEventSynchronize(ev[nst]);
+            for (int i = 0; i < nst; ++i) { float ms = 0.f; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); tsum[i] += ms; }
+            if (pass == 11 && !dense) fprintf(stderr, "[bigd timing] NPART=%d BN=%d BK=%d cluster=%d chains=%d D=%d: gemm_step %.3f ms, events %.3f ms, trajectory_end %.3f ms per pass (%d work items on %d CTAs)\n",
                                     NPART, BN, BK, CL, a.Nchain, D, tsum[0] / 8, tsum[1] / 8, tsum[2] / 8, ntiles, (int)cfg.gridDim.x);
+            if (pass == 11 && dense) fprintf(stderr, "[bigd timing] NPART=%d BN=%d BK=%d cluster=%d chains=%d D=%d dense metric: gemm_step %.3f ms, events %.3f ms, products %.3f ms, finish %.3f ms per pass (%d work items on %d CTAs)\n",
+                                             NPART, BN, BK, CL, a.Nchain, D, tsum[0] / 8, tsum[1] / 8, tsum[2] / 8, tsum[3] / 8, ntiles, (int)cfg.gridDim.x);
         }
         if ((pass & 7) == 7) {
             // chains that ended their last trajectory in this pass are still MD_PENDING for the events kernel's count: they are
@@ -386,19 +602,21 @@ int run_bigd(const hmc_random_args& a, cudaStream_t stream) {
             if (n == 0) break;
         }
     }
-    if (timing) for (int i = 0; i < 4; ++i) cudaEventDestroy(ev[i]);
+    if (timing) for (int i = 0; i <= nst; ++i) cudaEventDestroy(ev[i]);
     return bigd_loop_result(rc, kName);
 }
 
 }  // namespace
 
 bool hmc_random_bigd_supported(const hmc_random_args& a, const char** why) {
-    return bigd_covers(a.dtype, a.target, a.iter_begin, a.iter_end, why);
+    return bigd_covers(a.dtype, a.target, a.iter_begin, a.iter_end, why, true);
 }
 
 size_t hmc_random_bigd_workspace(const hmc_random_args& a) {
     BigdWs w;                                     // sized for the larger of the two variants
-    return carve(w, nullptr, a.Nchain, a.target.D, 3, 128);
+    MetricWs mw;
+    const size_t n = carve(w, nullptr, a.Nchain, a.target.D, 3, 128);
+    return a.target.Pt ? carve_metric(mw, nullptr, n, a.Nchain, a.target.D) : n;
 }
 
 int hmc_random_run_bigd(const hmc_random_args& a, cudaStream_t stream) {

@@ -48,6 +48,17 @@ def leap_frog_entry(D):
     return "hmc_leap_frog" if D <= 1024 else "hmc_leap_frog_bigd"
 
 
+def random_runs_bigd(D, dtype, kernel, cov_p_identity):
+    """Whether the random-trajectory sampler runs on the large-D GEMM path (csrc/api.cu's AUTO rule and the path's coverage):
+    float32 and 128 <= D <= 8192 with the identity metric, under kernel="bigd", or under "auto" for D % 256 == 0 and D > 1024;
+    a dense ``cov_p`` for 1024 < D <= 8192 under "bigd" or "auto" (up to D = 1024 the generic kernel runs a dense metric)."""
+    if dtype != "float32" or kernel not in ("auto", "bigd") or not 128 <= D <= 8192:
+        return False
+    if not cov_p_identity:
+        return D > 1024
+    return kernel == "bigd" or D % 256 == 0 or D > 1024
+
+
 def equicorrelated_cov(D, rho):
     """cov0 of the reference's drivers: (1 - rho) I + rho 1 1^T (case3-script.py:31-33)."""
     return (1.0 - rho) * np.eye(D) + rho * np.ones((D, D))
@@ -203,9 +214,12 @@ class sampler(object):
 class HMC_sampler(sampler):
     """HMC sampler for multivariate-normal targets (samplers.py:297-384), CUDA backed.
 
-    ``kernel`` of the random-trajectory sampler (float32, ``cov_p = I`` unless noted; "auto" picks as csrc/api.cu does):
+    ``kernel`` of the random-trajectory sampler (float32, ``cov_p = I`` unless noted; "auto" picks as csrc/api.cu does,
+    ``random_runs_bigd`` is the large-D rule):
       "tc"       tensor-core kernel, D % 4 == 0, D <= 100 (zero-padded 100-wide tile); auto for 52 <= D <= 100
-      "bigd"     large-D GEMM path, any 128 <= D <= 8192 (padded to D rounded up to 32); auto for D % 256 == 0 and D > 1024
+      "bigd"     large-D GEMM path, any 128 <= D <= 8192 (padded to D rounded up to 32); auto for D % 256 == 0 and D > 1024.
+                 A dense ``cov_p`` for 1024 < D <= 8192 (auto there too): its V, K and p = Lc z are batched tensor-core products
+                 at the trajectory ends
       "fast"     FFMA2 kernel, 20 < D <= 128; auto where neither of the above applies
       "generic"  warp-per-chain kernel, D <= 1024, float64 and dense ``cov_p`` too; auto for the rest
 
@@ -418,8 +432,7 @@ class HMC_sampler(sampler):
         a.seed = self.seed
         a.target = tgt
         a.flags = _L.FLAG_UNIFORM_DT if np.ndim(self.dt) == 0 or np.all(np.asarray(self.dt) == np.asarray(self.dt).flat[0]) else 0
-        bigd = self.dtype == "float32" and self._cov_p_identity and 128 <= D <= 8192 and \
-            (self.kernel == "bigd" or (self.kernel == "auto" and (D % 256 == 0 or D > 1024)))     # csrc/api.cu AUTO rule
+        bigd = random_runs_bigd(D, self.dtype, self.kernel, self._cov_p_identity)
         if self.tc_precision is None:
             self.tc_precision = "fp16x2" if bigd else "bf16x3"
         # (the fp16 split also needs |q - mu| < 16384: the tensor-core kernel checks it, word 16 + Nchain of state_g)
