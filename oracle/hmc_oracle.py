@@ -389,7 +389,11 @@ def gen_sample_NUTS(D, V, dVdq, q_start, draws, Nchain, Niter, thin_rate=1, warm
     ``on_dmax="stop"`` is this repo's benchmark extension (SURVEY H6): depth overflow ends the doubling
     loop keeping the live point, instead of aborting the whole run.
     With ``record`` the per-chain structured tapes are kept: p_tape[Nchain, Niter+1, D], and per chain the
-    flat lists dir_tape / u_tape in consumption order, plus n_leapfrog[Nchain, Niter] and depth[Nchain, Niter].
+    flat lists dir_tape / u_tape in consumption order, plus n_leapfrog[Nchain, Niter] and depth[Nchain, Niter], and per
+    (chain, iteration) what the tree builder met: n_instab_iter (|E - E_initial| > 1000 rejects), n_uturn_sub_iter
+    (sub-trajectory U-turn rejects), dmax_iter (the depth limit was hit), max_exp_arg_iter (largest |argument| of the exp()
+    calls of the progressive-sampling and biased-choice weights) and nonfinite_iter (some weight was inf or NaN).  Recording
+    changes nothing the sampler computes.
     """
     q_start = np.asarray(q_start, dtype=float)
     assert q_start.shape[0] == Nchain                                       # samplers.py:510
@@ -410,6 +414,17 @@ def gen_sample_NUTS(D, V, dVdq, q_start, draws, Nchain, Niter, thin_rate=1, warm
         res.u_tape = [[] for _ in range(Nchain)]
         res.n_leapfrog = np.zeros((Nchain, Niter), dtype=np.int64)
         res.depth = np.zeros((Nchain, Niter), dtype=np.int32)
+        res.n_instab_iter = np.zeros((Nchain, Niter), dtype=np.int32)
+        res.n_uturn_sub_iter = np.zeros((Nchain, Niter), dtype=np.int32)
+        res.dmax_iter = np.zeros((Nchain, Niter), dtype=bool)
+        res.max_exp_arg_iter = np.zeros((Nchain, Niter))
+        res.nonfinite_iter = np.zeros((Nchain, Niter), dtype=bool)
+
+    def note_weights(m, i, args, values):
+        """record only: the exp() arguments and the weights of one progressive-sampling or biased-choice step"""
+        res.max_exp_arg_iter[m, i - 1] = max(res.max_exp_arg_iter[m, i - 1], max(abs(v) for v in args))
+        if not all(np.isfinite(v) for v in values):
+            res.nonfinite_iter[m, i - 1] = True
 
     def E(q, p):
         return V(q) + kinetic(p, inv_cov_p)
@@ -450,6 +465,8 @@ def gen_sample_NUTS(D, V, dVdq, q_start, draws, Nchain, Niter, thin_rate=1, warm
             while (not left_terminate) or (not right_terminate):            # samplers.py:595 (Q6)
                 if d > d_max - 1:                                           # samplers.py:596-598 (Q7)
                     res.n_dmax += 1
+                    if record:
+                        res.dmax_iter[m, i - 1] = True
                     if on_dmax == "assert":
                         raise DMaxExceeded("Doubling number d exceeds d_max = %d" % d_max)
                     break
@@ -484,6 +501,8 @@ def gen_sample_NUTS(D, V, dVdq, q_start, draws, Nchain, Niter, thin_rate=1, warm
                             trajectory_reject = True
                             q_tmp = live_point_q_old
                             res.n_instability += 1
+                            if record:
+                                res.n_instab_iter[m, i - 1] += 1
                             break
                         if ((k + 1) % 2) == 1:                              # samplers.py:654-658
                             save_index = find_next(save_index_table)
@@ -506,6 +525,8 @@ def gen_sample_NUTS(D, V, dVdq, q_start, draws, Nchain, Niter, thin_rate=1, warm
                                 left_terminate_tmp = np.dot(-Dq_tmp, left_p_tmp) < 0
                                 if left_terminate_tmp and right_terminate_tmp:    # Q6: both
                                     trajectory_reject = True
+                                    if record:
+                                        res.n_uturn_sub_iter[m, i - 1] += 1
                                     q_tmp = live_point_q_old
                                     break
                                 if (l > 1) and release(k + 1, l):
@@ -520,6 +541,8 @@ def gen_sample_NUTS(D, V, dVdq, q_start, draws, Nchain, Niter, thin_rate=1, warm
                         u = draws.random()
                         if record:
                             res.u_tape[m].append(u)
+                            note_weights(m, i, (E_tmp - E_max_new_now, E_max_new_now - E_max_new_previous),
+                                         (numerator, pi_new, r))
                         if u < r:
                             live_point_q_new = q_tmp
                 if trajectory_reject:                                       # samplers.py:754-755
@@ -537,6 +560,8 @@ def gen_sample_NUTS(D, V, dVdq, q_start, draws, Nchain, Niter, thin_rate=1, warm
                 u = draws.random()                                          # samplers.py:773
                 if record:
                     res.u_tape[m].append(u)
+                    note_weights(m, i, (E_max_new_now - E_max_old_previous, E_max_new_now - E_max_old,
+                                        E_max_old_previous - E_max_old), (r, pi_old))
                 if u < A:
                     live_point_q_old = live_point_q_new
                 q_tmp = live_point_q_old
