@@ -270,6 +270,34 @@ int hmc_diag_variogram_all(int32_t dtype, const void* q, int64_t Nchain, int64_t
                            int32_t nlags, double* out_nlags_x_D, void* workspace, int64_t workspace_bytes, void* cuda_stream);
 
 /*
+ * Streamed diagnostics (csrc/diag_stream.cu): the partial sums of hmc_diag_moments and hmc_diag_variogram for the lags 1..T, folded
+ * in block by block from a ring q_ring [Nchain][R][D] (compute dtype; stored index j of chain c in row j % R, as
+ * hmc_random_args.store_ring = R writes it), so that R_q and n_eff_q of a run need only the last R stored samples per chain on the
+ * device.  The split is the one above: with n = (L_chain - 1) / 2, split chain 2m is stored indices [1, n] of chain m and 2m+1 is
+ * [n+1, 2n] (index 0 and, for an odd L_chain - 1, the last index are not used).
+ *
+ *   hmc_diag_stream_update : hands over stored indices [j0, j1) of every local chain; every index must be final (its thin window
+ *                            closed) and rows [j0 - T, j1) must still be in the ring, so R >= T + (j1 - j0).  Calls of one run cover
+ *                            [0, L_chain) in order; the call with j0 = 0 zeroes the accumulated sums.  Each index is added to its
+ *                            split chain's float64 shifted sum and sum of squares (state per chain and dimension); at index n or 2n the
+ *                            split chain's mean and ddof = 1 std are folded into the moment rows.  Every pair (i - t, i) with i in
+ *                            [j0, j1), 1 <= t <= T and both in one split chain is added to lag t: per chain over at most 64 new indices
+ *                            in the stream's precision (as the windowed kernel does over a whole split chain), then in float64.
+ *   hmc_diag_stream_finish : out4xD [4][D] = the rows hmc_diag_moments writes (sums of std_j, mean_j - c, (mean_j - c)^2, and c = the
+ *                            first used sample of local chain 0), out_lags [T][D] = the numerators hmc_diag_variogram writes for lags
+ *                            1..T.  Copies on the stream; the workspace is left as it was.
+ * `workspace`: device scratch of hmc_diag_stream_workspace_bytes(Nchain, D, T) = 8 D (4 + T + 3 Nchain) bytes, kept by the caller
+ * for the whole run (the library keeps nothing between calls).  The size is non-zero exactly for Nchain >= 1, 1 <= D <= 8192 and
+ * 1 <= T <= 2^20.  HMC_E_BADARG: R < T + (j1 - j0), T < 1 or T > n - 1, j0 / j1 outside 0 <= j0 <= j1 <= L_chain, D outside
+ * [1, 8192], a NULL ring, a missing or short workspace.
+ */
+int64_t hmc_diag_stream_workspace_bytes(int64_t Nchain, int32_t D, int32_t T);
+int hmc_diag_stream_update(int32_t dtype, const void* q_ring, int64_t Nchain, int32_t D, int32_t R, int64_t L_chain, int32_t T,
+                           int64_t j0, int64_t j1, void* workspace, int64_t workspace_bytes, void* cuda_stream);
+int hmc_diag_stream_finish(const void* workspace, int64_t workspace_bytes, int32_t D, int32_t T, double* out4xD, double* out_lags,
+                           void* cuda_stream);
+
+/*
  * Start points on the device: replaces utils.start_pts (utils.py:204-209, np.random.multivariate_normal(q0, cov0, size)).
  * out[m][:] = q0 + Lc z_m with z_m ~ N(0, I) from Philox keyed by (seed, chain_id0 + m), so the points do not depend on
  * how chains are sharded.  q0 [D], Lc [D][D] (row-major lower-triangular factor, Lc Lc^T = cov0) or NULL, sd [D]

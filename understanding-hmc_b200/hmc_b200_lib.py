@@ -21,7 +21,7 @@ EXPORTS = ["hmc_random_run", "hmc_nuts_run", "hmc_diag_moments", "hmc_diag_vario
            "hmc_ffma_peak", "hmc_version", "hmc_last_error_string", "hmc_start_pts", "hmc_summary_moments", "hmc_summary_hist",
            "hmc_summary_select", "hmc_random_workspace_bytes", "hmc_diag_variogram_all", "hmc_diag_variogram_all_workspace_bytes", "hmc_leap_frog",
            "hmc_nuts_workspace_bytes", "hmc_start_pts_workspace_bytes", "hmc_start_pts_bigd", "hmc_leap_frog_workspace_bytes",
-           "hmc_leap_frog_bigd"]
+           "hmc_leap_frog_bigd", "hmc_diag_stream_workspace_bytes", "hmc_diag_stream_update", "hmc_diag_stream_finish"]
 
 
 class Target(C.Structure):
@@ -89,6 +89,13 @@ def load():
     lib.hmc_diag_variogram_all.restype = C.c_int
     lib.hmc_diag_variogram_all_workspace_bytes.argtypes = [C.c_int64, C.c_int32]
     lib.hmc_diag_variogram_all_workspace_bytes.restype = C.c_int64
+    lib.hmc_diag_stream_workspace_bytes.argtypes = [C.c_int64, C.c_int32, C.c_int32]
+    lib.hmc_diag_stream_workspace_bytes.restype = C.c_int64
+    lib.hmc_diag_stream_update.argtypes = [C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int64,
+                                           C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.hmc_diag_stream_update.restype = C.c_int
+    lib.hmc_diag_stream_finish.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.hmc_diag_stream_finish.restype = C.c_int
     lib.hmc_leap_frog.argtypes = [C.c_int32, C.POINTER(Target), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                   C.c_void_p]
     lib.hmc_leap_frog.restype = C.c_int

@@ -14,7 +14,10 @@ Extra keyword-only constructor arguments (defaults keep the reference behaviour)
   tc_precision="bf16x3"|"fp16x2" (split of the tensor-core gradient product: three bf16 parts / six tensor passes -- the
   default of the D = 100 kernel and of NUTS on the large-D path -- or two fp16 parts / three passes -- the default of the
   large-D GEMM path of the random-trajectory sampler; at D = 100, rho = 0.95 fp16x2 is 10 % faster at 3x the trajectory error,
-  see DESIGN 4.0; a D = 100 run whose start points leave the fp16 range repeats itself with bf16x3).
+  see DESIGN 4.0; a D = 100 run whose start points leave the fp16 range repeats itself with bf16x3),
+  stream_stats=None|T ("Random" / "Fixed": keep only a ring of the last T + B stored samples per chain and fold each iteration
+  block's final samples into the partial sums of R_q and n_eff_q with lags up to T, csrc/diag_stream.cu; B = iter_block //
+  thin_rate stored samples per block, 64 by default.  q_chain, E_chain, dE_chain and sample_summary are not available then).
 """
 import os
 
@@ -57,6 +60,27 @@ def random_runs_bigd(D, dtype, kernel, cov_p_identity):
     if not cov_p_identity:
         return D > 1024
     return kernel == "bigd" or D % 256 == 0 or D > 1024
+
+
+def stream_blocks(Niter, warm_up_num, thin_rate, per_block):
+    """Iteration blocks of a stream_stats run: [(iter_begin, iter_end, j0, j1)], where stored indices [j0, j1) are final once iteration
+    iter_end has run and are handed to hmc_diag_stream_update after that block.  Iteration it >= warm_up_num writes stored index
+    (it - warm_up_num) // thin_rate and the last write of a thin window wins (samplers.py:465-471), so index j is final after iteration
+    min(warm_up_num + (j + 1) thin_rate - 1, Niter); a block ends exactly there, which also means it writes no index outside its own
+    [j0, j1) (index 0 is the start point, written by the first block).  At most per_block indices per block, except that the first block
+    takes more when it would otherwise run no iteration.  The ring then needs T + max(j1 - j0) rows."""
+    Lc = 1 + (Niter - warm_up_num) // thin_rate
+    per_block = max(1, int(per_block))
+    out, it0, j0 = [], 0, 0
+    while j0 < Lc:
+        j1 = min(j0 + per_block, Lc)
+        it1 = Niter if j1 == Lc else warm_up_num + j1 * thin_rate - 1
+        while it1 <= it0 and j1 < Lc and not out:          # a first block of no iteration: give it the next indices too
+            j1 = min(j1 + per_block, Lc)
+            it1 = Niter if j1 == Lc else warm_up_num + j1 * thin_rate - 1
+        out.append((it0, it1, j0, j1))
+        it0, j0 = it1, j1
+    return out
 
 
 def equicorrelated_cov(D, rho):
@@ -118,8 +142,14 @@ class sampler(object):
         self.dt_total = 0
         self.N_total_steps = 0
 
+    def _no_stream(self, what):
+        if getattr(self, "stream_stats", None) is not None:
+            raise RuntimeError("%s is not available with stream_stats=%d: the run keeps only a ring of its last stored samples "
+                               "(use stream_stats=None for the full stream)" % (what, self.stream_stats))
+
     @property
     def q_chain(self):
+        self._no_stream("q_chain")
         if self._q_host is None:
             if self._q_dev is None:
                 self._q_host = np.zeros((self.Nchain, self.L_chain, self.D), dtype=float)   # samplers.py:33
@@ -135,10 +165,25 @@ class sampler(object):
     @property
     def q_chain_device(self):
         """(Nchain, L_chain, D) CUDA tensor in the compute dtype (no host copy)."""
+        self._no_stream("q_chain_device")
         return self._q_dev
 
     def compute_convergence_stats(self):
-        """R_q, n_eff_q over stored samples 1.. (samplers.py:53-64), on the GPU."""
+        """R_q, n_eff_q over stored samples 1.. (samplers.py:53-64), on the GPU.  With stream_stats=T they come from the partial sums
+        streamed during gen_sample (lags up to T); n_eff_truncated [D] flags the dimensions whose truncation rule had not stopped by
+        lag T (their n_eff_q sums the autocorrelations up to there), and one warning is printed when there are any."""
+        if getattr(self, "stream_stats", None) is not None:
+            st = self._stream
+            assert st is not None, "compute_convergence_stats needs a finished gen_sample"
+            group = None if getattr(self, "distributed", False) else False
+            self.R_q, self.n_eff_q, self.n_eff_truncated = _utils.stream_stats_from_workspace(
+                st["ws_ptr"], st["ws_bytes"], self.D, self.stream_stats, self.L_chain, self.Nchain, group=group, device=st["device"])
+            nt = int(np.sum(self.n_eff_truncated))
+            if nt:
+                print("compute_convergence_stats: for %d of %d dimensions the n_eff truncation rule had not stopped by lag %d "
+                      "(stream_stats); their n_eff_q uses the lags up to there -- a larger stream_stats reaches further"
+                      % (nt, self.D, self.stream_stats))
+            return
         src = self._q_dev if self._q_dev is not None else self.q_chain
         group = None if getattr(self, "distributed", False) else False
         self.R_q, self.n_eff_q = _utils.convergence_stats(src[:, 1:, :], warm_up_num=0, thin_rate=1, group=group)
@@ -149,6 +194,7 @@ class sampler(object):
         reductions over the device-resident outputs (csrc/summary.cu): per-dimension mean / variance over stored samples
         1.., 2.5 / 97.5 percentiles, plot ranges and histograms of q1, q2 (all stored samples) and of the centred energies
         E and the energy differences dE (stored samples 1..).  Sharded runs all-reduce the counts."""
+        self._no_stream("sample_summary")
         q = self._q_dev
         assert q is not None, "sample_summary needs a finished gen_sample"
         group = None if getattr(self, "distributed", False) else False
@@ -234,7 +280,7 @@ class HMC_sampler(sampler):
                  cov_p=None, sampler_type="Fixed", L=None, global_dt=True, dt=None,
                  L_low=None, L_high=None, log2L=None, d_max=10, *,
                  dtype="float32", seed=0, kernel="auto", draws=None, on_dmax="assert", chain_id0=0,
-                 distributed=False, iter_block=None, target=None, tc_precision=None):
+                 distributed=False, iter_block=None, target=None, tc_precision=None, stream_stats=None):
         sampler.__init__(self, D=D, target_lnL=None, Nchain=Nchain, Niter=Niter, thin_rate=thin_rate,
                          warm_up_num=warm_up_num)
         self.V = V
@@ -288,10 +334,19 @@ class HMC_sampler(sampler):
         self.sum_L = 0
         self.n_leapfrog = None
         self.status = None
+        self.stream_stats = None if stream_stats is None else int(stream_stats)
+        self._stream = None
+        self.n_eff_truncated = None
+        if self.stream_stats is not None:
+            assert sampler_type in ("Random", "Fixed"), \
+                "stream_stats applies to the Random and Fixed samplers (NUTS keeps the full stream: hmc_nuts_args has no store_ring)"
+            n = (self.L_chain - 1) // 2
+            assert 1 <= self.stream_stats <= n - 1, "stream_stats = T needs 1 <= T <= n - 1 = %d (n = (L_chain - 1) // 2)" % (n - 1)
 
     # ---- reference-layout host views of the energy streams (samplers.py:359-360) ----
     @property
     def E_chain(self):
+        self._no_stream("E_chain")
         if self._E_host is None:
             self._E_host = np.zeros((self.Nchain, self.L_chain, 1)) if self._E_dev is None else \
                 self._E_dev.cpu().numpy()[:, :, None]
@@ -306,6 +361,7 @@ class HMC_sampler(sampler):
 
     @property
     def dE_chain(self):
+        self._no_stream("dE_chain")
         if self._dE_host is None:
             self._dE_host = np.zeros((self.Nchain, self.L_chain, 1)) if self._dE_dev is None else \
                 self._dE_dev.cpu().numpy()[:, :, None]
@@ -412,9 +468,14 @@ class HMC_sampler(sampler):
         f64 = torch.float64
         owns0 = self.chain_id0 == 0
         save_chain = N_save_chain0 > 0
-        self._q_dev = torch.empty((Nc, Lc, D), dtype=tdt, device=dev)     # every stored sample / energy is written by the kernel
-        self._E_dev = torch.empty((Nc, Lc), dtype=f64, device=dev)
-        self._dE_dev = torch.empty((Nc, Lc), dtype=f64, device=dev)
+        rows, blocks = Lc, None
+        if self.stream_stats is not None:          # a ring of T + (indices per block) rows: stored index j in row j % R
+            blocks = stream_blocks(self.Niter, self.warm_up_num, self.thin_rate,
+                                   int(self.iter_block) // self.thin_rate if self.iter_block else 64)
+            rows = self.stream_stats + max(j1 - j0 for (_, _, j0, j1) in blocks)
+        self._q_dev = torch.empty((Nc, rows, D), dtype=tdt, device=dev)   # every stored sample / energy is written by the kernel
+        self._E_dev = torch.empty((Nc, rows), dtype=f64, device=dev)
+        self._dE_dev = torch.empty((Nc, rows), dtype=f64, device=dev)
         self._q_host = self._E_host = self._dE_host = None
         keep["qs"] = self._to_device(torch, q_start, dev, tdt)
         keep["state_q"] = torch.empty((Nc, D), dtype=tdt, device=dev)
@@ -447,6 +508,12 @@ class HMC_sampler(sampler):
             assert keep["L_tape"].shape == (Nc, self.Niter) and keep["u_tape"].shape == (Nc, self.Niter)
             a.p_tape, a.L_tape, a.u_tape = (keep[k].data_ptr() for k in ("p_tape", "L_tape", "u_tape"))
         a.q_chain, a.E_chain, a.dE_chain = self._q_dev.data_ptr(), self._E_dev.data_ptr(), self._dE_dev.data_ptr()
+        if blocks is not None:
+            a.store_ring = rows
+            nbytes = int(_L.load().hmc_diag_stream_workspace_bytes(Nc, D, self.stream_stats))
+            keep["stream_ws"] = torch.empty((max(1, nbytes // 8),), dtype=f64, device=dev)
+            self._stream = dict(blocks=blocks, R=rows, ws=keep["stream_ws"], ws_ptr=keep["stream_ws"].data_ptr(), ws_bytes=nbytes,
+                                device=dev)
         a.state_q, a.state_g, a.state_eprev = keep["state_q"].data_ptr(), keep["state_g"].data_ptr(), \
             keep["state_e"].data_ptr()
         a.counters = counters.data_ptr()
@@ -475,9 +542,18 @@ class HMC_sampler(sampler):
             say("Running %d chains x %d iterations on %s (%s, kernel=%s)" %
                 (Nc, self.Niter, torch.cuda.get_device_name(dev), self.dtype, self.kernel))
         ev0.record()
-        for (b, e) in self._blocks():
-            a.iter_begin, a.iter_end = b, e
-            _L.check(lib.hmc_random_run(a, stream))
+        if self._stream is None:
+            for (b, e) in self._blocks():
+                a.iter_begin, a.iter_end = b, e
+                _L.check(lib.hmc_random_run(a, stream))
+        else:                                     # each block's final samples go into the streamed partial sums on the same stream
+            st = self._stream
+            dt_id = a.dtype
+            for (b, e, j0, j1) in st["blocks"]:
+                a.iter_begin, a.iter_end = b, e
+                _L.check(lib.hmc_random_run(a, stream))
+                _L.check(lib.hmc_diag_stream_update(dt_id, _L.C.c_void_p(a.q_chain), Nc, D, st["R"], self.L_chain, self.stream_stats,
+                                                    j0, j1, _L.C.c_void_p(st["ws_ptr"]), st["ws_bytes"], stream))
         ev1.record()
         ev1.synchronize()
         self.kernel_ms = ev0.elapsed_time(ev1)

@@ -109,7 +109,8 @@ ROW_SHIFT, ROW_COUNT, ROW_LAGS = 3, 4, 5        # layout of the packed statistic
 FFT_MIN_N = 192        # split chains at least this long take the all-lags FFT pass straight away (see _stats_from_partials)
 
 
-def _stats_from_partials(moments_fn, variogram_fn, n, D, m_local, group=None, lag_chunk=32, device=None, all_lags_fn=None):
+def _stats_from_partials(moments_fn, variogram_fn, n, D, m_local, group=None, lag_chunk=32, device=None, all_lags_fn=None, max_lag=None,
+                         info=None):
     """Rhat / n_eff from per-rank partial sums (utils.py:107-157).
 
     ``moments_fn(buf)`` fills the float64 buffer ``buf`` [5 + lag_chunk][D]: rows 0..2 = sum_j std_j, sum_j (mean_j - c),
@@ -127,7 +128,11 @@ def _stats_from_partials(moments_fn, variogram_fn, n, D, m_local, group=None, la
     ``all_lags_fn(buf)`` (optional) fills ``buf`` [n - 1][D] with the numerators of EVERY lag in one pass over the samples
     (csrc/diag_fft.cu: one FFT per chain and dimension, a fixed cost per chain).  Long split chains (n >= FFT_MIN_N) use it
     straight away; shorter ones try one windowed chunk first (a well-mixed chain ends within it) and switch when the
-    truncation rule has not fired.  Sharded runs all-reduce that one buffer."""
+    truncation rule has not fired.  Sharded runs all-reduce that one buffer.
+
+    ``max_lag`` (default n - 1: every lag) caps the lags the truncation rule may read, for sources that only have lags 1..max_lag
+    (the streamed partials of hmc_diag_stream_*).  A dimension whose rule has not stopped by then is closed with the lags it has and,
+    when ``info`` is a dict, flagged in ``info["n_eff_truncated"]`` [D] (always all False when max_lag >= n - 1)."""
     import torch
     import torch.distributed as dist
     distributed = dist.is_available() and dist.is_initialized() and (group is not False)
@@ -155,7 +160,7 @@ def _stats_from_partials(moments_fn, variogram_fn, n, D, m_local, group=None, la
 
     state = _NeffState(D)
     lag0 = 1
-    max_lag = n - 1
+    max_lag = n - 1 if max_lag is None else min(int(max_lag), n - 1)
     vbuf = None
     while lag0 <= max_lag:
         nl = min(lag_chunk, max_lag - lag0 + 1)
@@ -179,6 +184,8 @@ def _stats_from_partials(moments_fn, variogram_fn, n, D, m_local, group=None, la
         if _finish_n_eff(var, V_rows, m, n, state):
             break
         lag0 += nl
+    if info is not None:
+        info["n_eff_truncated"] = ~state.done if max_lag < n - 1 else np.zeros(D, dtype=bool)
     state.close(~state.done, np.full(D, state.t))        # chains too short to ever start (n < 3): use what exists
     n_eff = m * n / (1 + 2 * state.sum_rho)                                             # utils.py:157
     return R, n_eff
@@ -239,6 +246,33 @@ def _device_stats(x, n, group=None, lag_chunk=32):
 
     return _stats_from_partials(moments_fn, variogram_fn, n, D, 2 * Nchain, group=group, lag_chunk=lag_chunk, device=x.device,
                                 all_lags_fn=all_lags_fn)
+
+
+def stream_stats_from_workspace(workspace_ptr, workspace_bytes, D, T, L_chain, Nchain, group=None, device=None):
+    """(R, n_eff, n_eff_truncated) from the partial sums hmc_diag_stream_update accumulated in a workspace over stored indices
+    [0, L_chain) of Nchain local chains (csrc/diag_stream.cu).  The host finishing is _stats_from_partials' with the lags capped at T;
+    ranks are combined as for the full stream (one all-gather, one all-reduce of the T lag rows)."""
+    import torch
+    lib = _L.load()
+    n = (L_chain - 1) // 2
+    lags = _scratch("stream_lags", (T, D), torch.float64, device)
+
+    def moments_fn(buf):
+        _L.check(lib.hmc_diag_stream_finish(workspace_ptr, workspace_bytes, D, T, _L.ptr(buf), _L.ptr(lags), _L.current_stream_ptr()))
+        nl = min(T, buf.shape[0] - ROW_LAGS)
+        buf[ROW_LAGS:ROW_LAGS + nl] = lags[:nl]
+        return nl
+
+    def variogram_fn(lag0, nl, buf):
+        raise AssertionError("the streamed partials hold every lag up to T")
+
+    def all_lags_fn(buf):
+        buf.copy_(lags)
+
+    info = {}
+    R, n_eff = _stats_from_partials(moments_fn, variogram_fn, n, D, 2 * Nchain, group=group, device=device, all_lags_fn=all_lags_fn,
+                                    max_lag=T, info=info)
+    return R, n_eff, info["n_eff_truncated"]
 
 
 def convergence_stats(q_chain, thin_rate=5, warm_up_num=0, group=None):
