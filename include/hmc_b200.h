@@ -44,7 +44,8 @@ enum {
     HMC_KERNEL_AUTO = 0,    /* tensor-core kernel if it covers the run, else the large-D GEMM path (when a workspace is given and
                                D % 256 == 0 or D > 1024; with a dense momentum metric for D > 1024 only), else the FFMA2 kernel, else
                                the generic one.  NUTS: the tensor-core kernel,
-                               else the large-D path when a workspace is given, it covers the run and D > 256, else the generic one */
+                               else the large-D path when a workspace is given, it covers the run and D > 256, else the generic one
+                               (with hmc_nuts_args.store_ring > 0: the large-D path from D = 128, nothing else) */
     HMC_KERNEL_GENERIC = 1, /* one warp per chain, any D <= 1024 (NUTS: D <= 256), float or double (parity workhorse) */
     HMC_KERNEL_FAST = 2,    /* FP32 FFMA2 register-tile kernel, 20 < D <= 128, identity momentum metric */
     HMC_KERNEL_TC = 3,      /* tcgen05 tensor-core kernel (bf16x3 / fp16x2 split, fp32 accumulate in TMEM), D <= 100 and a multiple of 4
@@ -185,6 +186,10 @@ int64_t hmc_random_workspace_bytes(const hmc_random_args* args);
  * uniform per surviving inner step (samplers.py:748) and one per completed doubling (samplers.py:773).
  * Kernels: the generic one (D <= 256, float or double, any metric), the tensor-core one (D = 100, float32, identity metric,
  * d_max <= 12), the large-D path (any 128 <= D <= 8192, float32, identity metric; needs `workspace`).
+ * store_ring: as hmc_random_args.store_ring (0: L_chain rows per chain; R > 0: q_chain / E_chain / dE_chain hold R rows per
+ * chain and stored index j goes to row j % R), served by the large-D path only.  With store_ring > 0, AUTO takes the large-D path
+ * whenever `workspace` is given and the path covers the run (any 128 <= D <= 8192, not only D > 256); an explicit generic or tc
+ * kernel, or an AUTO run the path does not cover, is HMC_E_UNSUPPORTED.  store_ring < 0 is HMC_E_BADARG.
  */
 typedef struct hmc_nuts_args {
     int32_t dtype;
@@ -221,7 +226,8 @@ typedef struct hmc_nuts_args {
     int32_t* status;        /* [Nchain] bit0: d_max exceeded; may be NULL */
     int64_t* n_leapfrog;    /* [Nchain] leapfrog steps per chain (accumulated); may be NULL */
     int32_t flags;          /* HMC_FLAG_TC_FP16X2 selects the two-part fp16 split on the large-D path (default: bf16x3) */
-    int32_t reserved0;
+    int32_t store_ring;     /* 0: the reference layout (L_chain rows per chain); R > 0: a ring of the last R stored samples per chain
+                               (large-D path only, see above) */
     void* workspace;        /* scratch of hmc_nuts_workspace_bytes(args) bytes for HMC_KERNEL_BIGD (1024-byte aligned); NULL otherwise */
     int64_t workspace_bytes;
 } hmc_nuts_args;

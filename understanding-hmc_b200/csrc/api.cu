@@ -135,8 +135,21 @@ extern "C" int hmc_nuts_run(const hmc_nuts_args* args, void* cuda_stream) {
                 "p_tape, dir_tape and u_tape must be given together");
     HMC_REQUIRE((a.target.Mit == nullptr) == (a.target.Pt == nullptr) && (a.target.Pt == nullptr) == (a.target.Lct == nullptr),
                 "dense momentum metric: target.Pt, Mit and Lct must be given together");
+    HMC_REQUIRE(a.store_ring >= 0, "store_ring must be >= 0 (got %d)", a.store_ring);
     const char* why = "";
     int kernel = a.kernel;
+    // a ring of stored samples is written by the large-D path only: AUTO takes it wherever it covers the run, from D = 128
+    if (a.store_ring > 0 && (kernel == HMC_KERNEL_AUTO || kernel == HMC_KERNEL_GENERIC || kernel == HMC_KERNEL_TC)) {
+        if (kernel == HMC_KERNEL_AUTO && a.workspace && hmc_nuts_bigd_supported(a, &why)) {
+            kernel = HMC_KERNEL_BIGD;
+        } else {
+            hmc_set_error("NUTS with store_ring > 0 runs on the large-D path only (float32, identity momentum metric, 128 <= D <= 8192, "
+                          "hmc_nuts_args.workspace given): %s",
+                          kernel != HMC_KERNEL_AUTO ? "the generic and tensor-core kernels keep the full stream"
+                          : !a.workspace ? "no workspace given" : why);
+            return HMC_E_UNSUPPORTED;
+        }
+    }
     // tensor-core kernel where it applies, else the large-D GEMM path above the generic kernel's D <= 256, else the generic kernel
     if (kernel == HMC_KERNEL_AUTO)
         kernel = hmc_nuts_tc_supported(a, &why) ? HMC_KERNEL_TC

@@ -28,7 +28,9 @@
 // the layout of nuts_generic.cu, cursors of the injected streams in row R + 6).  Everything the GEMM touches is in the workspace,
 // Dp = D rounded up to 32 wide and zero in the padded dimensions (no force, no momentum, dt = 0 there), as in random_bigd.cu.
 // The position is kept shifted, x = q - mu; at every iteration end it is re-derived from the stored sample (x = (x + mu) - mu in
-// float32), so a run split into iteration blocks (resumed from state_q) is bit-identical to a single launch.
+// float32), so a run split into iteration blocks (resumed from state_q) is bit-identical to a single launch.  Nothing reads q_chain
+// back, so with store_ring > 0 the three outputs are a ring of the last store_ring stored samples per chain (stored index j in
+// row j % store_ring, the 32-bit wrap of hmc_store_index) and nothing else changes.
 //
 // Unfused: G is written and read back (8 B per element and pass) and the step kernel reads / writes x, p and stack rows on top
 // of the GEMM's operand traffic.
@@ -92,10 +94,10 @@ __global__ void __launch_bounds__(128) nuts_bigd_init(hmc_nuts_args a, NbWs w) {
     }
     const bool fresh = a.iter_begin == 0;
     const float* src = (fresh ? (const float*)a.q_start : (const float*)a.state_q) + (size_t)m * D;
-    const long Lc = 1 + (a.Niter - a.warm_up_num) / a.thin_rate;
+    const long Lrow = a.store_ring > 0 ? a.store_ring : 1 + (a.Niter - a.warm_up_num) / a.thin_rate;   // rows per chain of q_chain
     for (int j = lane; j < Dp; j += 32) {
         const float v = j < D ? src[j] : 0.f;
-        if (fresh && j < D) ((float*)a.q_chain)[(size_t)m * Lc * D + j] = v;           // samplers.py:548
+        if (fresh && j < D) ((float*)a.q_chain)[(size_t)m * Lrow * D + j] = v;         // samplers.py:548 (stored index 0)
         xr[j] = v - w.mu[j];
     }
     bigd_write_parts<NPART>(w.xp, w.Ncp, Dp, m, lane, xr);
@@ -119,7 +121,9 @@ __global__ void __launch_bounds__(32 * NB_WARPS) nuts_bigd_step(hmc_nuts_args a,
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int D = a.target.D, Dp = w.Dp, Dpad = a.target.D_pad;
     const int R = 2 * (a.d_max + 1);
-    const long Lc = 1 + (a.Niter - a.warm_up_num) / a.thin_rate;
+    // rows per chain of q_chain / E_chain / dE_chain: L_chain, or a ring of the last store_ring stored samples (index j in row j % store_ring)
+    const bool ring = a.store_ring > 0;
+    const long Lrow = ring ? a.store_ring : 1 + (a.Niter - a.warm_up_num) / a.thin_rate;
     const double vconst = a.target.v_const;
     const bool ext4 = (D & 3) == 0;            // the caller's rows (stored samples, state_q) are D wide: 16-byte aligned only then
     int alive = 0;
@@ -197,7 +201,7 @@ __global__ void __launch_bounds__(32 * NB_WARPS) nuts_bigd_step(hmc_nuts_args a,
         bool finish = false, new_doubling = false, traj_test = false, start_iter = false;
         if (c.ph == NB_CHAIN_START) {
             const double E0 = V + Kc;                                   // samplers.py:551-555
-            if (lane == 0) { a.E_chain[(size_t)m * Lc] = E0; a.dE_chain[(size_t)m * Lc] = 0.0; }
+            if (lane == 0) { a.E_chain[(size_t)m * Lrow] = E0; a.dE_chain[(size_t)m * Lrow] = 0.0; }
             c.E_prev = E0;
             const float s = nb_draw(a, Dp, m, c.it, lane, pr);          // samplers.py:565: the momentum of the first iteration
             c.E_initial = V + 0.5 * (double)s;                          // samplers.py:569 (same position, same gradient)
@@ -285,9 +289,9 @@ __global__ void __launch_bounds__(32 * NB_WARPS) nuts_bigd_step(hmc_nuts_args a,
         if (start_iter) {
             // samplers.py:571-594: stored energies, live point, both boundary points, running maxima
             if (c.it >= a.warm_up_num && lane == 0) {
-                const long idx = (c.it - a.warm_up_num) / a.thin_rate;
-                a.E_chain[(size_t)m * Lc + idx] = c.E_initial;
-                a.dE_chain[(size_t)m * Lc + idx] = c.E_initial - c.E_prev;
+                const long idx = hmc_store_index(c.it, a.warm_up_num, a.thin_rate, Lrow, ring);
+                a.E_chain[(size_t)m * Lrow + idx] = c.E_initial;
+                a.dE_chain[(size_t)m * Lrow + idx] = c.E_initial - c.E_prev;
             }
             store_row(R + 1, xr, 1.f);
             store_row(R + 2, xr, 1.f);
@@ -338,7 +342,8 @@ __global__ void __launch_bounds__(32 * NB_WARPS) nuts_bigd_step(hmc_nuts_args a,
             c.E_prev = c.E_initial;
             const bool keep = c.it >= a.warm_up_num;
             const bool last = c.it >= a.iter_end;
-            float* dst = keep ? (float*)a.q_chain + ((size_t)m * Lc + (c.it - a.warm_up_num) / a.thin_rate) * D : nullptr;
+            float* dst = keep ? (float*)a.q_chain + ((size_t)m * Lrow + hmc_store_index(c.it, a.warm_up_num, a.thin_rate, Lrow, ring)) * D
+                              : nullptr;
             float* sq = last ? (float*)a.state_q + (size_t)m * D : nullptr;
             const float* lo = row(R + 1);
             for (int j = 4 * lane; j < Dpad; j += 128) {

@@ -50,7 +50,7 @@ class NutsArgs(C.Structure):
                 ("u_tape", C.c_void_p), ("tape_dir_stride", C.c_int32), ("tape_u_stride", C.c_int32),
                 ("q_chain", C.c_void_p), ("E_chain", C.c_void_p), ("dE_chain", C.c_void_p), ("state_q", C.c_void_p),
                 ("state_eprev", C.c_void_p), ("scratch", C.c_void_p), ("counters", C.c_void_p), ("status", C.c_void_p),
-                ("n_leapfrog", C.c_void_p), ("flags", C.c_int32), ("reserved0", C.c_int32), ("workspace", C.c_void_p),
+                ("n_leapfrog", C.c_void_p), ("flags", C.c_int32), ("store_ring", C.c_int32), ("workspace", C.c_void_p),
                 ("workspace_bytes", C.c_int64)]
 
 

@@ -15,9 +15,10 @@ Extra keyword-only constructor arguments (defaults keep the reference behaviour)
   default of the D = 100 kernel and of NUTS on the large-D path -- or two fp16 parts / three passes -- the default of the
   large-D GEMM path of the random-trajectory sampler; at D = 100, rho = 0.95 fp16x2 is 10 % faster at 3x the trajectory error,
   see DESIGN 4.0; a D = 100 run whose start points leave the fp16 range repeats itself with bf16x3),
-  stream_stats=None|T ("Random" / "Fixed": keep only a ring of the last T + B stored samples per chain and fold each iteration
-  block's final samples into the partial sums of R_q and n_eff_q with lags up to T, csrc/diag_stream.cu; B = iter_block //
-  thin_rate stored samples per block, 64 by default.  q_chain, E_chain, dE_chain and sample_summary are not available then).
+  stream_stats=None|T ("Random" / "Fixed", and "NUTS" on the large-D path: keep only a ring of the last T + B stored samples per
+  chain and fold each iteration block's final samples into the partial sums of R_q and n_eff_q with lags up to T,
+  csrc/diag_stream.cu; B = iter_block // thin_rate stored samples per block, 64 by default.  q_chain, E_chain, dE_chain and
+  sample_summary are not available then).
 """
 import os
 
@@ -60,6 +61,15 @@ def random_runs_bigd(D, dtype, kernel, cov_p_identity):
     if not cov_p_identity:
         return D > 1024
     return kernel == "bigd" or D % 256 == 0 or D > 1024
+
+
+def nuts_runs_bigd(D, dtype, kernel, cov_p_identity, stream=False):
+    """Whether the NUTS sampler runs on the large-D GEMM path (csrc/api.cu's AUTO rule and the path's coverage): float32,
+    ``cov_p = I`` and 128 <= D <= 8192, under kernel="bigd", or under "auto" for D > 256 -- from D = 128 when the run keeps a ring
+    of its stored samples (``stream``: hmc_nuts_args.store_ring > 0 is served by this path only)."""
+    if dtype != "float32" or not cov_p_identity or kernel not in ("auto", "bigd") or not 128 <= D <= 8192:
+        return False
+    return kernel == "bigd" or D > 256 or bool(stream)
 
 
 def stream_blocks(Niter, warm_up_num, thin_rate, per_block):
@@ -272,7 +282,8 @@ class HMC_sampler(sampler):
     ``kernel`` of the NUTS sampler (reported as ``nuts_kernel``):
       "tc"       tensor-core kernel, D = 100, float32, ``cov_p = I``, d_max <= 12; auto there
       "bigd"     large-D GEMM path, any 128 <= D <= 8192, float32, ``cov_p = I`` (bf16x3 split unless tc_precision="fp16x2");
-                 auto for D > 256
+                 auto for D > 256, and from D = 128 with stream_stats (the only NUTS kernel that keeps a ring of stored samples;
+                 ``nuts_runs_bigd`` is the rule)
       "generic"  warp-per-chain kernel, D <= 256, float64 and dense ``cov_p`` too; auto for the rest
     """
 
@@ -338,8 +349,13 @@ class HMC_sampler(sampler):
         self._stream = None
         self.n_eff_truncated = None
         if self.stream_stats is not None:
-            assert sampler_type in ("Random", "Fixed"), \
-                "stream_stats applies to the Random and Fixed samplers (NUTS keeps the full stream: hmc_nuts_args has no store_ring)"
+            if sampler_type == "NUTS":
+                assert nuts_runs_bigd(D, dtype, kernel, self._cov_p_identity, stream=True), \
+                    "stream_stats with NUTS needs the large-D path (float32, cov_p = I, 128 <= D <= 8192, kernel 'auto' or 'bigd'): " \
+                    "the generic and tensor-core NUTS kernels keep the full stream"
+            else:
+                assert sampler_type in ("Random", "Fixed"), \
+                    "stream_stats applies to the Random, Fixed and NUTS samplers (Static runs no iterations)"
             n = (self.L_chain - 1) // 2
             assert 1 <= self.stream_stats <= n - 1, "stream_stats = T needs 1 <= T <= n - 1 = %d (n = (L_chain - 1) // 2)" % (n - 1)
 
@@ -450,6 +466,36 @@ class HMC_sampler(sampler):
             return 0
         return _L.FLAG_TC_FP16X2
 
+    def _stream_setup(self, torch, dev, keep):
+        """Rows per chain of the stored-sample arrays: L_chain, or with stream_stats=T a ring of T + (the largest block's stored
+        indices) rows (stored index j in row j % R).  In stream mode also plans the iteration blocks (stream_blocks), allocates the
+        workspace of the streamed partial sums and records both in self._stream."""
+        if self.stream_stats is None:
+            return self.L_chain
+        blocks = stream_blocks(self.Niter, self.warm_up_num, self.thin_rate,
+                               int(self.iter_block) // self.thin_rate if self.iter_block else 64)
+        rows = self.stream_stats + max(j1 - j0 for (_, _, j0, j1) in blocks)
+        nbytes = int(_L.load().hmc_diag_stream_workspace_bytes(self.Nchain, self.D, self.stream_stats))
+        keep["stream_ws"] = torch.empty((max(1, nbytes // 8),), dtype=torch.float64, device=dev)
+        self._stream = dict(blocks=blocks, R=rows, ws=keep["stream_ws"], ws_ptr=keep["stream_ws"].data_ptr(), ws_bytes=nbytes, device=dev)
+        return rows
+
+    def _run_blocks(self, run, a, stream):
+        """Launch the iteration blocks with run(a, stream) (hmc_random_run or hmc_nuts_run).  In stream mode each block's final
+        stored samples are folded into the streamed partial sums after it, on the same stream."""
+        if self._stream is None:
+            for (b, e) in self._blocks():
+                a.iter_begin, a.iter_end = b, e
+                _L.check(run(a, stream))
+            return
+        st = self._stream
+        lib = _L.load()
+        for (b, e, j0, j1) in st["blocks"]:
+            a.iter_begin, a.iter_end = b, e
+            _L.check(run(a, stream))
+            _L.check(lib.hmc_diag_stream_update(a.dtype, _L.C.c_void_p(a.q_chain), self.Nchain, self.D, st["R"], self.L_chain,
+                                                self.stream_stats, j0, j1, _L.C.c_void_p(st["ws_ptr"]), st["ws_bytes"], stream))
+
     @staticmethod
     def _set_workspace(torch, dev, a, nbytes):
         """Point the launch arguments a at a new 1024-byte aligned device workspace of nbytes; returns the tensor that owns it."""
@@ -464,15 +510,11 @@ class HMC_sampler(sampler):
         assert q_start.shape[0] == self.Nchain                                       # samplers.py:396
         dev = torch.device("cuda", torch.cuda.current_device())
         tgt, keep, tdt = self._build_target(torch, dev)
-        Nc, D, Lc = self.Nchain, self.D, self.L_chain
+        Nc, D = self.Nchain, self.D
         f64 = torch.float64
         owns0 = self.chain_id0 == 0
         save_chain = N_save_chain0 > 0
-        rows, blocks = Lc, None
-        if self.stream_stats is not None:          # a ring of T + (indices per block) rows: stored index j in row j % R
-            blocks = stream_blocks(self.Niter, self.warm_up_num, self.thin_rate,
-                                   int(self.iter_block) // self.thin_rate if self.iter_block else 64)
-            rows = self.stream_stats + max(j1 - j0 for (_, _, j0, j1) in blocks)
+        rows = self._stream_setup(torch, dev, keep)
         self._q_dev = torch.empty((Nc, rows, D), dtype=tdt, device=dev)   # every stored sample / energy is written by the kernel
         self._E_dev = torch.empty((Nc, rows), dtype=f64, device=dev)
         self._dE_dev = torch.empty((Nc, rows), dtype=f64, device=dev)
@@ -508,12 +550,8 @@ class HMC_sampler(sampler):
             assert keep["L_tape"].shape == (Nc, self.Niter) and keep["u_tape"].shape == (Nc, self.Niter)
             a.p_tape, a.L_tape, a.u_tape = (keep[k].data_ptr() for k in ("p_tape", "L_tape", "u_tape"))
         a.q_chain, a.E_chain, a.dE_chain = self._q_dev.data_ptr(), self._E_dev.data_ptr(), self._dE_dev.data_ptr()
-        if blocks is not None:
+        if self._stream is not None:
             a.store_ring = rows
-            nbytes = int(_L.load().hmc_diag_stream_workspace_bytes(Nc, D, self.stream_stats))
-            keep["stream_ws"] = torch.empty((max(1, nbytes // 8),), dtype=f64, device=dev)
-            self._stream = dict(blocks=blocks, R=rows, ws=keep["stream_ws"], ws_ptr=keep["stream_ws"].data_ptr(), ws_bytes=nbytes,
-                                device=dev)
         a.state_q, a.state_g, a.state_eprev = keep["state_q"].data_ptr(), keep["state_g"].data_ptr(), \
             keep["state_e"].data_ptr()
         a.counters = counters.data_ptr()
@@ -542,18 +580,7 @@ class HMC_sampler(sampler):
             say("Running %d chains x %d iterations on %s (%s, kernel=%s)" %
                 (Nc, self.Niter, torch.cuda.get_device_name(dev), self.dtype, self.kernel))
         ev0.record()
-        if self._stream is None:
-            for (b, e) in self._blocks():
-                a.iter_begin, a.iter_end = b, e
-                _L.check(lib.hmc_random_run(a, stream))
-        else:                                     # each block's final samples go into the streamed partial sums on the same stream
-            st = self._stream
-            dt_id = a.dtype
-            for (b, e, j0, j1) in st["blocks"]:
-                a.iter_begin, a.iter_end = b, e
-                _L.check(lib.hmc_random_run(a, stream))
-                _L.check(lib.hmc_diag_stream_update(dt_id, _L.C.c_void_p(a.q_chain), Nc, D, st["R"], self.L_chain, self.stream_stats,
-                                                    j0, j1, _L.C.c_void_p(st["ws_ptr"]), st["ws_bytes"], stream))
+        self._run_blocks(lib.hmc_random_run, a, stream)
         ev1.record()
         ev1.synchronize()
         self.kernel_ms = ev0.elapsed_time(ev1)
@@ -600,11 +627,12 @@ class HMC_sampler(sampler):
             self.phi_q = []                                                          # samplers.py:514 (never filled)
         dev = torch.device("cuda", torch.cuda.current_device())
         tgt, keep, tdt = self._build_target(torch, dev)
-        Nc, D, Lc = self.Nchain, self.D, self.L_chain
+        Nc, D = self.Nchain, self.D
         f64 = torch.float64
-        self._q_dev = torch.zeros((Nc, Lc, D), dtype=tdt, device=dev)
-        self._E_dev = torch.zeros((Nc, Lc), dtype=f64, device=dev)
-        self._dE_dev = torch.zeros((Nc, Lc), dtype=f64, device=dev)
+        rows = self._stream_setup(torch, dev, keep)
+        self._q_dev = torch.zeros((Nc, rows, D), dtype=tdt, device=dev)
+        self._E_dev = torch.zeros((Nc, rows), dtype=f64, device=dev)
+        self._dE_dev = torch.zeros((Nc, rows), dtype=f64, device=dev)
         self._q_host = self._E_host = self._dE_host = None
         qs = self._to_device(torch, q_start, dev, tdt)
         state_q = torch.empty((Nc, D), dtype=tdt, device=dev)
@@ -618,10 +646,9 @@ class HMC_sampler(sampler):
         a.dtype = _L.HMC_F32 if self.dtype == "float32" else _L.HMC_F64
         a.kernel = _L.KERNELS[self.kernel]
         # (mirror of the library's AUTO rule, for reports: csrc/api.cu hmc_nuts_run)
-        bigd_ok = self.dtype == "float32" and self._cov_p_identity and 128 <= D <= 8192
         if self.kernel in ("auto", "tc") and self.dtype == "float32" and D == 100 and self.d_max <= 12:
             self.nuts_kernel = "tc"
-        elif bigd_ok and (self.kernel == "bigd" or (self.kernel == "auto" and D > 256)):
+        elif nuts_runs_bigd(D, self.dtype, self.kernel, self._cov_p_identity, stream=self._stream is not None):
             self.nuts_kernel = "bigd"
         else:
             self.nuts_kernel = "generic"
@@ -639,6 +666,8 @@ class HMC_sampler(sampler):
             a.p_tape, a.dir_tape, a.u_tape = (keep[k].data_ptr() for k in ("p_tape", "dir_tape", "u_tape"))
             a.tape_dir_stride, a.tape_u_stride = keep["dir_tape"].shape[1], keep["u_tape"].shape[1]
         a.q_chain, a.E_chain, a.dE_chain = self._q_dev.data_ptr(), self._E_dev.data_ptr(), self._dE_dev.data_ptr()
+        if self._stream is not None:
+            a.store_ring = rows
         a.state_q, a.state_eprev = state_q.data_ptr(), state_e.data_ptr()
         a.scratch, a.counters, a.status, a.n_leapfrog = scratch.data_ptr(), counters.data_ptr(), status.data_ptr(), \
             nleap.data_ptr()
@@ -653,9 +682,7 @@ class HMC_sampler(sampler):
             print("Running %d NUTS chains x %d iterations on %s (%s, kernel=%s)" %
                   (Nc, self.Niter, torch.cuda.get_device_name(dev), self.dtype, self.nuts_kernel))
         ev0.record()
-        for (b, e) in self._blocks():
-            a.iter_begin, a.iter_end = b, e
-            _L.check(lib.hmc_nuts_run(a, stream))
+        self._run_blocks(lib.hmc_nuts_run, a, stream)
         ev1.record()
         ev1.synchronize()
         self.kernel_ms = ev0.elapsed_time(ev1)
